@@ -5,6 +5,7 @@ the fraction of the HBM roofline).
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path  (one process per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    # the reference's own modules on the host cores
     python bench.py --workload cfg5_e2e_b256_fusion ...      # under torchrun: encode -> gather -> VATLiDAR tokens
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also writes the last timed step's outputs to DIR/*.npy
 
 A "step" is one pass of the path (grouping -> pillar features -> BEV scatter) over one batch of synthetic sweeps per GPU.
 The timed region of K steps is repeated R times; every number is the MEDIAN region (max over ranks inside a region).
@@ -40,7 +41,9 @@ F_OUT = 64
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="steps in each timed region of the headline and cfg5 lines (--repeats regions of each kind); "
+                         "side measurements time min(K, 10) or min(K, 20) steps and say so in their fields")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--repeats", type=int, default=0, help="timed regions of K steps (0: max(5, ceil(100 / K)))")
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
@@ -64,7 +67,15 @@ def parse_args():
                     help="dtype of the feature rows on the wire in the multi-GPU gather")
     ap.add_argument("--cfg5-mode", default="fusion", choices=["fusion", "sharded", "backbone"],
                     help="cfg5: tokenise on the fusion rank after the gather, or on every rank (frames stay independent)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy; see "
+                         "dump_outputs and, for cfg5, dump_tokens")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of this repo's CUDA path: it needs --impl b200")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -351,8 +362,7 @@ def reference_eager_on_gpu(workload: str, n_frames: int, dev, steps: int = 10):
 def run_reference(args, rank):
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(1, min(args.warmup, 3))
-    steps = min(steps, 20)  # bound the whole run to a couple of minutes: one CPU step of 4 frames is ~1 s
+    steps, warmup = args.steps, max(1, min(args.warmup, 3))
     wl = DEFAULT_WORKLOAD if args.workload == CFG5 else args.workload
     r = cpu_reference_arm(wl, args.cpu_frames, steps, warmup)
     line = {
@@ -504,6 +514,8 @@ def encoder_numbers(wl: Workload, args, rank, world, K, R, lib, with_stage_event
             step(w, w % n_streams)
     torch.cuda.synchronize()
 
+    last = {}
+
     def pipelined_region():
         start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
@@ -514,18 +526,19 @@ def encoder_numbers(wl: Workload, args, rank, world, K, R, lib, with_stage_event
         for k in range(K):
             slot = k % n_streams
             with torch.cuda.stream(streams[slot]):
-                step(k, slot)
+                res = step(k, slot)
         for st_ in streams:
             cur.wait_stream(st_)
         stop.record(cur)
         barrier()
+        last["res"] = res
         return start.elapsed_time(stop)
 
     piped = timed_regions(pipelined_region, R, world, dev)
     stage_med = np.median(np.asarray(stage_rows), axis=0) if stage_rows else np.array([float("nan")] * 3)
     return {"serial_ms": serial, "piped_ms": piped, "stage_ms": stage_med, "n_raw": n_raw, "n_kept": n_kept,
             "m_avg": m_avg, "m_max": m_max, "launches_per_step": launches_per_step, "bufs": bufs, "streams": streams,
-            "step": step, "ev": (evs, ev_arrays)}
+            "step": step, "ev": (evs, ev_arrays), "last": last["res"]}
 
 
 def summarise(wl, enc, K, world, peak):
@@ -553,6 +566,57 @@ def summarise(wl, enc, K, world, peak):
     }
 
 
+DUMP_ARRAY_BYTES = 16 << 20  # per sampled array: a whole dump stays under 64 MB
+
+
+def dump_sample(n, row_bytes, seed):
+    """Indices 0..n-1, or a fixed seeded sorted sample of them when n rows of row_bytes exceed DUMP_ARRAY_BYTES."""
+    k = min(n, DUMP_ARRAY_BYTES // row_bytes)
+    return np.arange(n) if k == n else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def cells_of(t, cells):
+    """All channels of the cells (frame, y, x) with flat indices `cells` of an NCHW map: [cells, channels]."""
+    _, _, ny, nx = t.shape
+    return t[cells // (ny * nx), :, cells // nx % ny, cells % nx]
+
+
+def write_dump(out_dir, arrays):
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu()  # integers as float64 (exact), float64 kept, other floats as float32
+        a = a.float() if a.is_floating_point() and a.dtype != torch.float64 else a.double()
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+
+
+def dump_outputs(out_dir, res):
+    """Writes the arrays `encode_bev` returned in the last timed step as out_dir/<key>.npy: integer outputs as float64 (exact),
+    features and canvas as float32.  `pillar_features`, `voxel_coords` and `voxel_num_points` hold the first
+    `pillar_count[-1]` rows, or the same fixed seeded sample of them when those exceed 16 MB.  `bev` holds all channels of a
+    fixed seeded sample of the canvas cells, [cells, channels], cells in (frame, y, x) order; `bev_at_pillars` the same at the
+    cells of the dumped pillar rows (row i at voxel_coords[i]), where the mostly empty canvas holds its values."""
+    torch.cuda.synchronize()
+    counts = res["pillar_count"].cpu()
+    feats, coords, bev = res["pillar_features"], res["voxel_coords"], res["bev"]
+    rows = torch.from_numpy(dump_sample(int(counts[-1]), 4 * feats.shape[1], seed=0)).to(feats.device)
+    nb, c, ny, nx = bev.shape
+    cells = torch.from_numpy(dump_sample(nb * ny * nx, 4 * c, seed=1)).to(bev.device)
+    at = coords.index_select(0, rows).long()  # (frame, z, y, x)
+    write_dump(out_dir, {"pillar_count": counts, "pillar_features": feats.index_select(0, rows),
+                         "voxel_coords": coords.index_select(0, rows),
+                         "voxel_num_points": res["voxel_num_points"].index_select(0, rows),
+                         "bev": cells_of(bev, cells), "bev_at_pillars": bev[at[:, 0], :, at[:, 2], at[:, 3]]})
+
+
+def dump_tokens(out_dir, tok_out, checksum, extra=None):
+    """cfg5: the last token micro-batch [frames, cells, d] of the last timed step as rows [frames * cells, d] (a fixed seeded
+    sample beyond 16 MB), the running token checksum of the timed regions, and `extra` arrays (already sampled)."""
+    flat = tok_out.reshape(-1, tok_out.shape[-1])
+    rows = torch.from_numpy(dump_sample(flat.shape[0], 4 * flat.shape[1], seed=0)).to(flat.device)
+    write_dump(out_dir, {"tokens": flat.index_select(0, rows), "tokens_checksum": checksum, **(extra or {})})
+
+
 def run_b200(args, rank, world, local_rank):
     import torch.distributed as dist
 
@@ -569,7 +633,7 @@ def run_b200(args, rank, world, local_rank):
         opts = dist.ProcessGroupNCCL.Options(is_high_priority_stream=True)
         dist.init_process_group("nccl", device_id=dev, pg_options=opts)
     lib = _native.load()
-    K = max(1, args.steps)
+    K = args.steps
     R = args.repeats if args.repeats > 0 else max(5, math.ceil(100 / K))
     peak, peak_src = measured_peaks()
 
@@ -590,6 +654,8 @@ def run_b200(args, rank, world, local_rank):
     enc = encoder_numbers(wl, args, rank, world, K, R, lib)
     t1 = time.time()
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before the side measurements below reuse the step buffers
+        dump_outputs(args.dump_outputs, enc["last"])
     summ = summarise(wl, enc, K, world, peak)
     stages = summ["stages"]
     step, bufs, streams = enc["step"], enc["bufs"], enc["streams"]
@@ -1285,7 +1351,6 @@ def run_cfg5_backbone(args, rank, world, dev, wl, nb, total_frames, d_tok, K, R,
     buf = ops.EncodeBuffers(wl.n_max, nb, wl.grid, F_OUT, dev, with_bev=False)
     tok_out = torch.empty((nb, h2 * w2, d_tok), dtype=torch.float32, device=dev)
     checksum = torch.zeros(1, dtype=torch.float64, device=dev)
-    K5 = max(2, min(K, 6))
 
     def step(k):
         p, o = wl.dev_batches[k % wl.rot]
@@ -1305,15 +1370,20 @@ def run_cfg5_backbone(args, rank, world, dev, wl, nb, total_frames, d_tok, K, R,
         barrier()
         s.record()
         with torch.inference_mode():
-            for k in range(K5):
-                step(k)
+            for k in range(K):
+                last["f2d"] = step(k)
         e.record()
         barrier()
         return s.elapsed_time(e)
 
+    last = {}
     region()
     ms_all = timed_regions(region, max(3, min(R, 5)), world, dev)
-    ms = statistics.median(ms_all) / K5
+    ms = statistics.median(ms_all) / K
+    if args.dump_outputs and rank == 0:  # before the stage split below rewrites tok_out
+        f2d = last["f2d"]
+        cells = torch.from_numpy(dump_sample(f2d.shape[0] * f2d.shape[2] * f2d.shape[3], 4 * f2d.shape[1], seed=1))
+        dump_tokens(args.dump_outputs, tok_out, checksum, {"spatial_features_2d": cells_of(f2d, cells.to(f2d.device))})
     # stage split on this rank (serial, one step)
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
     with torch.inference_mode():
@@ -1329,7 +1399,7 @@ def run_cfg5_backbone(args, rank, world, dev, wl, nb, total_frames, d_tok, K, R,
     if rank == 0:
         tokens_bytes = total_frames * h2 * w2 * d_tok * 4
         line = {
-            "metric": METRIC, "value": total_frames / (ms * 1e-3), "unit": UNIT, "n_gpus": world, "steps": K5, "warmup": 1,
+            "metric": METRIC, "value": total_frames / (ms * 1e-3), "unit": UNIT, "n_gpus": world, "steps": K, "warmup": 1,
             "ms_per_step": ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32 (backbone: tf32 tensor cores)",
             "data": "synthetic", "repeats": len(ms_all),
             "config": {"workload": CFG5, "global_frames": total_frames, "frames_per_gpu": nb, "grid": [wl.nx, wl.ny, 1],
@@ -1373,7 +1443,6 @@ def run_cfg5(args, rank, world, dev, lib, K, R, peak, peak_src):
     streams = [torch.cuda.Stream(device=dev, priority=-1) for _ in range(n_slots)]
     micro = 16  # frames tokenised per call: the token tensor of 16 frames is 4.3 GB at d = 256
     tok_out = torch.empty((micro, wl.ny * wl.nx, d_tok), dtype=torch.float32, device=dev)
-    K5 = max(2, min(K, 6))
 
     def encode(k, slot):
         p, o = wl.dev_batches[k % wl.rot]
@@ -1418,7 +1487,7 @@ def run_cfg5(args, rank, world, dev, lib, K, R, peak, peak_src):
         tok_stream.wait_event(s)
         if gat is not None:
             gat.stream.wait_event(s)
-        for k in range(K5):
+        for k in range(K):
             slot = k % n_slots
             with torch.cuda.stream(streams[slot]):
                 if sent[slot] is not None:
@@ -1458,7 +1527,9 @@ def run_cfg5(args, rank, world, dev, lib, K, R, peak, peak_src):
     ms_all = timed_regions(region, max(3, min(R, 5)), world, dev)
     if gat is not None:
         gat.check()
-    ms = statistics.median(ms_all) / K5
+    ms = statistics.median(ms_all) / K
+    if args.dump_outputs and rank == 0:  # before the stage split below rewrites tok_out
+        dump_tokens(args.dump_outputs, tok_out, checksum)
     # stage split (rank 0, one step each, serial): encoder / tokeniser per 16 frames
     torch.cuda.synchronize()
     s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -1475,7 +1546,7 @@ def run_cfg5(args, rank, world, dev, lib, K, R, peak, peak_src):
     if rank == 0:
         tokens_bytes = total_frames * wl.ny * wl.nx * d_tok * 4
         line = {
-            "metric": METRIC, "value": total_frames / (ms * 1e-3), "unit": UNIT, "n_gpus": world, "steps": K5,
+            "metric": METRIC, "value": total_frames / (ms * 1e-3), "unit": UNIT, "n_gpus": world, "steps": K,
             "warmup": 1, "ms_per_step": ms, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
             "data": "synthetic", "repeats": len(ms_all),
             "config": {"workload": CFG5, "global_frames": total_frames, "frames_per_gpu": nb, "grid": [wl.nx, wl.ny, 1],

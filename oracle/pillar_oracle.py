@@ -24,6 +24,7 @@ Pieces (each cites the reference lines it restates; paths relative to ``src/lida
 from __future__ import annotations
 
 import ctypes
+import hashlib
 import os
 import subprocess
 from typing import Dict, List, Optional, Sequence, Tuple
@@ -178,6 +179,31 @@ def voxelize_batch(points: np.ndarray, frame_offsets: np.ndarray, point_cloud_ra
         "point_slot": ps_all,
         "pillars_per_frame": np.asarray(counts, np.int32),
     }
+
+
+def golden_backbone_inputs(module: torch.nn.Module, seed: int, nb: int, h: int, w: int):
+    """The inputs of a tests/golden/bb_*.npz case (tests/golden/make_golden_backbone.py) for a BaseBEVBackbone built right
+    after ``torch.manual_seed(seed)``: non-trivial BatchNorm statistics, every float parameter rounded to float16, and a
+    sparse pillar-like canvas [nb, 64, h, w] of float16 values.  Updates ``module`` in place; returns its state dict, the
+    canvas (float32) and the SHA-256 (32 uint8) of both, parameters in state-dict order."""
+    g = torch.Generator().manual_seed(seed + 100)
+    with torch.no_grad():
+        for mod in module.modules():
+            if isinstance(mod, torch.nn.BatchNorm2d):
+                mod.weight.copy_(0.5 + torch.rand(mod.weight.shape, generator=g))
+                mod.bias.copy_(0.2 * torch.randn(mod.bias.shape, generator=g))
+                mod.running_mean.copy_(0.2 * torch.randn(mod.bias.shape, generator=g))
+                mod.running_var.copy_(0.5 + 1.5 * torch.rand(mod.bias.shape, generator=g))
+        for v in module.state_dict().values():
+            if v.dtype == torch.float32:
+                v.copy_(v.half().float())
+    occ = torch.rand((nb, 1, h, w), generator=g) < 0.08
+    canvas = (torch.rand((nb, 64, h, w), generator=g) * occ).half().float()
+    sd = module.state_dict()
+    digest = hashlib.sha256()
+    for v in list(sd.values()) + [canvas]:
+        digest.update((v.half() if v.dtype == torch.float32 else v).numpy().tobytes())
+    return sd, canvas, np.frombuffer(digest.digest(), np.uint8)
 
 
 # --------------------------------------------------------------------------------------------------

@@ -13,6 +13,7 @@ norm_tokens.{weight,bias}, geo_mlp.{0,2}.{weight,bias}, view_embed.
 """
 from __future__ import annotations
 
+import hashlib
 import math
 
 import numpy as np
@@ -130,3 +131,22 @@ def random_token_params(c_in: int, d_model: int, seed: int):
         "geo_mlp.2.weight": u((d_model, d_model), 1.0 / math.sqrt(d_model)), "geo_mlp.2.bias": u((d_model,), 0.2),
         "view_embed": u((NUM_VIEWS, d_model), 0.5),
     }
+
+
+def golden_token_inputs(b: int, c: int, d: int, h: int, w: int, seed: int, occupancy: float):
+    """The seeded canvas [b, c, h, w] and weights of a tests/golden/tok_*.npz case (tests/golden/make_golden_tokens.py).
+    Below full occupancy it is a pillar canvas: most cells hold exact zeros in every channel, occupied ones are post-ReLU."""
+    rng = np.random.default_rng(seed)
+    bev = rng.standard_normal((b, c, h, w)).astype(np.float32)
+    if occupancy < 1.0:
+        occ = rng.random((b, 1, h, w)) < occupancy
+        bev = np.where(occ, np.maximum(bev, 0.0), 0.0).astype(np.float32)
+    return bev, random_token_params(c, d, seed + 7)
+
+
+def golden_inputs_sha256(bev: np.ndarray, sd: dict) -> np.ndarray:
+    """SHA-256 (32 uint8) of a canvas and its weights, weights in key order: pins the regenerated inputs of a compact golden."""
+    h = hashlib.sha256(np.ascontiguousarray(bev).tobytes())
+    for k in sorted(sd):
+        h.update(np.ascontiguousarray(sd[k]).tobytes())
+    return np.frombuffer(h.digest(), np.uint8)

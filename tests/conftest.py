@@ -20,6 +20,15 @@ def load_golden(name):
     z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
     d = {k: z[k] for k in z.files}
     d["state_dict"] = {k[3:]: d[k] for k in d if k.startswith("sd.")}
+    if "gen.seed" in d:  # a compact token golden: the canvas and weights come from their seed (make_golden_tokens.py)
+        from oracle import tokens_oracle as to
+
+        h, w = (int(v) for v in d["gen.hw"])
+        bev, sd = to.golden_token_inputs(int(d["gen.batch"]), int(d["c_in"]), int(d["d_model"]), h, w, int(d["gen.seed"]),
+                                         float(d["gen.occupancy"]))
+        b = d["out.tokens"].shape[0]
+        d["bev"], d["state_dict"] = bev[:b], sd
+        assert np.array_equal(to.golden_inputs_sha256(d["bev"], sd), d["gen.sha256"]), f"{name}: regenerated inputs differ"
     return d
 
 

@@ -4,7 +4,9 @@ Run in the build container (needs /root/reference or the oracle/_ref copy):  pyt
 Each .npz holds the module config, its complete state dict (random weights, non-trivial BatchNorm statistics), a sparse
 pillar-like canvas and the `spatial_features_2d` the unmodified `BaseBEVBackbone.forward` (base_bev_backbone.py:82-112)
 returns for it on the CPU in fp32.  Weights are stored as float16-representable values to keep the files small (the module is
-loaded with exactly these values on both sides, so nothing is lost)."""
+loaded with exactly these values on both sides, so nothing is lost).  A ``compact`` case stores instead of the state dict and
+the canvas only their recipe (``pillar_oracle.golden_backbone_inputs`` on a module built after ``torch.manual_seed(seed)``), the
+reference's state-dict keys in order and the SHA-256 of the inputs, so that no file exceeds 1 MB."""
 import json
 import os
 import sys
@@ -14,13 +16,14 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+from oracle import pillar_oracle as po  # noqa: E402
 from oracle import ref_loader as R  # noqa: E402
 
 CASES = {
     "bb_2level_half_stride": dict(cfg=dict(LAYER_NUMS=[1, 1], LAYER_STRIDES=[2, 2], NUM_FILTERS=[64, 128],
                                            UPSAMPLE_STRIDES=[0.5, 1], NUM_UPSAMPLE_FILTERS=[128, 128]), h=48, w=40, nb=2, seed=1),
     "bb_3level_up124": dict(cfg=dict(LAYER_NUMS=[1, 1, 0], LAYER_STRIDES=[2, 2, 2], NUM_FILTERS=[64, 128, 256],
-                                     UPSAMPLE_STRIDES=[1, 2, 4], NUM_UPSAMPLE_FILTERS=[64, 64, 64]), h=64, w=32, nb=1, seed=2),
+                                     UPSAMPLE_STRIDES=[1, 2, 4], NUM_UPSAMPLE_FILTERS=[64, 64, 64]), h=64, w=32, nb=1, seed=2, compact=True),
 }
 
 
@@ -29,25 +32,17 @@ def main():
     for name, c in CASES.items():
         torch.manual_seed(c["seed"])
         m = BB(R.AttrDict(c["cfg"]), 64).eval()
-        g = torch.Generator().manual_seed(c["seed"] + 100)
-        with torch.no_grad():
-            for mod in m.modules():
-                if isinstance(mod, torch.nn.BatchNorm2d):
-                    mod.weight.copy_(0.5 + torch.rand(mod.weight.shape, generator=g))
-                    mod.bias.copy_(0.2 * torch.randn(mod.bias.shape, generator=g))
-                    mod.running_mean.copy_(0.2 * torch.randn(mod.bias.shape, generator=g))
-                    mod.running_var.copy_(0.5 + 1.5 * torch.rand(mod.bias.shape, generator=g))
-            for k, v in m.state_dict().items():  # float16-representable parameters
-                if v.dtype == torch.float32:
-                    v.copy_(v.half().float())
-        occ = torch.rand((c["nb"], 1, c["h"], c["w"]), generator=g) < 0.08
-        canvas = (torch.rand((c["nb"], 64, c["h"], c["w"]), generator=g) * occ).half().float()
+        sd, canvas, sha = po.golden_backbone_inputs(m, c["seed"], c["nb"], c["h"], c["w"])
         with torch.inference_mode():
             out = m({"spatial_features": canvas.clone()})["spatial_features_2d"]
-        save = {"cfg": np.frombuffer(json.dumps(c["cfg"]).encode(), dtype=np.uint8), "canvas": canvas.numpy().astype(np.float16),
-                "out": out.numpy()}
-        for k, v in m.state_dict().items():
-            save["sd." + k] = v.numpy().astype(np.float16) if v.dtype == torch.float32 else v.numpy()
+        save = {"cfg": np.frombuffer(json.dumps(c["cfg"]).encode(), dtype=np.uint8), "out": out.numpy()}
+        if c.get("compact"):
+            save.update({"gen.seed": np.int32(c["seed"]), "gen.shape": np.int32([c["nb"], c["h"], c["w"]]),
+                         "sd_keys": np.frombuffer(json.dumps(list(sd)).encode(), np.uint8), "gen.sha256": sha})
+        else:
+            save["canvas"] = canvas.numpy().astype(np.float16)
+            for k, v in sd.items():
+                save["sd." + k] = v.numpy().astype(np.float16) if v.dtype == torch.float32 else v.numpy()
         path = os.path.join(HERE, name + ".npz")
         np.savez_compressed(path, **save)
         print(name, tuple(out.shape), os.path.getsize(path) // 1024, "KiB")

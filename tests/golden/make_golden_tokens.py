@@ -3,8 +3,10 @@ src/encoder-decoder/training/models/vat_lidar.py) and capturing the BEV K/V toke
 VAT block (forward pre-hook on ``blocks[0]``; vat_lidar.py:206-253,285).
 
 Run in the build container only:   python tests/golden/make_golden_tokens.py
-Every file stores the input canvas, the tokeniser weights under the reference's state_dict keys, the reference's
-geometry tables (``_grid``: vat_lidar.py:123-185) and the tokens.
+Every file stores the reference's geometry tables (``_grid``: vat_lidar.py:123-185) and the tokens, with either the input
+canvas and the tokeniser weights under the reference's state_dict keys, or (``compact``) only the recipe they are regenerated
+from (``tokens_oracle.golden_token_inputs``) and the SHA-256 of those inputs; a compact case may keep the tokens of
+its first ``keep`` frames only (frames are independent), so that no file exceeds 1 MB.
 """
 import os
 import sys
@@ -21,33 +23,33 @@ from oracle import tokens_oracle as to  # noqa: E402
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
-def run_case(name, *, b, c, d, h, w, seed, occupancy):
+def run_case(name, *, b, c, d, h, w, seed, occupancy, compact=False, keep=None):
     vat = ref_loader.load_vat_lidar()
     torch.manual_seed(seed)
     model = vat(c_in=c, d_model=d, n_queries=12, n_layers=1, n_heads=4).eval()
-    sd = to.random_token_params(c, d, seed + 7)
+    bev, sd = to.golden_token_inputs(b, c, d, h, w, seed, occupancy)
     res = model.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()}, strict=False)
     assert not res.unexpected_keys and all(not k.startswith(to.TOKEN_KEYS) for k in res.missing_keys)
-    rng = np.random.default_rng(seed)
-    bev = rng.standard_normal((b, c, h, w)).astype(np.float32)
-    if occupancy < 1.0:  # a pillar canvas: most cells hold exact zeros in every channel, occupied ones are post-ReLU
-        occ = rng.random((b, 1, h, w)) < occupancy
-        bev = np.where(occ, np.maximum(bev, 0.0), 0.0).astype(np.float32)
     tokens = ref_loader.vat_lidar_kv_tokens(model, torch.from_numpy(bev)).numpy()
     geom, sid = model._grid(h, w, torch.device("cpu"))
-    save = {"bev": bev, "out.tokens": tokens, "geom": geom.numpy(), "sid": sid.numpy().astype(np.int32),
+    save = {"out.tokens": tokens[:keep], "geom": geom.numpy(), "sid": sid.numpy().astype(np.int32),
             "c_in": np.int32(c), "d_model": np.int32(d)}
-    for k, v in sd.items():
-        save["sd." + k] = v
+    if compact:
+        save.update({"gen.batch": np.int32(b), "gen.hw": np.int32([h, w]), "gen.seed": np.int32(seed), "gen.occupancy": np.float64(occupancy),
+                     "gen.sha256": to.golden_inputs_sha256(bev[:keep], sd)})
+    else:
+        save["bev"] = bev[:keep]
+        for k, v in sd.items():
+            save["sd." + k] = v
     path = os.path.join(OUT, name + ".npz")
     np.savez_compressed(path, **save)
-    print(f"{name}: bev={bev.shape} tokens={tokens.shape} nonzero cells={(np.abs(bev).max(1) > 0).mean():.2f} "
+    print(f"{name}: bev={bev[:keep].shape} tokens={tokens[:keep].shape} nonzero cells={(np.abs(bev).max(1) > 0).mean():.2f} "
           f"-> {os.path.getsize(path) / 1024:.0f} KiB")
 
 
 def main():
     run_case("tok_c64_d128_16x16_dense", b=2, c=64, d=128, h=16, w=16, seed=0, occupancy=1.0)
-    run_case("tok_c64_d256_24x20_sparse", b=3, c=64, d=256, h=24, w=20, seed=1, occupancy=0.07)
+    run_case("tok_c64_d256_24x20_sparse", b=3, c=64, d=256, h=24, w=20, seed=1, occupancy=0.07, compact=True, keep=2)
     run_case("tok_c32_d128_13x9_odd", b=2, c=32, d=128, h=13, w=9, seed=2, occupancy=0.3)
     run_case("tok_c128_d384_8x8", b=1, c=128, d=384, h=8, w=8, seed=3, occupancy=0.5)
 

@@ -263,20 +263,32 @@ def test_points_to_backbone_without_a_canvas_equals_the_canvas_route():
 @pytest.mark.parametrize("name", ["bb_2level_half_stride", "bb_3level_up124"])
 def test_backbone_against_committed_reference_goldens(name):
     """tests/golden/bb_*.npz: config, state dict, canvas and the output of the reference's own BaseBEVBackbone.forward
-    (made by tests/golden/make_golden_backbone.py in the build container).  Nothing here reads /root/reference."""
+    (made by tests/golden/make_golden_backbone.py).  A compact file holds the seed of the state dict and canvas instead: they
+    are rebuilt here and must hash to what the reference module was run on, in the reference's state-dict key order."""
     import json
     import os
 
     from lidar_vision_vqa_b200.backbone import BaseBEVBackbone
+    from oracle import pillar_oracle as po
 
     z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name + ".npz"))
     cfg = json.loads(bytes(z["cfg"]).decode())
-    m = BaseBEVBackbone(cfg, 64).eval()
-    sd = {k[3:]: torch.from_numpy(z[k].astype(np.float32) if z[k].dtype == np.float16 else z[k]) for k in z.files if k.startswith("sd.")}
+    if "gen.seed" in z.files:
+        torch.manual_seed(int(z["gen.seed"]))
+        m = BaseBEVBackbone(cfg, 64).eval()
+        sd, canvas, sha = po.golden_backbone_inputs(m, int(z["gen.seed"]), *(int(v) for v in z["gen.shape"]))
+        assert list(sd.keys()) == json.loads(bytes(z["sd_keys"]).decode())
+        assert np.array_equal(sha, z["gen.sha256"]), "regenerated state dict / canvas differ from the reference's inputs"
+    else:
+        m = BaseBEVBackbone(cfg, 64).eval()
+        sd = {k[3:]: torch.from_numpy(z[k].astype(np.float32) if z[k].dtype == np.float16 else z[k]) for k in z.files
+              if k.startswith("sd.")}
+        canvas = torch.from_numpy(z["canvas"].astype(np.float32))
     m.load_state_dict(sd, strict=True)
+    assert m.num_bev_features == z["out"].shape[1]
     dev = _dev()
     m = m.to(dev)
-    canvas = torch.from_numpy(z["canvas"].astype(np.float32)).to(dev)
+    canvas = canvas.to(dev)
     with torch.inference_mode():
         out = m({"spatial_features": canvas})
     torch.cuda.synchronize()
