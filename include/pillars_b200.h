@@ -327,6 +327,19 @@ int pillars_set_stage_events(void *const *events4);
  * either choice. */
 int pillars_set_grouping(int mode);
 
+/* Canvas occupancy bitmaps for the next pillars_encode_bev or pillars_encode_stack on this thread, which consumes and
+ * clears them whether it succeeds or fails.  A canvas the library wrote before is mostly zeros already; with the bitmaps
+ * the scatter writes only the cells that are occupied now or were occupied in the canvas's previous contents.
+ * Layout: words [n_frames][ceil(nx*ny / 256)] of uint32 (device memory); bit k of word w of frame b covers the 8 cells
+ * 256*w + 8*k .. 256*w + 8*k + 7 of that frame's ny*nx plane (row-major y, x), set = "may be non-zero".
+ *   prev  the bitmap the last call on this canvas wrote into its next, describing what the canvas holds now; NULL when the
+ *         contents are unknown (fresh or written by anyone else): the whole canvas is written.
+ *   next  receives the occupancy this call leaves (all ones when it writes the canvas with the plain kernel).  Must not
+ *         alias prev: the caller keeps two bitmaps per canvas and swaps them after every call.
+ * The canvas, prev and next must be ordered with the call like the canvas alone (same stream or events).  It is an error
+ * for a call with bitmaps to write both bev and bev_half.  NULL, NULL clears the hook. */
+int pillars_set_canvas_occupancy(const uint32_t *prev, uint32_t *next);
+
 /* Measurement hook (thread-local): a zeroed device buffer of 32 uint64 that the grouping / feature kernels of subsequent calls
  * stamp with %globaltimer nanoseconds per phase (even slot: earliest stamp, stored complemented; odd slot: latest stamp);
  * NULL switches it off.  profiles/scripts/phase_times.py decodes it. */

@@ -41,6 +41,7 @@ EXPORTED_SYMBOLS = (
     "pillars_conv_prepare",
     "pillars_conv_forward",
     "pillars_canvas_to_rows",
+    "pillars_set_canvas_occupancy",
 )
 
 ABI_VERSION = 5
@@ -174,6 +175,8 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
     lib.pillars_rebase_segments.argtypes = [c_void_p, c_int32, c_int64, c_int64, c_void_p, c_int64, c_int32, c_void_p, c_void_p]
     lib.pillars_set_debug_times.restype = c_int
     lib.pillars_set_debug_times.argtypes = [c_void_p]
+    lib.pillars_set_canvas_occupancy.restype = c_int
+    lib.pillars_set_canvas_occupancy.argtypes = [c_void_p, c_void_p]
     lib.pillars_set_grouping.restype = c_int
     lib.pillars_set_grouping.argtypes = [c_int]
     lib.pillars_force_generic_features.restype = c_int

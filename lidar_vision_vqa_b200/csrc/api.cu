@@ -15,6 +15,20 @@ static thread_local int g_launches_last = 0;
 static thread_local cudaEvent_t g_stage_ev[4] = {nullptr, nullptr, nullptr, nullptr};
 static thread_local bool g_stage_on = false;
 
+// canvas occupancy bitmaps for the next pillars_encode_bev / pillars_encode_stack on this thread (one-shot)
+struct CanvasOccupancy {
+    const uint32_t *prev = nullptr;
+    uint32_t *next = nullptr;
+};
+static thread_local CanvasOccupancy g_occ;
+
+static CanvasOccupancy take_canvas_occupancy()
+{
+    const CanvasOccupancy o = g_occ;
+    g_occ = CanvasOccupancy{};
+    return o;
+}
+
 static void stage_mark(int i, cudaStream_t st)
 {
     if (g_stage_on && g_stage_ev[i]) cudaEventRecord(g_stage_ev[i], st);
@@ -145,6 +159,15 @@ int pillars_set_stage_events(void *const *events4)
     return 0;
 }
 
+int pillars_set_canvas_occupancy(const uint32_t *prev, uint32_t *next)
+{
+    g_occ = CanvasOccupancy{};
+    if (prev && !next) return fail(PILLARS_E_BADARG, "canvas occupancy: prev without next");
+    g_occ.prev = prev;
+    g_occ.next = next;
+    return 0;
+}
+
 int pillars_set_debug_times(void *buffer32)
 {
     g_dbg_times = static_cast<unsigned long long *>(buffer32);
@@ -199,11 +222,13 @@ int pillars_frame_offsets(const float *points_b, int64_t n, int32_t row_stride, 
 static int group_and_emit(const float *points, int64_t n, int32_t row_stride, int32_t col0, int32_t c_point,
                           const int32_t *frame_offsets, int32_t n_frames, const pillars_grid_t *grid,
                           const pillars_pfn_t *pfn, const pillars_outputs_t *out, void *workspace, size_t workspace_bytes,
-                          bool want_bev, int scatter_variant, void *stream)
+                          bool want_bev, int scatter_variant, void *stream, CanvasOccupancy occ = {})
 {
     g_launches = 0;
     int rc;
     if ((rc = check_grid(grid, n_frames))) return rc;
+    if (occ.next && out && out->bev && out->bev_half)
+        return fail(PILLARS_E_BADARG, "canvas occupancy is set but the call writes both bev and bev_half");
     if ((rc = check_points(points, n, row_stride, col0, c_point))) return rc;
     if (!frame_offsets || !out) return fail(PILLARS_E_BADARG, "frame_offsets / out is NULL");
     if (n > 0 && n_frames == 0) return fail(PILLARS_E_BADARG, "n_points = %lld with n_frames = 0", (long long)n);
@@ -301,11 +326,11 @@ static int group_and_emit(const float *points, int64_t n, int32_t row_stride, in
         cudaStream_t sst = st;
         if (out->bev &&
             (e = launch_scatter(out->pillar_features, ws.cell_row, n_frames, pfn->f_out, grid->grid[0], grid->grid[1],
-                                out->bev, scatter_variant, sst)) != cudaSuccess)
+                                out->bev, scatter_variant, sst, occ.prev, occ.next)) != cudaSuccess)
             return cuda_fail(e, "scatter");
         if (out->bev_half &&
             (e = launch_scatter_half(out->pillar_features, ws.cell_row, n_frames, pfn->f_out, grid->grid[0],
-                                     grid->grid[1], out->bev_half, sst)) != cudaSuccess)
+                                     grid->grid[1], out->bev_half, sst, occ.prev, occ.next)) != cudaSuccess)
             return cuda_fail(e, "scatter (float16 canvas: needs nx*ny % 8 == 0, f % 8 == 0)");
     }
     stage_mark(3, st);
@@ -340,9 +365,11 @@ int pillars_encode_bev(const float *points, int64_t n, int32_t row_stride, int32
                        const pillars_outputs_t *out, void *workspace, size_t workspace_bytes, int32_t scatter_variant,
                        void *stream)
 {
+    const CanvasOccupancy occ = take_canvas_occupancy();
     if (!pfn) return fail(PILLARS_E_BADARG, "pfn is NULL");
     return group_and_emit(points, n, row_stride, col0, pfn->c_point, frame_offsets, n_frames, grid, pfn, out, workspace,
-                          workspace_bytes, out && (out->bev != nullptr || out->bev_half != nullptr), scatter_variant, stream);
+                          workspace_bytes, out && (out->bev != nullptr || out->bev_half != nullptr), scatter_variant, stream,
+                          occ);
 }
 
 int pillars_pfn_dense(const float *voxels, const void *num_points, int32_t num_points_is_float, const void *coords,
@@ -436,6 +463,7 @@ int pillars_encode_stack(const float *points, int64_t n, int32_t row_stride, int
                          int32_t coords_cols, const pillars_outputs_t *out, void *workspace, size_t workspace_bytes,
                          int32_t scatter_variant, void *stream)
 {
+    const CanvasOccupancy occ = take_canvas_occupancy();
     g_launches = 0;
     int rc;
     if ((rc = check_grid(grid, n_frames))) return rc;
@@ -449,6 +477,8 @@ int pillars_encode_stack(const float *points, int64_t n, int32_t row_stride, int
         return fail(PILLARS_E_UNSUPPORTED, "membership outputs come from pillars_voxelize");
     const bool dynamic = mode == PILLARS_MODE_DYNAMIC;
     const bool want_bev = out->bev != nullptr || out->bev_half != nullptr;
+    if (occ.next && out->bev && out->bev_half)
+        return fail(PILLARS_E_BADARG, "canvas occupancy is set but the call writes both bev and bev_half");
     if ((want_bev || out->want_index_map) && (dynamic || grid->grid[2] != 1 || coords_cols != 4))
         return fail(PILLARS_E_UNSUPPORTED, "the fused BEV canvas / index map needs mode HARD, nz == 1 and 4-column coords");
     if (out->pillar_capacity < 0) return fail(PILLARS_E_BADARG, "pillar_capacity < 0");
@@ -558,10 +588,10 @@ int pillars_encode_stack(const float *points, int64_t n, int32_t row_stride, int
     if (want_bev) {
         const int f_last = sd.out[sd.n_layers - 1];
         if (out->bev && (e = launch_scatter(out->pillar_features, ws.cell_row, n_frames, f_last, grid->grid[0],
-                                            grid->grid[1], out->bev, scatter_variant, st)) != cudaSuccess)
+                                            grid->grid[1], out->bev, scatter_variant, st, occ.prev, occ.next)) != cudaSuccess)
             return cuda_fail(e, "scatter");
         if (out->bev_half && (e = launch_scatter_half(out->pillar_features, ws.cell_row, n_frames, f_last, grid->grid[0],
-                                                      grid->grid[1], out->bev_half, st)) != cudaSuccess)
+                                                      grid->grid[1], out->bev_half, st, occ.prev, occ.next)) != cudaSuccess)
             return cuda_fail(e, "scatter (float16 canvas)");
     }
     stage_mark(3, st);

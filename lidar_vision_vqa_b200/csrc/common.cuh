@@ -373,14 +373,16 @@ cudaError_t launch_pfn_multi_dense(const float *voxels, const void *num_points, 
 
 cudaError_t launch_build_cell_row(const void *coords, bool coords_float, int64_t m, const int32_t *m_dev, int nb, int nx,
                                   int ny, int nz, int32_t *cell_row, cudaStream_t st);
+// occ_prev / occ_next: the canvas occupancy bitmaps of pillars_set_canvas_occupancy (NULL: none); only the wide kernels
+// skip stores, the plain kernel writes everything and sets occ_next to all ones
 cudaError_t launch_scatter(const float *feats, const int32_t *cell_row, int nb, int f, int nx, int ny, float *bev,
-                           int variant, cudaStream_t st);
+                           int variant, cudaStream_t st, const uint32_t *occ_prev = nullptr, uint32_t *occ_next = nullptr);
 cudaError_t launch_rebase_segments(int32_t *coords, int n_seg, int64_t rows_per_seg, int64_t seg_stride,
                                    const int32_t *seg_counts, int64_t count_stride, int frames_per_seg, int32_t *overflow,
                                    cudaStream_t st);
 // float16 canvas (plane % 8 == 0, f % 8 == 0)
 cudaError_t launch_scatter_half(const float *feats, const int32_t *cell_row, int nb, int f, int nx, int ny, void *bev,
-                                cudaStream_t st);
+                                cudaStream_t st, const uint32_t *occ_prev = nullptr, uint32_t *occ_next = nullptr);
 
 // ---- BEV tokeniser (tokens.cu): head of VATLiDAR.forward, src/encoder-decoder/training/models/vat_lidar.py:206-253 ----
 struct TokenizerDev {

@@ -6,6 +6,12 @@
 // grouping stage or by k_build_cell_row) turns the scatter inside out: every output element is written exactly once,
 // in NCHW order, with full-line stores, zero-fill included, no atomics.
 //
+// On a canvas the library wrote before, most of those stores put zeros over zeros.  The wide kernels then take two
+// occupancy bitmaps (layout in include/pillars_b200.h, pillars_set_canvas_occupancy): bit = "these 8 cells of the frame
+// may be non-zero".  A lane writes its 8 cells x channels only when they are occupied now or were last time (zeros
+// where only the old bit is set); every other canvas element already holds its zero.  The store unit stays one 32-byte
+// sector, so no sector is ever written in part.
+//
 // Two kernels ship: the channel-group 256-bit store kernel (k_scatter_wide, 99 % of the measured copy peak) and a plain
 // kernel for shapes it does not cover (odd plane sizes, unaligned canvases, F not a multiple of 8).  The other store paths
 // that were measured and lost (bulk 1-D copies, TMA tile stores, persistent warps, zero-fill + patches) are kept as
@@ -148,6 +154,22 @@ k_scatter_plain(const float *__restrict__ feats, const int32_t *__restrict__ cel
     }
 }
 
+// ---- occupancy bitmaps ------------------------------------------------------------------------------
+// One bit per 8 cells, one word per 256 cells (a warp of the wide kernels), words_per_frame = ceil(plane / 256).
+__host__ __device__ __forceinline__ int64_t occ_words(int64_t plane) { return (plane + 255) >> 8; }
+
+// The occ_prev word of the calling warp of a wide-kernel CTA (blockIdx decoded as there), all ones when there is no
+// bitmap or the warp lies past the plane.
+__device__ __forceinline__ uint32_t occ_prev_word(const uint32_t *__restrict__ occ_prev, int64_t plane, int tiles_per_plane,
+                                                  int groups, int tile_major)
+{
+    if (!occ_prev) return 0xffffffffu;
+    const int tile = tile_major ? (blockIdx.x / groups) % tiles_per_plane : blockIdx.x % tiles_per_plane;
+    const int b = blockIdx.x / (groups * tiles_per_plane);
+    const int64_t word = (static_cast<int64_t>(tile) * blockDim.x + threadIdx.x) >> 5;
+    return word < occ_words(plane) ? __ldg(occ_prev + b * occ_words(plane) + word) : 0xffffffffu;
+}
+
 // ---- variant 4 ----------------------------------------------------------------------------------
 // Same warp-autonomous scheme with 256-bit accesses (sm_100: LDG.256 / STG.256): a lane owns 8 consecutive cells, a warp
 // 256 cells x all channels = 64 KB of the canvas, and every store instruction of the warp writes 1 KB contiguous.  Half the
@@ -171,11 +193,16 @@ __device__ __forceinline__ void stg256_cs(float *p, float a, float b, float c, f
 // the CTAs of one cell tile then each read one 32-byte sector of every pillar row, so no feature byte is fetched twice.
 // tile_major != 0: consecutive CTAs are the channel groups of one cell tile (index map and feature rows are shared by CTAs
 // that run together); 0: consecutive CTAs walk the plane for one channel group.
+// occ_next != NULL: a lane stores only where its bit of occ_prev (NULL: all set) or its "any cell occupied" test is set, and
+// the channel group 0 CTAs record the latter into occ_next.
 template <bool CS, int CPP>
 __global__ void __launch_bounds__(kThreads)
 k_scatter_wide(const float *__restrict__ feats, const int32_t *__restrict__ cell_row, int f, int64_t plane,
-               int tiles_per_plane, int chan_per_cta, int tile_major, float *__restrict__ bev)
+               int tiles_per_plane, int chan_per_cta, int tile_major, float *__restrict__ bev,
+               const uint32_t *__restrict__ occ_prev, uint32_t *__restrict__ occ_next)
 {
+    // the previous call on this canvas wrote occ_prev and finished before this call's first (non-PDL) launch
+    const uint32_t prev = occ_prev_word(occ_prev, plane, tiles_per_plane, f / chan_per_cta, tile_major);
     pdl_wait();  // feature rows and index map come from the kernels before this one
     const int groups = f / chan_per_cta;
     int b, tile, cg;
@@ -208,14 +235,14 @@ k_scatter_wide(const float *__restrict__ feats, const int32_t *__restrict__ cell
         if (CS) stg256_cs(p, a, b2, c, d, e, f2, g, h);
         else stg256(p, a, b2, c, d, e, f2, g, h);
     };
-    if (!__any_sync(0xffffffffu, any)) {
-        if (inb) {
+    const uint32_t now = __ballot_sync(0xffffffffu, any);
+    if (occ_next && cg == 0 && (threadIdx.x & 31) == 0 && inb) occ_next[b * occ_words(plane) + (cell0 >> 8)] = now;
+    if (!inb || !(any || ((prev >> (threadIdx.x & 31)) & 1u))) return;
+    if (now == 0) {
 #pragma unroll 8
-            for (int c = c_begin; c < c_end; ++c) store(dst + c * plane, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f);
-        }
+        for (int c = c_begin; c < c_end; ++c) store(dst + c * plane, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f);
         return;
     }
-    if (!inb) return;
     constexpr int kV = CPP / 4;  // 16-byte loads per row and pass
     for (int c0 = c_begin; c0 < c_end; c0 += CPP) {
         float4 v[8][kV];
@@ -251,10 +278,14 @@ __device__ __forceinline__ void ldg256_stream(const float *p, float (&v)[8])
 // The product's caller stores the BEV map as float16 (src/get-data/precompute_bev_features.py:394: bev.astype(np.float16));
 // converting in the scatter halves the dominant write.  Same work split as variant 4: a lane owns 8 cells = one 16-byte
 // store per channel, round-to-nearest-even like numpy / torch.
+// A lane's 16 bytes are half a sector: the pair of lanes that shares one decides together, so that no sector is written in
+// part (L2 would fetch the rest of it from DRAM).
 __global__ void __launch_bounds__(kThreads)
 k_scatter_wide_half(const float *__restrict__ feats, const int32_t *__restrict__ cell_row, int f, int64_t plane,
-                    int tiles_per_plane, __half *__restrict__ bev)
+                    int tiles_per_plane, __half *__restrict__ bev, const uint32_t *__restrict__ occ_prev,
+                    uint32_t *__restrict__ occ_next)
 {
+    const uint32_t prev = occ_prev_word(occ_prev, plane, tiles_per_plane, f >> 3, 0);
     const int groups = f >> 3;
     const int tile = blockIdx.x % tiles_per_plane;
     const int cg = (blockIdx.x / tiles_per_plane) % groups;
@@ -275,14 +306,15 @@ k_scatter_wide_half(const float *__restrict__ feats, const int32_t *__restrict__
     for (int k = 0; k < 8; ++k) any |= r[k] >= 0;
     const int c0 = cg * 8;
     __half *dst = bev + (static_cast<int64_t>(b) * f + c0) * plane + cell0;
-    if (!__any_sync(0xffffffffu, any)) {
-        if (inb) {
+    const uint32_t now = __ballot_sync(0xffffffffu, any);
+    if (occ_next && cg == 0 && (threadIdx.x & 31) == 0 && inb) occ_next[b * occ_words(plane) + (cell0 >> 8)] = now;
+    const uint32_t pair = (now | prev) | (((now | prev) >> 1) & 0x55555555u) | (((now | prev) & 0x55555555u) << 1);
+    if (!inb || !((pair >> (threadIdx.x & 31)) & 1u)) return;
+    if (now == 0) {
 #pragma unroll
-            for (int c = 0; c < 8; ++c) __stcs(reinterpret_cast<uint4 *>(dst + c * plane), make_uint4(0u, 0u, 0u, 0u));
-        }
+        for (int c = 0; c < 8; ++c) __stcs(reinterpret_cast<uint4 *>(dst + c * plane), make_uint4(0u, 0u, 0u, 0u));
         return;
     }
-    if (!inb) return;
     float v[8][8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
@@ -329,7 +361,7 @@ cudaError_t launch_rebase_segments(int32_t *coords, int n_seg, int64_t rows_per_
 }
 
 cudaError_t launch_scatter_half(const float *feats, const int32_t *cell_row, int nb, int f, int nx, int ny, void *bev,
-                                cudaStream_t st)
+                                cudaStream_t st, const uint32_t *occ_prev, uint32_t *occ_next)
 {
     const int64_t plane = static_cast<int64_t>(nx) * ny;
     if (nb == 0 || plane == 0 || f == 0) return cudaSuccess;
@@ -339,12 +371,12 @@ cudaError_t launch_scatter_half(const float *feats, const int32_t *cell_row, int
     const int bs = 128;
     const int tpp = static_cast<int>((plane + bs * 8 - 1) / (bs * 8));
     const unsigned grid = static_cast<unsigned>(nb) * tpp * (f / 8);
-    k_scatter_wide_half<<<grid, bs, 0, st>>>(feats, cell_row, f, plane, tpp, static_cast<__half *>(bev));
+    k_scatter_wide_half<<<grid, bs, 0, st>>>(feats, cell_row, f, plane, tpp, static_cast<__half *>(bev), occ_prev, occ_next);
     note_launch();
     return cudaGetLastError();
 }
 cudaError_t launch_scatter(const float *feats, const int32_t *cell_row, int nb, int f, int nx, int ny, float *bev,
-                           int variant, cudaStream_t st)
+                           int variant, cudaStream_t st, const uint32_t *occ_prev, uint32_t *occ_next)
 {
     const int64_t plane = static_cast<int64_t>(nx) * ny;
     if (nb == 0 || plane == 0 || f == 0) return cudaSuccess;
@@ -360,11 +392,20 @@ cudaError_t launch_scatter(const float *feats, const int32_t *cell_row, int nb, 
         const unsigned grid = static_cast<unsigned>(nb) * tpp * (f / chan);
         static const bool cs = getenv("PILLARS_SCATTER_CS") != nullptr;
         const cudaError_t err = cs ? launch_pdl(k_scatter_wide<true, 8>, dim3(grid), dim3(bs), 0, st, feats, cell_row, f, plane,
-                                                tpp, chan, 0, bev)
+                                                tpp, chan, 0, bev, occ_prev, occ_next)
                                    : launch_pdl(k_scatter_wide<false, 8>, dim3(grid), dim3(bs), 0, st, feats, cell_row, f,
-                                                plane, tpp, chan, 0, bev);
+                                                plane, tpp, chan, 0, bev, occ_prev, occ_next);
         if (err != cudaSuccess) return err;
-    } else if (vec_ok) {
+        note_launch();
+        return cudaGetLastError();
+    }
+    // the plain kernel writes the whole canvas: the next call on it must not skip anything ("all dirty")
+    if (occ_next) {
+        const cudaError_t err = cudaMemsetAsync(occ_next, 0xFF, sizeof(uint32_t) * nb * occ_words(plane), st);
+        if (err != cudaSuccess) return err;
+        note_launch();
+    }
+    if (vec_ok) {
         const int tpp = static_cast<int>((plane + kThreads * 4 - 1) / (kThreads * 4));
         k_scatter_plain<true, 8, false><<<static_cast<unsigned>(nb) * tpp, kThreads, 0, st>>>(feats, cell_row, f, plane, tpp, bev);
     } else {

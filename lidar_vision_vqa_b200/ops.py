@@ -377,10 +377,11 @@ def encode_stack(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSp
         off = lib.pillars_workspace_cell_row_offset(n, nb, ctypes.byref(g))
         res["cell_row"] = buffers.ws[off:off + 4 * nb * ny * nx].view(torch.int32).view(nb, ny, nx)
     nat = stack.native()
-    check(lib.pillars_encode_stack(points.data_ptr(), n, stride, col0, frame_offsets.data_ptr(), nb, ctypes.byref(g),
-                                   ctypes.byref(nat), _native.MODE_DYNAMIC if dynamic else _native.MODE_HARD, coords_cols,
-                                   ctypes.byref(out), ws.data_ptr(), ws.numel(), SCATTER_VARIANTS[scatter_variant],
-                                   _stream_ptr()), "pillars_encode_stack")
+    mode = _native.MODE_DYNAMIC if dynamic else _native.MODE_HARD
+    variant, stream = SCATTER_VARIANTS[scatter_variant], _stream_ptr()
+    check(_encode_canvas(buffers if with_bev else None, lib, lambda: lib.pillars_encode_stack(
+        points.data_ptr(), n, stride, col0, frame_offsets.data_ptr(), nb, ctypes.byref(g), ctypes.byref(nat), mode,
+        coords_cols, ctypes.byref(out), ws.data_ptr(), ws.numel(), variant, stream)), "pillars_encode_stack")
     return res
 
 
@@ -420,7 +421,13 @@ def scatter_bev(pillar_features: torch.Tensor, coords: torch.Tensor, batch_size:
 
 class EncodeBuffers:
     """Pre-allocated outputs + workspace for repeated :func:`encode_bev` calls on same-shaped batches (no allocator
-    traffic inside a timed loop)."""
+    traffic inside a timed loop).
+
+    The BEV canvas is reused, and a canvas the library wrote last is mostly zeros already: the buffers keep two occupancy
+    bitmaps (pillars_set_canvas_occupancy) so that the next call writes only the cells that are or were occupied.  Writes
+    to ``bev`` through torch (in place, through views, ``out=``) are seen by its version counter and make the next call
+    write the whole canvas again.  Writes torch cannot see (raw pointers, DLPack, other native libraries) must be
+    followed by :meth:`invalidate_canvas` before the buffers are used again."""
 
     def __init__(self, n_points: int, n_frames: int, grid: GridSpec, f_out: int, device, *, with_bev: bool = True,
                  capacity: Optional[int] = None, ws_slot: int = 0, bev_dtype: torch.dtype = torch.float32,
@@ -446,11 +453,49 @@ class EncodeBuffers:
             self.voxel_coords = torch.empty((cap, 4), dtype=torch.int32, device=device)
             self.pillar_count = torch.empty((n_frames + 1,), dtype=torch.int32, device=device)
         self.voxel_num_points = torch.empty((cap,), dtype=torch.int32, device=device)
-        self.bev = torch.empty((n_frames, f_out * nz, ny, nx), dtype=bev_dtype, device=device) if with_bev else None
+        self.bev = None
+        if with_bev:
+            with torch.inference_mode(False):  # an inference tensor has no version counter
+                self.bev = torch.empty((n_frames, f_out * nz, ny, nx), dtype=bev_dtype, device=device)
+            # [2, n_frames, ceil(ny*nx / 256)] bitmaps, all dirty; the library reads [parity] and writes [1 - parity]
+            self._occupancy = torch.full((2, n_frames, (ny * nx + 255) // 256), -1, dtype=torch.int32, device=device)
+            self._parity = 0
+            self._canvas_version = self.bev._version  # of the library's last write; None: contents unknown
         g = grid.native()
         need = _native.load().pillars_workspace_bytes(n_points, n_frames, ctypes.byref(g))
         self.ws = torch.empty(need, dtype=torch.uint8, device=device)
         self.ws_slot = ws_slot
+
+    def invalidate_canvas(self) -> None:
+        """The next call writes the whole canvas: call after writing ``bev`` in a way torch's version counter does not
+        see."""
+        self._canvas_version = None
+
+    def _set_canvas_occupancy(self, lib) -> None:
+        """Hands the bitmaps to the next native call on this thread; immediately before that call."""
+        prev = self._occupancy[self._parity].data_ptr() if self._canvas_version == self.bev._version else None
+        check(lib.pillars_set_canvas_occupancy(prev, self._occupancy[1 - self._parity].data_ptr()),
+              "pillars_set_canvas_occupancy")
+
+    def _canvas_written(self, ok: bool) -> None:
+        if ok:
+            self._parity ^= 1
+            self._canvas_version = self.bev._version
+        else:
+            self._canvas_version = None
+
+
+def _encode_canvas(buffers: Optional[EncodeBuffers], lib, call) -> int:
+    """Runs the native `call` (returns its code) with the canvas occupancy of `buffers`, when it writes their canvas."""
+    if buffers is None:
+        return call()
+    buffers._set_canvas_occupancy(lib)
+    rc = 1
+    try:
+        rc = call()
+    finally:
+        buffers._canvas_written(rc == 0)
+    return rc
 
 
 def encode_bev(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, pfn: PfnParams, *, col0: int = 0,
@@ -487,6 +532,8 @@ def encode_bev(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec
     if with_bev:
         if buffers.bev is None:
             raise ValueError("buffers were created without a BEV canvas")
+        if buffers.n_frames != nb:
+            raise ValueError("buffers were created for another batch size")
         if buffers.bev.dtype == torch.float16:
             out.bev_half = buffers.bev.data_ptr()
         else:
@@ -507,9 +554,10 @@ def encode_bev(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec
         nx, ny, _ = grid.grid_size
         res["cell_row"] = buffers.ws[off:off + 4 * nb * ny * nx].view(torch.int32).view(nb, ny, nx)
     nat = pfn.native()
-    check(lib.pillars_encode_bev(points.data_ptr(), n, stride, col0, frame_offsets.data_ptr(), nb, ctypes.byref(g),
-                                 ctypes.byref(nat), ctypes.byref(out), buffers.ws.data_ptr(), buffers.ws.numel(),
-                                 SCATTER_VARIANTS[scatter_variant], _stream_ptr()), "pillars_encode_bev")
+    variant, stream = SCATTER_VARIANTS[scatter_variant], _stream_ptr()
+    check(_encode_canvas(buffers if with_bev else None, lib, lambda: lib.pillars_encode_bev(
+        points.data_ptr(), n, stride, col0, frame_offsets.data_ptr(), nb, ctypes.byref(g), ctypes.byref(nat),
+        ctypes.byref(out), buffers.ws.data_ptr(), buffers.ws.numel(), variant, stream)), "pillars_encode_bev")
     return res
 
 
