@@ -345,8 +345,9 @@ int pillars_set_canvas_occupancy(const uint32_t *prev, uint32_t *next);
  * NULL switches it off.  profiles/scripts/phase_times.py decodes it. */
 int pillars_set_debug_times(void *buffer32);
 
-/* Test / measurement hook: non-zero makes pillars_encode_bev ignore the host weight copies and run the generic feature
- * kernel (thread-local). */
+/* Test / measurement hook (thread-local): non-zero sends every call to the general feature kernel instead of the
+ * streaming one -- pillars_encode_bev to k_pillar_features, pillars_encode_stack to the general stack kernel,
+ * pillars_pfn_dense to the faithful padded kernel (pfn->folded is then ignored). */
 int pillars_force_generic_features(int on);
 
 #ifdef __cplusplus

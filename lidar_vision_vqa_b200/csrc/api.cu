@@ -3,7 +3,6 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -129,17 +128,23 @@ static bool stream_kernel_covers(const pillars_pfn_t &pfn)
     return pfn.use_absolute_xyz && !pfn.with_distance && pfn.c_point <= 5 && pfn.f_out == 64;
 }
 
-static PfnDev make_pfn_dev(const pillars_pfn_t &pfn, const float voxel[3])
+static PfnDev make_pfn_dev(const float *weight, const float *scale, const float *shift, const float offset[3],
+                           const float voxel[3])
 {
     PfnDev d;
-    d.weight = pfn.weight;
-    d.scale = pfn.scale;
-    d.shift = pfn.shift;
+    d.weight = weight;
+    d.scale = scale;
+    d.shift = shift;
     for (int i = 0; i < 3; ++i) {
-        d.off[i] = pfn.offset[i];
+        d.off[i] = offset[i];
         d.vsz[i] = voxel[i];
     }
     return d;
+}
+
+static PfnDev make_pfn_dev(const pillars_pfn_t &pfn, const float voxel[3])
+{
+    return make_pfn_dev(pfn.weight, pfn.scale, pfn.shift, pfn.offset, voxel);
 }
 
 }  // namespace pillars
@@ -219,118 +224,200 @@ int pillars_frame_offsets(const float *points_b, int64_t n, int32_t row_stride, 
     return 0;
 }
 
-static int group_and_emit(const float *points, int64_t n, int32_t row_stride, int32_t col0, int32_t c_point,
-                          const int32_t *frame_offsets, int32_t n_frames, const pillars_grid_t *grid,
-                          const pillars_pfn_t *pfn, const pillars_outputs_t *out, void *workspace, size_t workspace_bytes,
-                          bool want_bev, int scatter_variant, void *stream, CanvasOccupancy occ = {})
+// One call of the fused encoder, as its entry point normalised it.  The features are those of `pfn`
+// (pillars_encode_bev), of `stack` (pillars_encode_stack) or none (pillars_voxelize).
+struct EncodeCall {
+    const float *points;
+    int64_t n;
+    int stride, col0, c_point;
+    const int32_t *frame_offsets;
+    int nb;
+    const pillars_grid_t *grid;
+    const pillars_outputs_t *out;
+    void *workspace;
+    size_t workspace_bytes;
+    int scatter_variant;
+    void *stream;
+    CanvasOccupancy occ;
+    const pillars_pfn_t *pfn;  // checked by check_pfn
+    const StackDev *stack;     // checked by check_stack
+    bool dynamic;              // PILLARS_MODE_DYNAMIC
+    int coords_cols;
+};
+
+// Which kernels compute the per-pillar outputs of a call
+enum FeatureRoute {
+    kRouteEmit,    // k_emit_voxels only (pillars_voxelize)
+    kRoutePfn,     // the general one-layer kernel (pfn.cu)
+    kRouteMulti,   // the general stack kernel (pfn_multi.cu)
+    kRouteStream,  // the streaming kernel (pfn_stream.cu), on the point records the grouping emits
+};
+
+// The streaming kernel covers the mainstream configurations; everything else runs a general kernel.  For stacks these are
+// Waymo's own PFN, NUM_FILTERS [64, 64] (waymo_models/pointpillar_1x.yaml:34), and DynamicPillarVFE
+// (dynamic_pillar_vfe.py:14-142) with NUM_FILTERS [64] or [64, 64], in the standard feature layout.  A hard one-layer stack
+// and an empty batch stay on the general kernel.
+static FeatureRoute pick_route(const EncodeCall &c)
+{
+    if (!c.pfn && !c.stack) return kRouteEmit;
+    // (the streaming kernel's per-pillar record packs x and y into 16 bits each)
+    const bool stream_ok = !g_force_generic && c.grid->grid[0] <= 0xFFFF && c.grid->grid[1] <= 0xFFFF;
+    if (c.pfn) return stream_ok && stream_kernel_covers(*c.pfn) ? kRouteStream : kRoutePfn;
+    const StackDev &s = *c.stack;
+    const bool layers = s.n_layers == 2 ? s.out[0] == 32 && s.out[1] == 64 : c.dynamic && s.out[0] == 64;
+    const bool covered = layers && s.layout == PILLARS_LAYOUT_PILLAR_VFE && s.use_abs && !s.with_dist && c.c_point <= 5 &&
+                         c.coords_cols == 4 && c.n > 0;
+    return stream_ok && covered ? kRouteStream : kRouteMulti;
+}
+
+// What the three entry points share: the common checks, then grouping -> (dynamic rows) -> (fold) -> features -> scatter.
+static int encode(const EncodeCall &c)
 {
     g_launches = 0;
+    const pillars_grid_t *grid = c.grid;
+    const pillars_outputs_t *out = c.out;
     int rc;
-    if ((rc = check_grid(grid, n_frames))) return rc;
-    if (occ.next && out && out->bev && out->bev_half)
-        return fail(PILLARS_E_BADARG, "canvas occupancy is set but the call writes both bev and bev_half");
-    if ((rc = check_points(points, n, row_stride, col0, c_point))) return rc;
-    if (!frame_offsets || !out) return fail(PILLARS_E_BADARG, "frame_offsets / out is NULL");
-    if (n > 0 && n_frames == 0) return fail(PILLARS_E_BADARG, "n_points = %lld with n_frames = 0", (long long)n);
-    if (pfn && (rc = check_pfn(pfn))) return rc;
-    if (pfn && pfn->c_point != c_point) return fail(PILLARS_E_BADARG, "pfn->c_point != c_point");
-    if (pfn && !out->pillar_features) return fail(PILLARS_E_BADARG, "pillar_features output is required");
-    if (want_bev && ((!out->bev && !out->bev_half) || !pfn)) return fail(PILLARS_E_BADARG, "bev output / pfn missing");
-    if ((want_bev || out->want_index_map) && grid->grid[2] != 1) return fail(PILLARS_E_UNSUPPORTED, "BEV scatter / index map needs nz == 1");
+    if ((rc = check_grid(grid, c.nb))) return rc;
+    if ((rc = check_points(c.points, c.n, c.stride, c.col0, c.c_point))) return rc;
+    if (!c.frame_offsets || !out) return fail(PILLARS_E_BADARG, "frame_offsets / out is NULL");
+    if (c.n > 0 && c.nb == 0) return fail(PILLARS_E_BADARG, "n_points = %lld with n_frames = 0", (long long)c.n);
+    const bool features = c.pfn || c.stack;
+    if (features && !out->pillar_features) return fail(PILLARS_E_BADARG, "pillar_features output is required");
     if (out->pillar_capacity < 0) return fail(PILLARS_E_BADARG, "pillar_capacity < 0");
-    const int64_t cells_xy = static_cast<int64_t>(grid->grid[0]) * grid->grid[1];
-    if (!workspace || reinterpret_cast<uintptr_t>(workspace) % 256 != 0)
+    if (c.occ.next && out->bev && out->bev_half)
+        return fail(PILLARS_E_BADARG, "canvas occupancy is set but the call writes both bev and bev_half");
+    const bool want_bev = features && (out->bev || out->bev_half);
+    const bool want_map = want_bev || out->want_index_map;
+    if (want_map && grid->grid[2] != 1) return fail(PILLARS_E_UNSUPPORTED, "BEV scatter / index map needs nz == 1");
+    if (!c.workspace || reinterpret_cast<uintptr_t>(c.workspace) % 256 != 0)
         return fail(PILLARS_E_WORKSPACE, "workspace NULL or not 256-byte aligned");
+    const int64_t cells_xy = static_cast<int64_t>(grid->grid[0]) * grid->grid[1];
     const int64_t cells = cells_xy * grid->grid[2];
-    const Workspace ws = carve_workspace(workspace, n, n_frames, cells_xy, cells,
-                                         resolve_group_mode(true, n, n_frames, cells));
-    if (ws.total_bytes > workspace_bytes)
-        return fail(PILLARS_E_WORKSPACE, "workspace has %zu bytes, %zu needed", workspace_bytes, ws.total_bytes);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const GridDev gd = make_grid_dev(*grid);
+    // the dynamic variant ranks the cells of the dense index-map region itself: it keeps the hash table
+    const Workspace ws = carve_workspace(c.workspace, c.n, c.nb, cells_xy, cells,
+                                         resolve_group_mode(!c.dynamic, c.n, c.nb, cells));
+    if (ws.total_bytes > c.workspace_bytes)
+        return fail(PILLARS_E_WORKSPACE, "workspace has %zu bytes, %zu needed", c.workspace_bytes, ws.total_bytes);
+
+    cudaStream_t st = static_cast<cudaStream_t>(c.stream);
+    GridDev gd = make_grid_dev(*grid);
+    if (c.dynamic) {
+        gd.ignore_z = 1;
+        gd.max_points = 0x7FFFFFFF;
+        gd.max_voxels = 0x7FFFFFFF;
+    }
+    const FeatureRoute route = pick_route(c);
+    const bool membership = out->voxels || out->point_pillar || out->point_slot;
+    const int idx_bits = idx_bits_for(c.n > 1 ? c.n : 2);
+    // layer 0; its offset and voxel size also place the pillar centres for the grouping and the streaming kernel
+    PfnDev l0{};
+    if (c.pfn) l0 = make_pfn_dev(*c.pfn, grid->voxel);
+    if (c.stack) l0 = make_pfn_dev(c.stack->weight[0], c.stack->scale[0], c.stack->shift[0], c.stack->off, c.stack->vsz);
     cudaError_t e;
     stage_mark(0, st);
 
-    if (out->point_pillar && n > 0) {
-        if ((e = cudaMemsetAsync(out->point_pillar, 0xFF, sizeof(int32_t) * n, st)) != cudaSuccess) return cuda_fail(e, "memset");
+    if (out->point_pillar && c.n > 0) {
+        if ((e = cudaMemsetAsync(out->point_pillar, 0xFF, sizeof(int32_t) * c.n, st)) != cudaSuccess) return cuda_fail(e, "memset");
         note_launch();
     }
-    if (out->point_slot && n > 0) {
-        if ((e = cudaMemsetAsync(out->point_slot, 0xFF, sizeof(int32_t) * n, st)) != cudaSuccess) return cuda_fail(e, "memset");
+    if (out->point_slot && c.n > 0) {
+        if ((e = cudaMemsetAsync(out->point_slot, 0xFF, sizeof(int32_t) * c.n, st)) != cudaSuccess) return cuda_fail(e, "memset");
         note_launch();
     }
-    // Feature kernel choice.  The streaming kernel covers the mainstream configuration; everything else runs the generic
-    // 16-lanes-per-pillar kernel.
-    const bool membership = out->voxels || out->point_pillar || out->point_slot;
-    // (the streaming kernel's per-pillar record packs x and y into 16 bits each)
-    const bool fast = pfn && stream_kernel_covers(*pfn) && !g_force_generic && grid->grid[0] <= 0xFFFF && grid->grid[1] <= 0xFFFF;
     PlaceExtras px{};
-    px.records = fast;
-    if (fast) {
-        for (int i = 0; i < 3; ++i) {
-            px.vsz[i] = grid->voxel[i];
-            px.off[i] = pfn->offset[i];
-        }
-        px.voxel_coords = out->voxel_coords;
-        px.voxel_num_points = out->voxel_num_points;
-        px.write_cell_row = want_bev || out->want_index_map;
-    }
+    px.records = route == kRouteStream;
     px.capacity = out->pillar_capacity;
-    if ((e = launch_group_points(points, n, row_stride, col0, c_point, frame_offsets, n_frames, gd, ws, out->pillar_count,
-                                 /*want_index_lists=*/membership || !fast, px, st)) != cudaSuccess)
+    if (px.records) {
+        for (int i = 0; i < 3; ++i) {
+            px.vsz[i] = l0.vsz[i];
+            px.off[i] = l0.off[i];
+        }
+        if (!c.dynamic) {  // (launch_dynamic_rows writes these for the dynamic variant)
+            px.voxel_coords = out->voxel_coords;
+            px.voxel_num_points = out->voxel_num_points;
+            px.write_cell_row = want_map;
+        }
+    }
+    if ((e = launch_group_points(c.points, c.n, c.stride, c.col0, c.c_point, c.frame_offsets, c.nb, gd, ws, out->pillar_count,
+                                 /*want_index_lists=*/membership || route != kRouteStream, px, st)) != cudaSuccess)
         return cuda_fail(e, "group_points");
     stage_mark(1, st);
 
-    FeatureJob job{};
-    job.points = points;
-    job.n = n;
-    job.stride = row_stride;
-    job.col0 = col0;
-    job.c_point = c_point;
-    job.nb = n_frames;
-    job.idx_bits = idx_bits_for(n > 1 ? n : 2);
-    job.do_features = pfn != nullptr && !fast;
-    if (pfn) {
-        job.use_abs = pfn->use_absolute_xyz != 0;
-        job.with_dist = pfn->with_distance != 0;
-        job.pfn = make_pfn_dev(*pfn, grid->voxel);
-        job.c_in = pfn->c_in;
-        job.f_out = pfn->f_out;
-    }
-    job.out = *out;
-    job.write_cell_row = (want_bev || out->want_index_map) && !fast;
-    if (!fast || membership) {
+    // membership outputs (pillars_voxelize, pillars_encode_bev) come from k_emit_voxels, whatever computes the features
+    if (route == kRouteEmit || route == kRoutePfn || membership) {
+        FeatureJob job{};
+        job.points = c.points;
+        job.n = c.n;
+        job.stride = c.stride;
+        job.col0 = c.col0;
+        job.c_point = c.c_point;
+        job.nb = c.nb;
+        job.idx_bits = idx_bits;
+        job.do_features = route == kRoutePfn;
+        if (c.pfn) {
+            job.use_abs = c.pfn->use_absolute_xyz != 0;
+            job.with_dist = c.pfn->with_distance != 0;
+        }
+        job.pfn = l0;
+        job.out = *out;
+        job.write_cell_row = want_map && route != kRouteStream;
         if ((e = launch_pillar_features(job, gd, ws, st)) != cudaSuccess) return cuda_fail(e, "pillar_features");
     }
-    if (fast) {
-        const float *folded = pfn->folded;
+    if (route == kRouteStream) {
+        // the dynamic variant's pillar entries get their rows (sorted-key order) between the grouping and the feature kernel
+        if (c.dynamic &&
+            (e = launch_dynamic_rows(gd, ws, c.nb, c.n, out->pillar_capacity, out->voxel_coords, out->voxel_num_points, st)) != cudaSuccess)
+            return cuda_fail(e, "dynamic_rows");
+        const bool two = c.stack && c.stack->n_layers == 2;
+        const float *folded = c.pfn ? c.pfn->folded : nullptr;
         if (!folded) {  // the caller did not prepare the table: fold into the workspace (one more single-block launch)
-            if ((e = launch_fold_pfn(job.pfn, pfn->c_point, pfn->c_in, ws.folded, st)) != cudaSuccess)
+            const int c_in = c.pfn ? c.pfn->c_in : stack_c_in(*c.stack, c.c_point);
+            if ((e = launch_fold_pfn(l0, c.c_point, c_in, ws.folded, st, two ? 32 : 64)) != cudaSuccess)
                 return cuda_fail(e, "fold_pfn");
             folded = ws.folded;
         }
+        if (two && (e = launch_fold_pfn2(c.stack->weight[1], c.stack->scale[1], c.stack->shift[1], ws.folded2, st)) != cudaSuccess)
+            return cuda_fail(e, "fold_pfn2");
         FastJob fj{};
-        fj.n = n;
-        fj.idx_bits = job.idx_bits;
+        fj.dynamic = c.dynamic;
+        fj.n = c.n;
+        fj.idx_bits = idx_bits;
         fj.pillar_features = out->pillar_features;
+        fj.folded2 = two ? ws.folded2 : nullptr;
         for (int i = 0; i < 3; ++i) {
-            fj.vsz[i] = grid->voxel[i];
-            fj.off[i] = pfn->offset[i];
+            fj.vsz[i] = l0.vsz[i];
+            fj.off[i] = l0.off[i];
         }
         if ((e = launch_pillar_features_stream(fj, folded, gd, ws, st)) != cudaSuccess)
             return cuda_fail(e, "pillar_features_stream");
     }
+    if (route == kRouteMulti) {
+        MultiJob job{};
+        job.points = c.points;
+        job.n = c.n;
+        job.stride = c.stride;
+        job.col0 = c.col0;
+        job.c_point = c.c_point;
+        job.nb = c.nb;
+        job.idx_bits = idx_bits;
+        job.dynamic = c.dynamic;
+        job.write_cell_row = want_map;
+        job.pillar_features = out->pillar_features;
+        job.voxel_coords = out->voxel_coords;
+        job.voxel_num_points = out->voxel_num_points;
+        job.coords_cols = c.coords_cols;
+        job.capacity = out->pillar_capacity;
+        if ((e = launch_pfn_multi_lists(job, *c.stack, gd, ws, st)) != cudaSuccess) return cuda_fail(e, "pfn_multi");
+    }
     stage_mark(2, st);
 
     if (want_bev) {
-        cudaStream_t sst = st;
-        if (out->bev &&
-            (e = launch_scatter(out->pillar_features, ws.cell_row, n_frames, pfn->f_out, grid->grid[0], grid->grid[1],
-                                out->bev, scatter_variant, sst, occ.prev, occ.next)) != cudaSuccess)
+        const int f = c.pfn ? c.pfn->f_out : c.stack->out[c.stack->n_layers - 1];
+        if (out->bev && (e = launch_scatter(out->pillar_features, ws.cell_row, c.nb, f, grid->grid[0], grid->grid[1], out->bev,
+                                            c.scatter_variant, st, c.occ.prev, c.occ.next)) != cudaSuccess)
             return cuda_fail(e, "scatter");
-        if (out->bev_half &&
-            (e = launch_scatter_half(out->pillar_features, ws.cell_row, n_frames, pfn->f_out, grid->grid[0],
-                                     grid->grid[1], out->bev_half, sst, occ.prev, occ.next)) != cudaSuccess)
+        if (out->bev_half && (e = launch_scatter_half(out->pillar_features, ws.cell_row, c.nb, f, grid->grid[0], grid->grid[1],
+                                                      out->bev_half, st, c.occ.prev, c.occ.next)) != cudaSuccess)
             return cuda_fail(e, "scatter (float16 canvas: needs nx*ny % 8 == 0, f % 8 == 0)");
     }
     stage_mark(3, st);
@@ -356,8 +443,8 @@ int pillars_voxelize(const float *points, int64_t n, int32_t row_stride, int32_t
                      const int32_t *frame_offsets, int32_t n_frames, const pillars_grid_t *grid,
                      const pillars_outputs_t *out, void *workspace, size_t workspace_bytes, void *stream)
 {
-    return group_and_emit(points, n, row_stride, col0, c_point, frame_offsets, n_frames, grid, nullptr, out, workspace,
-                          workspace_bytes, false, 0, stream);
+    return encode({points, n, row_stride, col0, c_point, frame_offsets, n_frames, grid, out, workspace, workspace_bytes, 0,
+                   stream});
 }
 
 int pillars_encode_bev(const float *points, int64_t n, int32_t row_stride, int32_t col0, const int32_t *frame_offsets,
@@ -366,10 +453,10 @@ int pillars_encode_bev(const float *points, int64_t n, int32_t row_stride, int32
                        void *stream)
 {
     const CanvasOccupancy occ = take_canvas_occupancy();
-    if (!pfn) return fail(PILLARS_E_BADARG, "pfn is NULL");
-    return group_and_emit(points, n, row_stride, col0, pfn->c_point, frame_offsets, n_frames, grid, pfn, out, workspace,
-                          workspace_bytes, out && (out->bev != nullptr || out->bev_half != nullptr), scatter_variant, stream,
-                          occ);
+    int rc;
+    if ((rc = check_pfn(pfn))) return rc;
+    return encode({points, n, row_stride, col0, pfn->c_point, frame_offsets, n_frames, grid, out, workspace, workspace_bytes,
+                   scatter_variant, stream, occ, pfn});
 }
 
 int pillars_pfn_dense(const float *voxels, const void *num_points, int32_t num_points_is_float, const void *coords,
@@ -391,8 +478,8 @@ int pillars_pfn_dense(const float *voxels, const void *num_points, int32_t num_p
                         ? launch_pfn_padded(voxels, num_points, num_points_is_float != 0, coords, coords_is_float != 0, m,
                                             max_points, pfn->c_point, pd, pfn->folded, out, static_cast<cudaStream_t>(stream))
                         : launch_pfn_dense(voxels, num_points, num_points_is_float != 0, coords, coords_is_float != 0, m,
-                                           max_points, pfn->c_point, pfn->c_in, pfn->f_out, pfn->use_absolute_xyz != 0,
-                                           pfn->with_distance != 0, pd, out, static_cast<cudaStream_t>(stream));
+                                           max_points, pfn->c_point, pfn->use_absolute_xyz != 0, pfn->with_distance != 0, pd,
+                                           out, static_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) return cuda_fail(e, "pillars_pfn_dense");
     g_launches_last = g_launches;
     return 0;
@@ -464,162 +551,56 @@ int pillars_encode_stack(const float *points, int64_t n, int32_t row_stride, int
                          int32_t scatter_variant, void *stream)
 {
     const CanvasOccupancy occ = take_canvas_occupancy();
-    g_launches = 0;
-    int rc;
-    if ((rc = check_grid(grid, n_frames))) return rc;
     StackDev sd{};
-    if ((rc = check_stack(stack, &sd, grid->voxel))) return rc;
-    if ((rc = check_points(points, n, row_stride, col0, stack->c_point))) return rc;
+    int rc;
+    if ((rc = check_stack(stack, &sd, grid ? grid->voxel : nullptr))) return rc;
     if (mode != PILLARS_MODE_HARD && mode != PILLARS_MODE_DYNAMIC) return fail(PILLARS_E_BADARG, "mode = %d", mode);
     if (coords_cols != 3 && coords_cols != 4) return fail(PILLARS_E_BADARG, "coords_cols = %d", coords_cols);
-    if (!frame_offsets || !out || !out->pillar_features) return fail(PILLARS_E_BADARG, "frame_offsets / out / pillar_features NULL");
-    if (out->voxels || out->point_pillar || out->point_slot)
-        return fail(PILLARS_E_UNSUPPORTED, "membership outputs come from pillars_voxelize");
     const bool dynamic = mode == PILLARS_MODE_DYNAMIC;
-    const bool want_bev = out->bev != nullptr || out->bev_half != nullptr;
-    if (occ.next && out->bev && out->bev_half)
-        return fail(PILLARS_E_BADARG, "canvas occupancy is set but the call writes both bev and bev_half");
-    if ((want_bev || out->want_index_map) && (dynamic || grid->grid[2] != 1 || coords_cols != 4))
-        return fail(PILLARS_E_UNSUPPORTED, "the fused BEV canvas / index map needs mode HARD, nz == 1 and 4-column coords");
-    if (out->pillar_capacity < 0) return fail(PILLARS_E_BADARG, "pillar_capacity < 0");
-    const int64_t cells_xy = static_cast<int64_t>(grid->grid[0]) * grid->grid[1];
-    if (!workspace || reinterpret_cast<uintptr_t>(workspace) % 256 != 0)
-        return fail(PILLARS_E_WORKSPACE, "workspace NULL or not 256-byte aligned");
-    if (n > 0 && n_frames == 0) return fail(PILLARS_E_BADARG, "n_points = %lld with n_frames = 0", (long long)n);
-    const int64_t cells = cells_xy * grid->grid[2];
-    // the dynamic variant ranks the cells of the dense index-map region itself: it keeps the hash table
-    const Workspace ws = carve_workspace(workspace, n, n_frames, cells_xy, cells,
-                                         resolve_group_mode(!dynamic, n, n_frames, cells));
-    if (ws.total_bytes > workspace_bytes)
-        return fail(PILLARS_E_WORKSPACE, "workspace has %zu bytes, %zu needed", workspace_bytes, ws.total_bytes);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    GridDev gd = make_grid_dev(*grid);
-    if (dynamic) {
-        gd.ignore_z = 1;
-        gd.max_points = 0x7FFFFFFF;
-        gd.max_voxels = 0x7FFFFFFF;
-    }
-    cudaError_t e;
-    stage_mark(0, st);
-    // Waymo's own PFN, NUM_FILTERS [64, 64] (waymo_models/pointpillar_1x.yaml:34), in the mainstream feature layout: the
-    // streaming kernel's two-layer variant (records grouped by the placement stage, as in pillars_encode_bev) replaces the
-    // general kernel below.  PILLARS_STACK_FAST=0 keeps the general kernel (A/B measurements).
-    static const bool fast_env = !(getenv("PILLARS_STACK_FAST") && atoi(getenv("PILLARS_STACK_FAST")) == 0);
-    const bool fast2 = fast_env && !dynamic && sd.n_layers == 2 && sd.out[0] == 32 && sd.out[1] == 64 && sd.layout == 0 &&
-                       sd.use_abs && !sd.with_dist && stack->c_point <= 5 && coords_cols == 4 && grid->grid[0] <= 0xFFFF &&
-                       grid->grid[1] <= 0xFFFF && n > 0;
-    // DynamicPillarVFE (dynamic_pillar_vfe.py:14-142) with NUM_FILTERS [64] or [64, 64] in the standard layout: the same
-    // streaming kernels in their dynamic variant; the pillar entries get their rows (sorted-key order) from
-    // launch_dynamic_rows between the grouping and the feature kernel.
-    const bool fast_dyn = fast_env && dynamic && sd.layout == 0 && sd.use_abs && !sd.with_dist && stack->c_point <= 5 &&
-                          coords_cols == 4 && grid->grid[0] <= 0xFFFF && grid->grid[1] <= 0xFFFF && n > 0 &&
-                          ((sd.n_layers == 1 && sd.out[0] == 64) || (sd.n_layers == 2 && sd.out[0] == 32 && sd.out[1] == 64));
-    PlaceExtras px{};
-    px.capacity = out->pillar_capacity;
-    if (fast_dyn) {
-        px.records = true;
-        for (int i = 0; i < 3; ++i) {
-            px.vsz[i] = grid->voxel[i];
-            px.off[i] = sd.off[i];
-        }
-    }
-    if (fast2) {
-        px.records = true;
-        for (int i = 0; i < 3; ++i) {
-            px.vsz[i] = grid->voxel[i];
-            px.off[i] = sd.off[i];
-        }
-        px.voxel_coords = out->voxel_coords;
-        px.voxel_num_points = out->voxel_num_points;
-        px.write_cell_row = want_bev || out->want_index_map;
-    }
-    if ((e = launch_group_points(points, n, row_stride, col0, stack->c_point, frame_offsets, n_frames, gd, ws,
-                                 out->pillar_count, /*want_index_lists=*/!fast2 && !fast_dyn, px, st)) != cudaSuccess)
-        return cuda_fail(e, "group_points");
-    stage_mark(1, st);
-    if (fast_dyn &&
-        (e = launch_dynamic_rows(gd, ws, n_frames, n, out->pillar_capacity, out->voxel_coords, out->voxel_num_points, st)) != cudaSuccess)
-        return cuda_fail(e, "dynamic_rows");
-    if (fast2 || fast_dyn) {
-        const bool two = sd.n_layers == 2;
-        PfnDev l0{};
-        l0.weight = sd.weight[0];
-        l0.scale = sd.scale[0];
-        l0.shift = sd.shift[0];
-        for (int i = 0; i < 3; ++i) {
-            l0.off[i] = sd.off[i];
-            l0.vsz[i] = sd.vsz[i];
-        }
-        if ((e = launch_fold_pfn(l0, stack->c_point, stack_c_in(sd, stack->c_point), ws.folded, st, two ? 32 : 64)) != cudaSuccess)
-            return cuda_fail(e, "fold_pfn");
-        if (two && (e = launch_fold_pfn2(sd.weight[1], sd.scale[1], sd.shift[1], ws.folded2, st)) != cudaSuccess)
-            return cuda_fail(e, "fold_pfn2");
-        FastJob fj{};
-        fj.dynamic = fast_dyn;
-        fj.n = n;
-        fj.idx_bits = idx_bits_for(n > 1 ? n : 2);
-        fj.pillar_features = out->pillar_features;
-        fj.folded2 = two ? ws.folded2 : nullptr;
-        for (int i = 0; i < 3; ++i) {
-            fj.vsz[i] = grid->voxel[i];
-            fj.off[i] = sd.off[i];
-        }
-        if ((e = launch_pillar_features_stream(fj, ws.folded, gd, ws, st)) != cudaSuccess)
-            return cuda_fail(e, "pillar_features_stream (stack)");
-    }
-    MultiJob job{};
-    job.points = points;
-    job.n = n;
-    job.stride = row_stride;
-    job.col0 = col0;
-    job.c_point = stack->c_point;
-    job.nb = n_frames;
-    job.idx_bits = idx_bits_for(n > 1 ? n : 2);
-    job.dynamic = dynamic;
-    job.write_cell_row = want_bev || out->want_index_map;
-    job.pillar_features = out->pillar_features;
-    job.voxel_coords = out->voxel_coords;
-    job.voxel_num_points = out->voxel_num_points;
-    job.coords_cols = coords_cols;
-    job.capacity = out->pillar_capacity;
-    if (!fast2 && !fast_dyn && (e = launch_pfn_multi_lists(job, sd, gd, ws, st)) != cudaSuccess)
-        return cuda_fail(e, "pfn_multi");
-    stage_mark(2, st);
-    if (want_bev) {
-        const int f_last = sd.out[sd.n_layers - 1];
-        if (out->bev && (e = launch_scatter(out->pillar_features, ws.cell_row, n_frames, f_last, grid->grid[0],
-                                            grid->grid[1], out->bev, scatter_variant, st, occ.prev, occ.next)) != cudaSuccess)
-            return cuda_fail(e, "scatter");
-        if (out->bev_half && (e = launch_scatter_half(out->pillar_features, ws.cell_row, n_frames, f_last, grid->grid[0],
-                                                      grid->grid[1], out->bev_half, st, occ.prev, occ.next)) != cudaSuccess)
-            return cuda_fail(e, "scatter (float16 canvas)");
-    }
-    stage_mark(3, st);
-    g_launches_last = g_launches;
-    return 0;
+    if (out && (out->voxels || out->point_pillar || out->point_slot))
+        return fail(PILLARS_E_UNSUPPORTED, "membership outputs come from pillars_voxelize");
+    if (out && (out->bev || out->bev_half || out->want_index_map) && (dynamic || coords_cols != 4))
+        return fail(PILLARS_E_UNSUPPORTED, "the fused BEV canvas / index map needs mode HARD and 4-column coords");
+    return encode({points, n, row_stride, col0, stack->c_point, frame_offsets, n_frames, grid, out, workspace, workspace_bytes,
+                   scatter_variant, stream, occ, nullptr, &sd, dynamic, coords_cols});
+}
+
+// What pillars_scatter_bev and pillars_scatter_bev_half share: the argument checks and the index map, built in the
+// workspace.  *cell_row stays NULL when there is nothing to scatter (n_frames == 0).
+static int scatter_cell_row(bool half, const float *feats, const void *coords, int32_t coords_is_float, int64_t m,
+                            const int32_t *m_dev, int32_t n_frames, int32_t f, int32_t nx, int32_t ny, int32_t nz,
+                            const void *canvas, void *workspace, size_t workspace_bytes, cudaStream_t st, int32_t **cell_row)
+{
+    g_launches = 0;
+    *cell_row = nullptr;
+    const char *what = half ? "pillars_scatter_bev_half" : "pillars_scatter_bev";
+    if (m < 0 || n_frames < 0 || f < 1 || nx < 1 || ny < 1 || nz < 1) return fail(PILLARS_E_BADARG, "%s: bad size", what);
+    if (n_frames > 0 && !canvas) return fail(PILLARS_E_BADARG, "%s: canvas is NULL", what);
+    if (m > 0 && (!feats || !coords)) return fail(PILLARS_E_BADARG, "feats / coords NULL");
+    if (m > 0 && reinterpret_cast<uintptr_t>(coords) % 16 != 0) return fail(PILLARS_E_BADARG, "coords must be 16-byte aligned");
+    if (half && ((static_cast<int64_t>(nx) * ny * nz) % 8 != 0 || f % 8 != 0))
+        return fail(PILLARS_E_UNSUPPORTED, "float16 canvas needs nx*ny*nz %% 8 == 0 and f %% 8 == 0");
+    const size_t need = sizeof(int32_t) * static_cast<size_t>(n_frames) * nx * ny * nz;
+    if (need > 0 && (!workspace || workspace_bytes < need || reinterpret_cast<uintptr_t>(workspace) % 16 != 0))
+        return fail(PILLARS_E_WORKSPACE, "workspace has %zu bytes, %zu needed", workspace_bytes, need);
+    if (n_frames == 0) return 0;
+    *cell_row = static_cast<int32_t *>(workspace);
+    const cudaError_t e = launch_build_cell_row(coords, coords_is_float != 0, m, m_dev, n_frames, nx, ny, nz, *cell_row, st);
+    return e == cudaSuccess ? 0 : cuda_fail(e, "build_cell_row");
 }
 
 int pillars_scatter_bev(const float *feats, const void *coords, int32_t coords_is_float, int64_t m, const int32_t *m_dev,
                         int32_t n_frames, int32_t f, int32_t nx, int32_t ny, int32_t nz, float *bev, void *workspace,
                         size_t workspace_bytes, int32_t variant, void *stream)
 {
-    g_launches = 0;
-    if (m < 0 || n_frames < 0 || f < 1 || nx < 1 || ny < 1 || nz < 1) return fail(PILLARS_E_BADARG, "pillars_scatter_bev: bad size");
-    if (n_frames > 0 && !bev) return fail(PILLARS_E_BADARG, "bev is NULL");
-    if (m > 0 && (!feats || !coords)) return fail(PILLARS_E_BADARG, "feats / coords NULL");
-    if (m > 0 && reinterpret_cast<uintptr_t>(coords) % 16 != 0) return fail(PILLARS_E_BADARG, "coords must be 16-byte aligned");
-    const size_t need = sizeof(int32_t) * static_cast<size_t>(n_frames) * nx * ny * nz;
-    if (need > 0 && (!workspace || workspace_bytes < need || reinterpret_cast<uintptr_t>(workspace) % 16 != 0))
-        return fail(PILLARS_E_WORKSPACE, "workspace has %zu bytes, %zu needed", workspace_bytes, need);
-    if (n_frames == 0) return 0;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    int32_t *cell_row = static_cast<int32_t *>(workspace);
-    cudaError_t e;
-    if ((e = launch_build_cell_row(coords, coords_is_float != 0, m, m_dev, n_frames, nx, ny, nz, cell_row, st)) != cudaSuccess)
-        return cuda_fail(e, "build_cell_row");
+    int32_t *cell_row;
+    const int rc = scatter_cell_row(false, feats, coords, coords_is_float, m, m_dev, n_frames, f, nx, ny, nz, bev, workspace,
+                                    workspace_bytes, st, &cell_row);
+    if (rc || !cell_row) return rc;
     // the canvas of the 3-D variant is the 2-D one with nz*ny rows per channel
-    if ((e = launch_scatter(feats, cell_row, n_frames, f, nx, ny * nz, bev, variant, st)) != cudaSuccess)
-        return cuda_fail(e, "scatter");
+    const cudaError_t e = launch_scatter(feats, cell_row, n_frames, f, nx, ny * nz, bev, variant, st);
+    if (e != cudaSuccess) return cuda_fail(e, "scatter");
     g_launches_last = g_launches;
     return 0;
 }
@@ -645,24 +626,13 @@ int pillars_scatter_bev_half(const float *feats, const void *coords, int32_t coo
                              const int32_t *m_dev, int32_t n_frames, int32_t f, int32_t nx, int32_t ny, int32_t nz,
                              void *bev_half, void *workspace, size_t workspace_bytes, void *stream)
 {
-    g_launches = 0;
-    if (m < 0 || n_frames < 0 || f < 1 || nx < 1 || ny < 1 || nz < 1) return fail(PILLARS_E_BADARG, "pillars_scatter_bev_half: bad size");
-    if (n_frames > 0 && !bev_half) return fail(PILLARS_E_BADARG, "bev_half is NULL");
-    if (m > 0 && (!feats || !coords)) return fail(PILLARS_E_BADARG, "feats / coords NULL");
-    if (m > 0 && reinterpret_cast<uintptr_t>(coords) % 16 != 0) return fail(PILLARS_E_BADARG, "coords must be 16-byte aligned");
-    if ((static_cast<int64_t>(nx) * ny * nz) % 8 != 0 || f % 8 != 0)
-        return fail(PILLARS_E_UNSUPPORTED, "float16 canvas needs nx*ny*nz %% 8 == 0 and f %% 8 == 0");
-    const size_t need = sizeof(int32_t) * static_cast<size_t>(n_frames) * nx * ny * nz;
-    if (need > 0 && (!workspace || workspace_bytes < need || reinterpret_cast<uintptr_t>(workspace) % 16 != 0))
-        return fail(PILLARS_E_WORKSPACE, "workspace has %zu bytes, %zu needed", workspace_bytes, need);
-    if (n_frames == 0) return 0;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    int32_t *cell_row = static_cast<int32_t *>(workspace);
-    cudaError_t e;
-    if ((e = launch_build_cell_row(coords, coords_is_float != 0, m, m_dev, n_frames, nx, ny, nz, cell_row, st)) != cudaSuccess)
-        return cuda_fail(e, "build_cell_row");
-    if ((e = launch_scatter_half(feats, cell_row, n_frames, f, nx, ny * nz, bev_half, st)) != cudaSuccess)
-        return cuda_fail(e, "scatter (float16 canvas)");
+    int32_t *cell_row;
+    const int rc = scatter_cell_row(true, feats, coords, coords_is_float, m, m_dev, n_frames, f, nx, ny, nz, bev_half,
+                                    workspace, workspace_bytes, st, &cell_row);
+    if (rc || !cell_row) return rc;
+    const cudaError_t e = launch_scatter_half(feats, cell_row, n_frames, f, nx, ny * nz, bev_half, st);
+    if (e != cudaSuccess) return cuda_fail(e, "scatter (float16 canvas)");
     g_launches_last = g_launches;
     return 0;
 }

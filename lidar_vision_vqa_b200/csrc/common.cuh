@@ -303,8 +303,6 @@ struct FeatureJob {
     bool with_dist;
     bool do_features;          // run the PFN (needs pfn + pillar_features)
     PfnDev pfn;
-    int c_in;
-    int f_out;
     pillars_outputs_t out;     // by value; NULL members are skipped
     bool write_cell_row;       // fill ws.cell_row for the BEV scatter
 };
@@ -333,8 +331,8 @@ cudaError_t launch_pillar_features_stream(const FastJob &job, const float *folde
                                           cudaStream_t st);
 
 cudaError_t launch_pfn_dense(const float *voxels, const void *num_points, bool np_float, const void *coords,
-                             bool coords_float, int64_t m, int max_points, int c_point, int c_in, int f_out,
-                             bool use_abs, bool with_dist, const PfnDev &pfn, float *out, cudaStream_t st);
+                             bool coords_float, int64_t m, int max_points, int c_point, bool use_abs, bool with_dist,
+                             const PfnDev &pfn, float *out, cudaStream_t st);
 
 // ---- general feature stack (pfn_multi.cu) -----------------------------------------------------
 struct StackDev {

@@ -483,11 +483,9 @@ cudaError_t launch_pillar_features(const FeatureJob &job, const GridDev &gd, con
 }
 
 cudaError_t launch_pfn_dense(const float *voxels, const void *num_points, bool np_float, const void *coords,
-                             bool coords_float, int64_t m, int max_points, int c_point, int c_in, int f_out,
-                             bool use_abs, bool with_dist, const PfnDev &pfn, float *out, cudaStream_t st)
+                             bool coords_float, int64_t m, int max_points, int c_point, bool use_abs, bool with_dist,
+                             const PfnDev &pfn, float *out, cudaStream_t st)
 {
-    (void)c_in;
-    (void)f_out;
     if (m == 0) return cudaSuccess;
     DenseParams p{};
     p.voxels = voxels;

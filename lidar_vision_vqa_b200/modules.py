@@ -151,17 +151,23 @@ class _PillarVFEBase(VFETemplate):
         """What the streaming / single-layer kernels are instantiated for; everything else runs the general kernel."""
         return len(self.pfn_layers) == 1 and self.LAYOUT == 0 and int(self.num_filters[-1]) == 64
 
+    def _cache_key(self, device):
+        """Identifies the folded form: the device plus storage and version of every parameter and statistic."""
+        self._check_eval()
+        return (str(device),) + tuple((t.data_ptr(), _tensor_version(t)) for t in self._layer_tensors())
+
+    def _fold_args(self, layer):
+        """(linear weight, BatchNorm tuple or None, bias or None) of one PFNLayer, as ops.fold_layer takes them."""
+        if not self.use_norm:
+            return layer.linear.weight, None, layer.linear.bias
+        norm = layer.norm
+        return layer.linear.weight, (norm.weight, norm.bias, norm.running_mean, norm.running_var, norm.eps), None
+
     def _params(self, device) -> ops.PfnParams:
         """The single-layer form consumed by the streaming / dense kernels."""
-        self._check_eval()
-        layer = self.pfn_layers[0]
-        key = (str(device),) + tuple((t.data_ptr(), _tensor_version(t)) for t in self._layer_tensors())
+        key = self._cache_key(device)
         if self._folded is None or key != self._folded_key:
-            bn = None
-            if self.use_norm:
-                bn = (layer.norm.weight, layer.norm.bias, layer.norm.running_mean, layer.norm.running_var,
-                      layer.norm.eps)
-            self._folded = ops.fold_pfn(layer.linear.weight, bn, None if self.use_norm else layer.linear.bias,
+            self._folded = ops.fold_pfn(*self._fold_args(self.pfn_layers[0]),
                                         c_point=self.num_raw_point_features, use_absolute_xyz=self.use_absolute_xyz,
                                         with_distance=self.with_distance, voxel_size=self.voxel_size,
                                         point_cloud_range=self.point_cloud_range, device=device)
@@ -170,18 +176,11 @@ class _PillarVFEBase(VFETemplate):
 
     def _stack(self, device) -> ops.PfnStackParams:
         """Any one- or two-layer configuration, for the general feature kernel (csrc/pfn_multi.cu)."""
-        self._check_eval()
+        key = self._cache_key(device)
         if len(self.pfn_layers) > 2:
             raise NotImplementedError("PFN stacks of more than two layers are not built (no reference config uses one)")
-        key = (str(device),) + tuple((t.data_ptr(), _tensor_version(t)) for t in self._layer_tensors())
         if self._stack_folded is None or key != self._stack_key:
-            layers = []
-            for layer in self.pfn_layers:
-                bn = None
-                if self.use_norm:
-                    bn = (layer.norm.weight, layer.norm.bias, layer.norm.running_mean, layer.norm.running_var,
-                          layer.norm.eps)
-                layers.append((layer.linear.weight, bn, None if self.use_norm else layer.linear.bias))
+            layers = [self._fold_args(layer) for layer in self.pfn_layers]
             self._stack_folded = ops.fold_pfn_stack(layers, c_point=self.num_raw_point_features,
                                                     use_absolute_xyz=self.use_absolute_xyz,
                                                     with_distance=self.with_distance, voxel_size=self.voxel_size,
@@ -272,29 +271,19 @@ class PillarVFEFromPoints(_PillarVFEBase):
             offs = ops.frame_offsets_from_points(points, batch_size)
             col0 = 1
         if self._single_layer():
-            buffers = None
-            if self.output_ring > 0:
-                buffers = self._ring_buffers(points.shape[0], batch_size, points.device)
-            if self.emit_index_map and buffers is None:  # the map is a view of the workspace: keep that alive with the result
-                buffers = ops.EncodeBuffers(points.shape[0], batch_size, self.grid, int(self.num_filters[-1]), points.device,
-                                            with_bev=self.fuse_scatter)
-            res = ops.encode_bev(points, offs, self.grid, self._params(points.device), col0=col0, buffers=buffers,
-                                 with_bev=self.fuse_scatter, scatter_variant=self.scatter_variant,
-                                 want_index_map=self.emit_index_map)
-            if self.emit_index_map:
-                batch_dict["bev_index_map"] = res["cell_row"]
+            params, encode = self._params(points.device), ops.encode_bev
         else:
-            buffers = None
-            if self.output_ring > 0:
-                buffers = self._ring_buffers(points.shape[0], batch_size, points.device)
-            if self.emit_index_map and buffers is None:  # the map is a view of the workspace: keep that alive with the result
-                buffers = ops.EncodeBuffers(points.shape[0], batch_size, self.grid, int(self.num_filters[-1]), points.device,
-                                            with_bev=self.fuse_scatter)
-            res = ops.encode_stack(points, offs, self.grid, self._stack(points.device), col0=col0,
-                                   with_bev=self.fuse_scatter, scatter_variant=self.scatter_variant, buffers=buffers,
-                                   want_index_map=self.emit_index_map)
-            if self.emit_index_map:
-                batch_dict["bev_index_map"] = res["cell_row"]
+            params, encode = self._stack(points.device), ops.encode_stack
+        buffers = None
+        if self.output_ring > 0:
+            buffers = self._ring_buffers(points.shape[0], batch_size, points.device)
+        if self.emit_index_map and buffers is None:  # the map is a view of the workspace: keep that alive with the result
+            buffers = ops.EncodeBuffers(points.shape[0], batch_size, self.grid, int(self.num_filters[-1]), points.device,
+                                        with_bev=self.fuse_scatter)
+        res = encode(points, offs, self.grid, params, col0=col0, buffers=buffers, with_bev=self.fuse_scatter,
+                     scatter_variant=self.scatter_variant, want_index_map=self.emit_index_map)
+        if self.emit_index_map:
+            batch_dict["bev_index_map"] = res["cell_row"]
         if self.fuse_scatter:
             batch_dict["spatial_features"] = res["bev"]
             batch_dict["_b200_scatter_done"] = True

@@ -115,21 +115,10 @@ class PfnParams:
 def fold_pfn(weight: torch.Tensor, bn: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, float]],
              bias: Optional[torch.Tensor], *, c_point: int, use_absolute_xyz: bool, with_distance: bool, voxel_size,
              point_cloud_range, device) -> PfnParams:
-    """BatchNorm1d(eval) folded in float64: scale = gamma/sqrt(var+eps), shift = beta - mean*scale
-    (pillar_vfe.py:21-25,38-40); USE_NORM false: scale 1, shift = linear.bias."""
-    w = weight.detach().to(device=device, dtype=torch.float32).contiguous()
-    f = w.shape[0]
-    if bn is not None:
-        gamma, beta, mean, var, eps = bn
-        sc = gamma.detach().double() / torch.sqrt(var.detach().double() + eps)
-        sh = beta.detach().double() - mean.detach().double() * sc
-    else:
-        sc = torch.ones(f, dtype=torch.float64)
-        sh = bias.detach().double() if bias is not None else torch.zeros(f, dtype=torch.float64)
+    """One PFN layer folded by :func:`fold_layer`, with the streaming kernel's table prepared where it applies."""
     # pillar_vfe.py:79-81: python floats (double), later promoted into fp32 tensor arithmetic
     off = tuple(float(voxel_size[i]) / 2 + float(point_cloud_range[i]) for i in range(3))
-    sc32, sh32 = sc.to(torch.float32).contiguous(), sh.to(torch.float32).contiguous()
-    return PfnParams(w, sc32.to(device), sh32.to(device), int(c_point), bool(use_absolute_xyz), bool(with_distance),
+    return PfnParams(*fold_layer(weight, bn, bias, device), int(c_point), bool(use_absolute_xyz), bool(with_distance),
                      off).prepare()
 
 
@@ -167,7 +156,9 @@ class PfnStackParams:
 
 
 def fold_layer(weight: torch.Tensor, bn, bias, device) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """(weight fp32, scale, shift) of one layer on `device`; BatchNorm1d(eval) folded in float64."""
+    """(weight fp32, scale, shift) of one layer on `device`.  BatchNorm1d(eval) folded in float64 on the host:
+    scale = gamma/sqrt(var+eps), shift = beta - mean*scale (pillar_vfe.py:21-25,38-40); USE_NORM false: scale 1,
+    shift = linear.bias."""
     w = weight.detach().to(device=device, dtype=torch.float32).contiguous()
     f = w.shape[0]
     if bn is not None:
@@ -210,6 +201,22 @@ def _check_points(points: torch.Tensor, frame_offsets: torch.Tensor):
         raise ValueError("frame_offsets must be an int32 CUDA tensor")
 
 
+_OUTPUT_KEYS = ("pillar_features", "voxel_coords", "voxel_num_points", "voxels", "point_pillar", "point_slot", "pillar_count")
+
+
+def _outputs(res: Dict[str, torch.Tensor], capacity: int, want_index_map: bool = False) -> PillarsOutputs:
+    """The library's view of the output tensors in ``res``; an output without a key is skipped."""
+    out = PillarsOutputs()
+    out.pillar_capacity = capacity
+    for key in _OUTPUT_KEYS:
+        setattr(out, key, _ptr(res.get(key)))
+    bev = res.get("bev")
+    if bev is not None:
+        setattr(out, "bev_half" if bev.dtype == torch.float16 else "bev", bev.data_ptr())
+    out.want_index_map = int(want_index_map)
+    return out
+
+
 def voxelize(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, *, col0: int = 0,
              c_point: Optional[int] = None, capacity: Optional[int] = None, want_voxels: bool = True,
              want_membership: bool = False, ws_slot: int = 0) -> Dict[str, torch.Tensor]:
@@ -224,7 +231,6 @@ def voxelize(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, 
     cap = max(int(cap), 1)
     dev = points.device
     g = grid.native()
-    out = PillarsOutputs()
     res = {
         "voxel_coords": torch.empty((cap, 4), dtype=torch.int32, device=dev),
         "voxel_num_points": torch.empty((cap,), dtype=torch.int32, device=dev),
@@ -235,13 +241,7 @@ def voxelize(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, 
     if want_membership:
         res["point_pillar"] = torch.empty((n,), dtype=torch.int32, device=dev)
         res["point_slot"] = torch.empty((n,), dtype=torch.int32, device=dev)
-    out.pillar_capacity = cap
-    out.voxel_coords = _ptr(res["voxel_coords"])
-    out.voxel_num_points = _ptr(res["voxel_num_points"])
-    out.voxels = _ptr(res.get("voxels"))
-    out.point_pillar = _ptr(res.get("point_pillar"))
-    out.point_slot = _ptr(res.get("point_slot"))
-    out.pillar_count = _ptr(res["pillar_count"])
+    out = _outputs(res, cap)
     need = lib.pillars_workspace_bytes(n, nb, ctypes.byref(g))
     ws = workspace(need, dev, ws_slot)
     check(lib.pillars_voxelize(points.data_ptr(), n, stride, col0, c_point, frame_offsets.data_ptr(), nb,
@@ -250,29 +250,31 @@ def voxelize(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, 
     return res
 
 
+def _padded_inputs(voxels: torch.Tensor, num_points: torch.Tensor, coords: torch.Tensor, c_point: int):
+    """Checks the reference's padded input and brings ``num_points`` and ``coords`` to what the library reads, with a
+    flag that is 1 for float32: float32 and int32 pass through, other floating types become float32, other integer types
+    int32; bool and complex tensors are refused."""
+    _require_device(voxels)
+    if voxels.dtype != torch.float32 or voxels.dim() != 3:
+        raise ValueError("voxels must be float32 [M,P,C]")
+    if voxels.shape[2] != c_point:
+        raise ValueError(f"voxels have {voxels.shape[2]} channels, the PFN was built for {c_point}")
+
+    def norm(t, name):
+        if t.dtype == torch.bool or t.dtype.is_complex:
+            raise ValueError(f"{name}: unsupported dtype {t.dtype}")
+        is_float = t.dtype.is_floating_point
+        return t.to(torch.float32 if is_float else torch.int32).contiguous(), int(is_float)
+
+    return (voxels.contiguous(), *norm(num_points, "voxel_num_points"), *norm(coords, "voxel_coords"))
+
+
 def pfn_dense(voxels: torch.Tensor, num_points: torch.Tensor, coords: torch.Tensor, pfn: PfnParams,
               voxel_size) -> torch.Tensor:
     """PillarVFE.forward on the reference's padded input: ``voxels [M,P,C]``, ``num_points [M]``, ``coords [M,4]``
     (int32 or float32 each).  Returns ``[M, F]``."""
-    _require_device(voxels)
-    if voxels.dtype != torch.float32 or voxels.dim() != 3:
-        raise ValueError("voxels must be float32 [M,P,C]")
-    voxels = voxels.contiguous()
-    m, p, c = voxels.shape
-    if c != pfn.c_point:
-        raise ValueError(f"voxels have {c} channels, the PFN was built for {pfn.c_point}")
-
-    def norm(t, name):
-        if t.dtype in (torch.float32, torch.int32):
-            return t.contiguous(), int(t.dtype == torch.float32)
-        if t.dtype in (torch.int64, torch.int16, torch.uint8):
-            return t.to(torch.int32).contiguous(), 0
-        if t.dtype.is_floating_point:
-            return t.to(torch.float32).contiguous(), 1
-        raise ValueError(f"{name}: unsupported dtype {t.dtype}")
-
-    npts, np_f = norm(num_points, "voxel_num_points")
-    crd, crd_f = norm(coords, "voxel_coords")
+    voxels, npts, np_f, crd, crd_f = _padded_inputs(voxels, num_points, coords, pfn.c_point)
+    m, p, _ = voxels.shape
     out = torch.empty((m, pfn.weight.shape[0]), dtype=torch.float32, device=voxels.device)
     vs = (ctypes.c_float * 3)(*[float(v) for v in voxel_size])
     nat = pfn.native()
@@ -284,23 +286,8 @@ def pfn_dense(voxels: torch.Tensor, num_points: torch.Tensor, coords: torch.Tens
 def pfn_dense_stack(voxels: torch.Tensor, num_points: torch.Tensor, coords: torch.Tensor, stack: PfnStackParams,
                     voxel_size) -> torch.Tensor:
     """PillarVFE.forward on padded voxels through a one- or two-layer stack (pillar_vfe.py:94-123 with :44-49)."""
-    _require_device(voxels)
-    if voxels.dtype != torch.float32 or voxels.dim() != 3:
-        raise ValueError("voxels must be float32 [M,P,C]")
-    voxels = voxels.contiguous()
-    m, p, c = voxels.shape
-    if c != stack.c_point:
-        raise ValueError(f"voxels have {c} channels, the PFN was built for {stack.c_point}")
-
-    def norm(t):
-        if t.dtype in (torch.float32, torch.int32):
-            return t.contiguous(), int(t.dtype == torch.float32)
-        if t.dtype.is_floating_point:
-            return t.to(torch.float32).contiguous(), 1
-        return t.to(torch.int32).contiguous(), 0
-
-    npts, np_f = norm(num_points)
-    crd, crd_f = norm(coords)
+    voxels, npts, np_f, crd, crd_f = _padded_inputs(voxels, num_points, coords, stack.c_point)
+    m, p, _ = voxels.shape
     out = torch.empty((m, stack.f_out), dtype=torch.float32, device=voxels.device)
     vs = (ctypes.c_float * 3)(*[float(v) for v in voxel_size])
     nat = stack.native()
@@ -320,69 +307,32 @@ def encode_stack(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSp
     ``dynamic=True``: DynamicPillarVFE / DynamicPillarVFESimple2D semantics (dynamic_pillar_vfe.py:90-142, :193-240).
     ``buffers`` (hard mode, 4-column coords): pre-allocated outputs + workspace, as for :func:`encode_bev`;
     ``want_index_map`` (needs ``buffers``, whose workspace it is a view of): ``cell_row`` as in :func:`encode_bev`."""
-    _check_points(points, frame_offsets)
-    lib = _native.load()
-    n, stride = points.shape
-    nb = frame_offsets.numel() - 1
-    if stride - col0 < stack.c_point:
-        raise ValueError("points have fewer channels than the PFN expects")
-    dev = points.device
-    nx, ny, nz = grid.grid_size
-    g = grid.native()
-    need = lib.pillars_workspace_bytes(n, nb, ctypes.byref(g))
-    out = PillarsOutputs()
-    if buffers is not None:
-        if dynamic or coords_cols != 4:
-            raise ValueError("EncodeBuffers hold hard-mode outputs with (b, z, y, x) coordinates")
-        if buffers.pillar_features.shape[1] != stack.f_out or buffers.n_frames != nb:
-            raise ValueError("buffers were created for another feature width / batch size")
-        if buffers.ws.numel() < need:
-            raise ValueError("EncodeBuffers workspace too small for this batch")
-        res = {"pillar_features": buffers.pillar_features, "voxel_coords": buffers.voxel_coords,
-               "voxel_num_points": buffers.voxel_num_points, "pillar_count": buffers.pillar_count}
-        out.pillar_capacity = buffers.capacity
-        ws = buffers.ws
-        if with_bev:
-            if buffers.bev is None:
-                raise ValueError("buffers were created without a BEV canvas")
-            res["bev"] = buffers.bev
-    else:
+    if buffers is not None and (dynamic or coords_cols != 4):
+        raise ValueError("EncodeBuffers hold hard-mode outputs with (b, z, y, x) coordinates")
+    if want_index_map and buffers is None:
+        raise ValueError("want_index_map needs EncodeBuffers (the map is a view of their workspace)")
+
+    def fresh(n, nb, need):  # outputs of this call alone; the workspace is the cached one of `ws_slot`
         cap = capacity
         if cap is None:
             cap = n if dynamic else min(n, nb * grid.max_voxels)
         cap = max(int(cap), 1)  # an empty batch still needs non-NULL output pointers
+        dev = points.device
+        nx, ny, nz = grid.grid_size
         res = {
             "pillar_features": torch.empty((cap, stack.f_out), dtype=torch.float32, device=dev),
             "voxel_coords": torch.empty((cap, coords_cols), dtype=torch.int32, device=dev),
             "voxel_num_points": torch.empty((cap,), dtype=torch.int32, device=dev),
             "pillar_count": torch.empty((nb + 1,), dtype=torch.int32, device=dev),
         }
-        out.pillar_capacity = cap
         if with_bev:
             res["bev"] = torch.empty((nb, stack.f_out * nz, ny, nx), dtype=torch.float32, device=dev)
-        ws = workspace(need, dev, ws_slot)
-    out.pillar_features = res["pillar_features"].data_ptr()
-    out.voxel_coords = res["voxel_coords"].data_ptr()
-    out.voxel_num_points = res["voxel_num_points"].data_ptr()
-    out.pillar_count = res["pillar_count"].data_ptr()
-    if with_bev:
-        if res["bev"].dtype == torch.float16:
-            out.bev_half = res["bev"].data_ptr()
-        else:
-            out.bev = res["bev"].data_ptr()
-    if want_index_map:
-        if buffers is None:
-            raise ValueError("want_index_map needs EncodeBuffers (the map is a view of their workspace)")
-        out.want_index_map = 1
-        off = lib.pillars_workspace_cell_row_offset(n, nb, ctypes.byref(g))
-        res["cell_row"] = buffers.ws[off:off + 4 * nb * ny * nx].view(torch.int32).view(nb, ny, nx)
+        return res, workspace(need, dev, ws_slot)
+
     nat = stack.native()
     mode = _native.MODE_DYNAMIC if dynamic else _native.MODE_HARD
-    variant, stream = SCATTER_VARIANTS[scatter_variant], _stream_ptr()
-    check(_encode_canvas(buffers if with_bev else None, lib, lambda: lib.pillars_encode_stack(
-        points.data_ptr(), n, stride, col0, frame_offsets.data_ptr(), nb, ctypes.byref(g), ctypes.byref(nat), mode,
-        coords_cols, ctypes.byref(out), ws.data_ptr(), ws.numel(), variant, stream)), "pillars_encode_stack")
-    return res
+    return _encode("pillars_encode_stack", (ctypes.byref(nat), mode, coords_cols), points, frame_offsets, grid,
+                   stack.f_out, stack.c_point, col0, buffers, with_bev, want_index_map, scatter_variant, fresh)
 
 
 def scatter_bev(pillar_features: torch.Tensor, coords: torch.Tensor, batch_size: int, nx: int, ny: int, nz: int = 1, *,
@@ -498,6 +448,55 @@ def _encode_canvas(buffers: Optional[EncodeBuffers], lib, call) -> int:
     return rc
 
 
+def _encode(entry: str, features: tuple, points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, f_out: int,
+            c_point: int, col0: int, buffers: Optional[EncodeBuffers], with_bev: bool, want_index_map: bool,
+            scatter_variant: str, fresh=None, want_membership: bool = False, want_voxels: bool = False
+            ) -> Dict[str, torch.Tensor]:
+    """What :func:`encode_bev` and :func:`encode_stack` share: the checks, the outputs, the ``cell_row`` view and the
+    native call ``entry``, whose feature arguments are ``features``.  The outputs and the workspace are those of
+    ``buffers``, or without buffers ``fresh(n, nb, workspace_bytes) -> (result dict, workspace)``."""
+    lib = _native.load()
+    n, nb = points.shape[0], frame_offsets.numel() - 1
+    g = grid.native()
+    need = lib.pillars_workspace_bytes(n, nb, ctypes.byref(g))
+    if buffers is not None:  # (the library would write past them)
+        if buffers.pillar_features.shape[1] != f_out or buffers.n_frames != nb:
+            raise ValueError("buffers were created for another feature width / batch size")
+        if buffers.ws.numel() < need:
+            raise ValueError("EncodeBuffers workspace too small for this batch")
+        if with_bev and buffers.bev is None:
+            raise ValueError("buffers were created without a BEV canvas")
+    _check_points(points, frame_offsets)
+    stride = points.shape[1]
+    if stride - col0 < c_point:
+        raise ValueError("points have fewer channels than the PFN expects")
+    if buffers is not None:
+        res = {"pillar_features": buffers.pillar_features, "voxel_coords": buffers.voxel_coords,
+               "voxel_num_points": buffers.voxel_num_points, "pillar_count": buffers.pillar_count}
+        if with_bev:
+            res["bev"] = buffers.bev
+        ws = buffers.ws
+    else:
+        res, ws = fresh(n, nb, need)
+    cap = res["pillar_features"].shape[0]
+    if want_membership:
+        res["point_pillar"] = torch.empty((n,), dtype=torch.int32, device=points.device)
+        res["point_slot"] = torch.empty((n,), dtype=torch.int32, device=points.device)
+    if want_voxels:
+        res["voxels"] = torch.empty((cap, grid.max_points, c_point), dtype=torch.float32, device=points.device)
+    out = _outputs(res, cap, want_index_map)
+    if want_index_map:
+        # the workspace layout depends on the point count of THIS call
+        off = lib.pillars_workspace_cell_row_offset(n, nb, ctypes.byref(g))
+        nx, ny, _ = grid.grid_size
+        res["cell_row"] = ws[off:off + 4 * nb * ny * nx].view(torch.int32).view(nb, ny, nx)
+    call = getattr(lib, entry)
+    args = (points.data_ptr(), n, stride, col0, frame_offsets.data_ptr(), nb, ctypes.byref(g), *features, ctypes.byref(out),
+            ws.data_ptr(), ws.numel(), SCATTER_VARIANTS[scatter_variant], _stream_ptr())
+    check(_encode_canvas(buffers if with_bev else None, lib, lambda: call(*args)), entry)
+    return res
+
+
 def encode_bev(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, pfn: PfnParams, *, col0: int = 0,
                buffers: Optional[EncodeBuffers] = None, with_bev: bool = True, scatter_variant: str = "auto",
                want_membership: bool = False, want_voxels: bool = False, want_index_map: bool = False
@@ -507,58 +506,14 @@ def encode_bev(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec
     the workspace, valid until ``buffers`` is reused -- the input of the BEV tokeniser (tokens.py) and of the backbone's
     first layer (backbone.py); it does not need a canvas (``with_bev=False``).
     Everything is enqueued on the current stream; nothing synchronises."""
-    _check_points(points, frame_offsets)
-    lib = _native.load()
-    n, stride = points.shape
-    nb = frame_offsets.numel() - 1
-    if stride - col0 < pfn.c_point:
-        raise ValueError("points have fewer channels than the PFN expects")
-    dev = points.device
     f_out = int(pfn.weight.shape[0])
-    if buffers is None:
-        buffers = EncodeBuffers(n, nb, grid, f_out, dev, with_bev=with_bev)
-    g = grid.native()
-    need = lib.pillars_workspace_bytes(n, nb, ctypes.byref(g))
-    if buffers.ws.numel() < need:
-        raise ValueError("EncodeBuffers workspace too small for this batch")
-    res = {"pillar_features": buffers.pillar_features, "voxel_coords": buffers.voxel_coords,
-           "voxel_num_points": buffers.voxel_num_points, "pillar_count": buffers.pillar_count}
-    out = PillarsOutputs()
-    out.pillar_capacity = buffers.capacity
-    out.pillar_features = buffers.pillar_features.data_ptr()
-    out.voxel_coords = buffers.voxel_coords.data_ptr()
-    out.voxel_num_points = buffers.voxel_num_points.data_ptr()
-    out.pillar_count = buffers.pillar_count.data_ptr()
-    if with_bev:
-        if buffers.bev is None:
-            raise ValueError("buffers were created without a BEV canvas")
-        if buffers.n_frames != nb:
-            raise ValueError("buffers were created for another batch size")
-        if buffers.bev.dtype == torch.float16:
-            out.bev_half = buffers.bev.data_ptr()
-        else:
-            out.bev = buffers.bev.data_ptr()
-        res["bev"] = buffers.bev
-    if want_membership:
-        res["point_pillar"] = torch.empty((n,), dtype=torch.int32, device=dev)
-        res["point_slot"] = torch.empty((n,), dtype=torch.int32, device=dev)
-        out.point_pillar = res["point_pillar"].data_ptr()
-        out.point_slot = res["point_slot"].data_ptr()
-    if want_voxels:
-        res["voxels"] = torch.empty((buffers.capacity, grid.max_points, pfn.c_point), dtype=torch.float32, device=dev)
-        out.voxels = res["voxels"].data_ptr()
-    if want_index_map:
-        out.want_index_map = 1
-        # the workspace layout depends on the point count of THIS call
-        off = lib.pillars_workspace_cell_row_offset(n, nb, ctypes.byref(g))
-        nx, ny, _ = grid.grid_size
-        res["cell_row"] = buffers.ws[off:off + 4 * nb * ny * nx].view(torch.int32).view(nb, ny, nx)
+    if buffers is None:  # the call's own, so that the cell_row view keeps its workspace alive
+        _require_device(points)
+        buffers = EncodeBuffers(points.shape[0], frame_offsets.numel() - 1, grid, f_out, points.device, with_bev=with_bev)
     nat = pfn.native()
-    variant, stream = SCATTER_VARIANTS[scatter_variant], _stream_ptr()
-    check(_encode_canvas(buffers if with_bev else None, lib, lambda: lib.pillars_encode_bev(
-        points.data_ptr(), n, stride, col0, frame_offsets.data_ptr(), nb, ctypes.byref(g), ctypes.byref(nat),
-        ctypes.byref(out), buffers.ws.data_ptr(), buffers.ws.numel(), variant, stream)), "pillars_encode_bev")
-    return res
+    return _encode("pillars_encode_bev", (ctypes.byref(nat),), points, frame_offsets, grid, f_out, pfn.c_point, col0,
+                   buffers, with_bev, want_index_map, scatter_variant, want_membership=want_membership,
+                   want_voxels=want_voxels)
 
 
 def rebase_segments(coords: torch.Tensor, segment_counts: torch.Tensor, frames_per_segment: int,

@@ -1,11 +1,13 @@
 """Two-layer PFN ([64,64], waymo_models/pointpillar_1x.yaml:34) through pillars_encode_stack vs the single-layer path.
-Usage: python profiles/scripts/stack_times.py [workload]"""
+Usage: python profiles/scripts/stack_times.py [--generic] [workload]   (--generic: the general kernel, ops.force_generic_features)"""
 import os, sys, numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import lidar_vision_vqa_b200 as L
 from lidar_vision_vqa_b200 import _native, ops, synth
 from oracle import pillar_oracle as po
-wl = sys.argv[1] if len(sys.argv) > 1 else "cfg2_nuscenes32_b16_pillar0.2_bev512"
+argv = [a for a in sys.argv[1:] if a != "--generic"]
+wl = argv[0] if argv else "cfg2_nuscenes32_b16_pillar0.2_bev512"
+ops.force_generic_features("--generic" in sys.argv)
 dev = torch.device("cuda:0")
 model, gc, nb = synth.WORKLOADS[wl]
 grid = L.GridSpec.from_range(gc.point_cloud_range, gc.voxel_size, gc.max_points_per_voxel, gc.max_voxels)
