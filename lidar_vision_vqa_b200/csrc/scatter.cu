@@ -6,13 +6,14 @@
 // grouping stage or by k_build_cell_row) turns the scatter inside out: every output element is written exactly once,
 // in NCHW order, with full-line stores, zero-fill included, no atomics.
 //
-// On a canvas the library wrote before, most of those stores put zeros over zeros.  The wide kernels then take two
-// occupancy bitmaps (layout in include/pillars_b200.h, pillars_set_canvas_occupancy): bit = "these 8 cells of the frame
-// may be non-zero".  A lane writes its 8 cells x channels only when they are occupied now or were last time (zeros
-// where only the old bit is set); every other canvas element already holds its zero.  The store unit stays one 32-byte
-// sector, so no sector is ever written in part.
+// On a canvas the library wrote before, most of those stores put zeros over zeros.  The caller then passes two occupancy
+// bitmaps (layout in include/pillars_b200.h, pillars_set_canvas_occupancy): bit = "these 8 cells of the frame may be
+// non-zero".  With the previous bitmap, k_scatter_sparse reads the index map once and writes only the 8-cell groups that
+// are occupied now or were last time (zeros where only the old bit is set); every other canvas element already holds its
+// zero.  The store unit stays one 32-byte sector, so no sector is ever written in part.  Without it (fresh or invalidated
+// canvas) the full-write kernels run and record the next bitmap.
 //
-// Two kernels ship: the channel-group 256-bit store kernel (k_scatter_wide, 99 % of the measured copy peak) and a plain
+// Full writes: the channel-group 256-bit store kernel (k_scatter_wide, 99 % of the measured copy peak) and a plain
 // kernel for shapes it does not cover (odd plane sizes, unaligned canvases, F not a multiple of 8).  The other store paths
 // that were measured and lost (bulk 1-D copies, TMA tile stores, persistent warps, zero-fill + patches) are kept as
 // evidence, out of the product library: profiles/micro/r01_scatter_variants.cu.txt, numbers in
@@ -158,18 +159,6 @@ k_scatter_plain(const float *__restrict__ feats, const int32_t *__restrict__ cel
 // One bit per 8 cells, one word per 256 cells (a warp of the wide kernels), words_per_frame = ceil(plane / 256).
 __host__ __device__ __forceinline__ int64_t occ_words(int64_t plane) { return (plane + 255) >> 8; }
 
-// The occ_prev word of the calling warp of a wide-kernel CTA (blockIdx decoded as there), all ones when there is no
-// bitmap or the warp lies past the plane.
-__device__ __forceinline__ uint32_t occ_prev_word(const uint32_t *__restrict__ occ_prev, int64_t plane, int tiles_per_plane,
-                                                  int groups, int tile_major)
-{
-    if (!occ_prev) return 0xffffffffu;
-    const int tile = tile_major ? (blockIdx.x / groups) % tiles_per_plane : blockIdx.x % tiles_per_plane;
-    const int b = blockIdx.x / (groups * tiles_per_plane);
-    const int64_t word = (static_cast<int64_t>(tile) * blockDim.x + threadIdx.x) >> 5;
-    return word < occ_words(plane) ? __ldg(occ_prev + b * occ_words(plane) + word) : 0xffffffffu;
-}
-
 // ---- variant 4 ----------------------------------------------------------------------------------
 // Same warp-autonomous scheme with 256-bit accesses (sm_100: LDG.256 / STG.256): a lane owns 8 consecutive cells, a warp
 // 256 cells x all channels = 64 KB of the canvas, and every store instruction of the warp writes 1 KB contiguous.  Half the
@@ -193,16 +182,12 @@ __device__ __forceinline__ void stg256_cs(float *p, float a, float b, float c, f
 // the CTAs of one cell tile then each read one 32-byte sector of every pillar row, so no feature byte is fetched twice.
 // tile_major != 0: consecutive CTAs are the channel groups of one cell tile (index map and feature rows are shared by CTAs
 // that run together); 0: consecutive CTAs walk the plane for one channel group.
-// occ_next != NULL: a lane stores only where its bit of occ_prev (NULL: all set) or its "any cell occupied" test is set, and
-// the channel group 0 CTAs record the latter into occ_next.
+// occ_next != NULL: the channel group 0 CTAs record each lane's "any cell occupied" test into occ_next.
 template <bool CS, int CPP>
 __global__ void __launch_bounds__(kThreads)
 k_scatter_wide(const float *__restrict__ feats, const int32_t *__restrict__ cell_row, int f, int64_t plane,
-               int tiles_per_plane, int chan_per_cta, int tile_major, float *__restrict__ bev,
-               const uint32_t *__restrict__ occ_prev, uint32_t *__restrict__ occ_next)
+               int tiles_per_plane, int chan_per_cta, int tile_major, float *__restrict__ bev, uint32_t *__restrict__ occ_next)
 {
-    // the previous call on this canvas wrote occ_prev and finished before this call's first (non-PDL) launch
-    const uint32_t prev = occ_prev_word(occ_prev, plane, tiles_per_plane, f / chan_per_cta, tile_major);
     pdl_wait();  // feature rows and index map come from the kernels before this one
     const int groups = f / chan_per_cta;
     int b, tile, cg;
@@ -237,7 +222,7 @@ k_scatter_wide(const float *__restrict__ feats, const int32_t *__restrict__ cell
     };
     const uint32_t now = __ballot_sync(0xffffffffu, any);
     if (occ_next && cg == 0 && (threadIdx.x & 31) == 0 && inb) occ_next[b * occ_words(plane) + (cell0 >> 8)] = now;
-    if (!inb || !(any || ((prev >> (threadIdx.x & 31)) & 1u))) return;
+    if (!inb) return;
     if (now == 0) {
 #pragma unroll 8
         for (int c = c_begin; c < c_end; ++c) store(dst + c * plane, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f);
@@ -278,14 +263,10 @@ __device__ __forceinline__ void ldg256_stream(const float *p, float (&v)[8])
 // The product's caller stores the BEV map as float16 (src/get-data/precompute_bev_features.py:394: bev.astype(np.float16));
 // converting in the scatter halves the dominant write.  Same work split as variant 4: a lane owns 8 cells = one 16-byte
 // store per channel, round-to-nearest-even like numpy / torch.
-// A lane's 16 bytes are half a sector: the pair of lanes that shares one decides together, so that no sector is written in
-// part (L2 would fetch the rest of it from DRAM).
 __global__ void __launch_bounds__(kThreads)
 k_scatter_wide_half(const float *__restrict__ feats, const int32_t *__restrict__ cell_row, int f, int64_t plane,
-                    int tiles_per_plane, __half *__restrict__ bev, const uint32_t *__restrict__ occ_prev,
-                    uint32_t *__restrict__ occ_next)
+                    int tiles_per_plane, __half *__restrict__ bev, uint32_t *__restrict__ occ_next)
 {
-    const uint32_t prev = occ_prev_word(occ_prev, plane, tiles_per_plane, f >> 3, 0);
     const int groups = f >> 3;
     const int tile = blockIdx.x % tiles_per_plane;
     const int cg = (blockIdx.x / tiles_per_plane) % groups;
@@ -308,8 +289,7 @@ k_scatter_wide_half(const float *__restrict__ feats, const int32_t *__restrict__
     __half *dst = bev + (static_cast<int64_t>(b) * f + c0) * plane + cell0;
     const uint32_t now = __ballot_sync(0xffffffffu, any);
     if (occ_next && cg == 0 && (threadIdx.x & 31) == 0 && inb) occ_next[b * occ_words(plane) + (cell0 >> 8)] = now;
-    const uint32_t pair = (now | prev) | (((now | prev) >> 1) & 0x55555555u) | (((now | prev) & 0x55555555u) << 1);
-    if (!inb || !((pair >> (threadIdx.x & 31)) & 1u)) return;
+    if (!inb) return;
     if (now == 0) {
 #pragma unroll
         for (int c = 0; c < 8; ++c) __stcs(reinterpret_cast<uint4 *>(dst + c * plane), make_uint4(0u, 0u, 0u, 0u));
@@ -331,6 +311,114 @@ k_scatter_wide_half(const float *__restrict__ feats, const int32_t *__restrict__
         h = __floats2half2_rn(v[4][c], v[5][c]); o.z = *reinterpret_cast<uint32_t *>(&h);
         h = __floats2half2_rn(v[6][c], v[7][c]); o.w = *reinterpret_cast<uint32_t *>(&h);
         *reinterpret_cast<uint4 *>(dst + c * plane) = o;
+    }
+}
+
+// ---- reused canvas: dirty groups only -------------------------------------------------------------
+// With occ_prev, every canvas element outside prev's groups already holds its zero, so only the 8-cell groups of
+// prev | now need stores.  A CTA owns a span of kSparseWarps bitmap words (256 cells each) of one frame, all channels:
+//  1. each warp takes one word: prev (loaded before pdl_wait), the index map of its 256 cells (a lane = one group, two
+//     16-byte loads), now = ballot of "any cell occupied", recorded into occ_next.  The groups of now | prev store their
+//     8 row indices (-1 = empty cell) and position, in cell order, in the warp's part of a shared list;
+//  2. the CTA walks the items (dirty group, 8-channel chunk), chunk by chunk, so that a warp's stores go to one channel
+//     plane, close together.  A lane loads the group's rows (one 32-byte sector each, nothing for an empty cell) and
+//     stores 8 channels x 8 cells: 8 STG.256, or 8 16-byte stores on the float16 canvas.
+// The index map is read once, not once per channel group, and a clean empty group costs nothing more.  On the float16
+// canvas a lane's 16 bytes are half a sector: the lane pairs are dirty together (pair-closed masks keep both halves in
+// adjacent list slots at even offsets, so one warp store instruction writes both).  A pair is one 32-byte sector when
+// the canvas is 32-byte aligned and the plane a multiple of 16 cells (the bench's shapes); otherwise pairs straddle
+// sectors, which costs speed, not correctness.  Both canvases launch it with PDL (the float16 full-write kernel keeps
+// its plain launch).
+// Span: 1024 cells.  The dirty groups are unevenly spread over the plane; short CTAs balance them over the SMs, and the
+// grid (cfg1: 256 CTAs, cfg2: 4096, cfg4: 8192; 5 fit on an SM at 96 registers x 128 threads, 4 of the float16 kernel at
+// 98) leaves SMs free for a concurrent stream's grouping as it drains.  Longer spans (2, 4 or 8 words per warp) were
+// measured and are slower: cfg2 105k / 101k sweeps/s at 2 / 4 words against 107k; cfg4 cycling batches 243 us at 2 words
+// against 229 us (B200; profiles/r04_ab.txt, r04_scatter_sparse.json).
+constexpr int kSparseWarps = 4;
+
+template <bool HALF>
+__global__ void __launch_bounds__(kSparseWarps * 32)
+k_scatter_sparse(const float *__restrict__ feats, const int32_t *__restrict__ cell_row, int f, int64_t plane,
+                 int spans_per_plane, void *__restrict__ bev, const uint32_t *__restrict__ occ_prev,
+                 uint32_t *__restrict__ occ_next)
+{
+    constexpr int kGroups = kSparseWarps * 32;
+    __shared__ int4 s_rows[2 * kGroups];
+    __shared__ int32_t s_cell[kGroups];  // the group's first cell, relative to the span
+    __shared__ int s_count[kSparseWarps];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int b = blockIdx.x / spans_per_plane;
+    const int64_t words = occ_words(plane);
+    const int64_t span_word = static_cast<int64_t>(blockIdx.x % spans_per_plane) * kSparseWarps;
+    const int64_t word = span_word + warp;
+    // the previous call on this canvas wrote occ_prev and finished before this call's first (non-PDL) launch
+    const uint32_t prev = word < words ? __ldg(occ_prev + b * words + word) : 0u;
+    pdl_wait();  // feature rows and index map come from the kernels before this one
+    const int64_t cell0 = word * 256 + lane * 8;
+    const bool inb = cell0 < plane;  // plane % 8 == 0: a lane is entirely inside or outside
+    int4 v = make_int4(-1, -1, -1, -1), w = v;
+    if (inb) {
+        const int4 *src = reinterpret_cast<const int4 *>(cell_row + b * plane + cell0);
+        v = __ldg(src);
+        w = __ldg(src + 1);
+    }
+    const bool any = (v.x & v.y & v.z & v.w & w.x & w.y & w.z & w.w) >= 0;  // some row index is not -1
+    const uint32_t now = __ballot_sync(0xffffffffu, any);
+    if (lane == 0 && word < words) occ_next[b * words + word] = now;
+    uint32_t dirty = now | prev;
+    if (HALF) dirty |= ((dirty >> 1) & 0x55555555u) | ((dirty & 0x55555555u) << 1);
+    dirty &= __ballot_sync(0xffffffffu, inb);
+    if ((dirty >> lane) & 1u) {
+        const int s = warp * 32 + __popc(dirty & ((1u << lane) - 1u));
+        s_rows[2 * s] = v;
+        s_rows[2 * s + 1] = w;
+        s_cell[s] = static_cast<int>(cell0 - span_word * 256);
+    }
+    const int n = __popc(dirty);
+    if (lane == 0) s_count[warp] = n;
+    __syncthreads();
+    int off[kSparseWarps];  // list position of each warp's first group
+    off[0] = 0;
+#pragma unroll
+    for (int k = 1; k < kSparseWarps; ++k) off[k] = off[k - 1] + s_count[k - 1];
+    const int total = off[kSparseWarps - 1] + s_count[kSparseWarps - 1];
+    const int items = total * (f >> 3);
+    const int64_t span_base = static_cast<int64_t>(b) * f * plane + span_word * 256;
+    for (int i = threadIdx.x; i < items; i += blockDim.x) {
+        const int chunk = i / total, g = i - chunk * total;
+        int s = g;
+#pragma unroll
+        for (int k = 1; k < kSparseWarps; ++k)
+            if (g >= off[k]) s = k * 32 + g - off[k];
+        const int4 v = s_rows[2 * s], w = s_rows[2 * s + 1];
+        const int r[8] = {v.x, v.y, v.z, v.w, w.x, w.y, w.z, w.w};
+        const int c0 = chunk * 8;
+        float x[8][8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+#pragma unroll
+            for (int c = 0; c < 8; ++c) x[k][c] = 0.f;
+            if (r[k] >= 0) ldg256_stream(feats + static_cast<int64_t>(r[k]) * f + c0, x[k]);
+        }
+        const int64_t at = span_base + static_cast<int64_t>(c0) * plane + s_cell[s];
+        if (HALF) {
+            __half *dst = static_cast<__half *>(bev) + at;
+#pragma unroll
+            for (int c = 0; c < 8; ++c) {
+                uint4 o;
+                __half2 h;
+                h = __floats2half2_rn(x[0][c], x[1][c]); o.x = *reinterpret_cast<uint32_t *>(&h);
+                h = __floats2half2_rn(x[2][c], x[3][c]); o.y = *reinterpret_cast<uint32_t *>(&h);
+                h = __floats2half2_rn(x[4][c], x[5][c]); o.z = *reinterpret_cast<uint32_t *>(&h);
+                h = __floats2half2_rn(x[6][c], x[7][c]); o.w = *reinterpret_cast<uint32_t *>(&h);
+                *reinterpret_cast<uint4 *>(dst + c * plane) = o;
+            }
+        } else {
+            float *dst = static_cast<float *>(bev) + at;
+#pragma unroll
+            for (int c = 0; c < 8; ++c)
+                stg256(dst + c * plane, x[0][c], x[1][c], x[2][c], x[3][c], x[4][c], x[5][c], x[6][c], x[7][c]);
+        }
     }
 }
 
@@ -360,6 +448,20 @@ cudaError_t launch_rebase_segments(int32_t *coords, int n_seg, int64_t rows_per_
     return cudaGetLastError();
 }
 
+// k_scatter_sparse for a canvas with a previous bitmap (needs plane % 8 == 0, f % 8 == 0, 32-byte aligned feature rows
+// and a canvas aligned to its store unit).
+template <bool HALF>
+cudaError_t launch_scatter_sparse(const float *feats, const int32_t *cell_row, int nb, int f, int64_t plane, void *bev,
+                                  cudaStream_t st, const uint32_t *occ_prev, uint32_t *occ_next)
+{
+    const int spp = static_cast<int>((occ_words(plane) + kSparseWarps - 1) / kSparseWarps);
+    const cudaError_t err = launch_pdl(k_scatter_sparse<HALF>, dim3(static_cast<unsigned>(nb) * spp), dim3(kSparseWarps * 32),
+                                       0, st, feats, cell_row, f, plane, spp, bev, occ_prev, occ_next);
+    if (err != cudaSuccess) return err;
+    note_launch();
+    return cudaGetLastError();
+}
+
 cudaError_t launch_scatter_half(const float *feats, const int32_t *cell_row, int nb, int f, int nx, int ny, void *bev,
                                 cudaStream_t st, const uint32_t *occ_prev, uint32_t *occ_next)
 {
@@ -368,10 +470,11 @@ cudaError_t launch_scatter_half(const float *feats, const int32_t *cell_row, int
     if (plane % 8 != 0 || f % 8 != 0 || reinterpret_cast<uintptr_t>(bev) % 16 != 0 ||
         reinterpret_cast<uintptr_t>(feats) % 32 != 0)
         return cudaErrorInvalidValue;
+    if (occ_prev) return launch_scatter_sparse<true>(feats, cell_row, nb, f, plane, bev, st, occ_prev, occ_next);
     const int bs = 128;
     const int tpp = static_cast<int>((plane + bs * 8 - 1) / (bs * 8));
     const unsigned grid = static_cast<unsigned>(nb) * tpp * (f / 8);
-    k_scatter_wide_half<<<grid, bs, 0, st>>>(feats, cell_row, f, plane, tpp, static_cast<__half *>(bev), occ_prev, occ_next);
+    k_scatter_wide_half<<<grid, bs, 0, st>>>(feats, cell_row, f, plane, tpp, static_cast<__half *>(bev), occ_next);
     note_launch();
     return cudaGetLastError();
 }
@@ -385,6 +488,8 @@ cudaError_t launch_scatter(const float *feats, const int32_t *cell_row, int nb, 
     const bool wide_ok = vec_ok && (plane % 8 == 0) && (reinterpret_cast<uintptr_t>(bev) % 32 == 0);
     // measured on B200, cfg2 (profiles/r01_scatter_variants.md): channel-group 256-bit stores 172 us, direct stores with all
     // channels per warp 203 us
+    if (variant != 1 && wide_ok && occ_prev && reinterpret_cast<uintptr_t>(feats) % 32 == 0)
+        return launch_scatter_sparse<false>(feats, cell_row, nb, f, plane, bev, st, occ_prev, occ_next);
     if (variant != 1 && wide_ok) {
         // a CTA owns 128 lanes x 8 cells x 8 channels: few long sequential write streams per CTA
         constexpr int bs = 128, chan = 8;
@@ -392,9 +497,9 @@ cudaError_t launch_scatter(const float *feats, const int32_t *cell_row, int nb, 
         const unsigned grid = static_cast<unsigned>(nb) * tpp * (f / chan);
         static const bool cs = getenv("PILLARS_SCATTER_CS") != nullptr;
         const cudaError_t err = cs ? launch_pdl(k_scatter_wide<true, 8>, dim3(grid), dim3(bs), 0, st, feats, cell_row, f, plane,
-                                                tpp, chan, 0, bev, occ_prev, occ_next)
+                                                tpp, chan, 0, bev, occ_next)
                                    : launch_pdl(k_scatter_wide<false, 8>, dim3(grid), dim3(bs), 0, st, feats, cell_row, f,
-                                                plane, tpp, chan, 0, bev, occ_prev, occ_next);
+                                                plane, tpp, chan, 0, bev, occ_next);
         if (err != cudaSuccess) return err;
         note_launch();
         return cudaGetLastError();

@@ -1,6 +1,7 @@
 """Scatter stage on a reused canvas (EncodeBuffers' occupancy bitmaps), timed with the library's stage events.
-Regimes, one EncodeBuffers each: `same` (one batch, re-encoded), `cycle5` (5 batches cycling through the buffers) and
-`invalidated` (invalidate_canvas() before every call: the whole canvas is written, as without bitmaps).  Reports the 32-byte
+Regimes, one EncodeBuffers each: `empty` (an empty batch on a canvas whose bitmap is all clear: nothing is stored, the
+stage is one pass over the index map and the bitmaps), `same` (one batch, re-encoded), `cycle5` (5 batches cycling through
+the buffers) and `invalidated` (invalidate_canvas() before every call: the whole canvas is written, as without bitmaps).  Reports the 32-byte
 canvas sectors written (popcount of prev | next times the channels), the bytes that makes, the minimum traffic of the stage
 (those writes + the index map + the feature rows) and its rate against MEASURED_PEAKS.json.
 Usage: python profiles/scripts/scatter_reuse.py [out.json]   (B200; cfg2 and cfg4, fp32 canvas)"""
@@ -49,6 +50,7 @@ def run(name, dev, lib, peak):
         pts, offs = synth.make_batch(nb, model, 5, seed0=r * nb)
         batches.append((torch.from_numpy(pts).to(dev), torch.from_numpy(offs).to(dev)))
     n_max = max(p.shape[0] for p, _ in batches)
+    batches.append((torch.zeros((0, 5), dtype=torch.float32, device=dev), torch.zeros(nb + 1, dtype=torch.int32, device=dev)))
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(4)] for _ in range(CALLS)]
     for e4 in evs:  # torch only reports times of events it recorded itself once
         for e in e4:
@@ -57,7 +59,8 @@ def run(name, dev, lib, peak):
     arrs = [(ctypes.c_void_p * 4)(*[e.cuda_event for e in e4]) for e4 in evs]
     sectors_total = nb * ((nx * ny + 255) // 256) * 32
     out = {"grid": [nx, ny], "frames": nb, "canvas_bytes": 4 * F * nx * ny * nb}
-    for regime, pick in (("same", lambda k: 0), ("cycle5", lambda k: k % 5), ("invalidated", lambda k: k % 5)):
+    for regime, pick in (("empty", lambda k: 5), ("same", lambda k: 0), ("cycle5", lambda k: k % 5),
+                         ("invalidated", lambda k: k % 5)):
         bufs = ops.EncodeBuffers(n_max, nb, grid, F, dev)
         for k in range(6):
             ops.encode_bev(*batches[pick(k)], grid, pfn, buffers=bufs)
