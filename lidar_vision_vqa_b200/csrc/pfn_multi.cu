@@ -20,8 +20,6 @@
 // the max of layer 0, then layer 1 on [x, max]) and layer 0 is recomputed instead of stored, so pillars of any length
 // (the dynamic variant has no cap) need no scratch.  Not the headline kernel: it exists for coverage and is bound by
 // shared-memory traffic; the mainstream single-layer configuration runs pfn_stream.cu.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace pillars {
@@ -624,12 +622,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_pfn_multi_reg(const __grid_cons
 // picks the register-resident kernel when the configuration is one of its instantiations, else the general one
 bool launch_reg_variant(const MultiParams &p, const StackDev &sd, unsigned blocks, cudaStream_t st)
 {
-    static int off = -1;
-    if (off < 0) {
-        const char *e = getenv("PILLARS_MULTI_GENERIC");
-        off = e ? atoi(e) : 0;
-    }
-    if (off || !sd.use_abs || sd.with_dist) return false;
+    if (!sd.use_abs || sd.with_dist) return false;
     if (reinterpret_cast<uintptr_t>(p.points) % 4 != 0) return false;
     const bool two = sd.n_layers == 2;
     if (two && (sd.out[0] > 32 || sd.out[1] > 64)) return false;

@@ -28,7 +28,6 @@
 // stage lists those, and every warp that runs out of chunks takes entries from that list (warp-cooperative path reading the
 // records from global memory; 8-bit radix select of the P-th smallest point index when n > P).
 #include <cmath>
-#include <cstdlib>
 
 #include "group_common.cuh"
 
@@ -60,8 +59,9 @@ struct WalkParams {
     const uint4 *long_list;       // pillars of more than 32 points: {list start, n, row, x | y << 16} {z, -, -, -}
     const uint32_t *long_count;   // entries - 1
     uint32_t *long_cursor;        // next entry to process - 1 (shared by all warps of the grid)
-    uint32_t *chunk_cursor;       // next chunk of the shared pool - 1 (chunks of the pool are handed out one at a time)
-    uint32_t pool_256;            // share of the chunks (in 1/256) that forms the pool at the end of the list
+    uint32_t *chunk_cursor;       // two-layer stacks: next chunk - 1 (chunks are handed out one at a time)
+    int idx_bits;                 // bits of a point index; in the pad before `folded`, so that the fields below keep the
+                                  // 16-byte alignment that lets ptxas fetch them with 128-bit constant loads
     const float *folded;          // [PILLARS_FOLDED_FLOATS], see launch_fold_pfn
     float *pillar_features;
     const float *folded2;         // two-layer stacks: [32][64] per-point half of layer 1 | [32][64] pillar-max half | [64] shift
@@ -69,7 +69,6 @@ struct WalkParams {
     int sh_cells, sh_cells_xy, sh_nx;
     float vsz[3], off[3];
     float fx_scale[3], fx_inv[3];  // fixed-point scale of the mean sums per axis (a power of two) and its inverse
-    int idx_bits;
     unsigned long long *dbg;
 };
 
@@ -598,12 +597,12 @@ k_pillar_walk(const __grid_constant__ WalkParams p)
     // A warp owns a contiguous range of chunks.  (Handing chunks out one at a time through a grid-wide cursor was measured
     // SLOWER, 37-39 us against 33 us on cfg2, although per-warp times vary by +-40 %: neighbouring chunks then run on different
     // SMs and every window is fetched twice.)
-    // The LAST `pool_256`/256 of the chunks can be left unassigned: warps that finish their range take them one at a time
-    // from a grid-wide cursor.  One layer: measured without gain (cfg2 34.8 us static, 36.9 us with 19-62 % pooled, 38.9 us all
-    // pooled; cfg3 120.8 / 114.9 / 123.9 us; profiles/r02_walk_pool.txt) -- the late warps are not short of chunks, the SM is
-    // short of issue slots -- so the pool is empty by default (PILLARS_WALK_POOL).  Two-layer stacks are the opposite case (a
-    // chunk costs 5-10x more arithmetic, and 2.5x more when its pillars hold one point each; static ranges left the last
-    // warp running at 196 us when the first was done at 18 us): there every chunk comes from the cursor.
+    // Leaving the last chunks unassigned, for warps that finish their range to take one at a time from a grid-wide cursor,
+    // was measured without gain for one layer (cfg2 34.8 us static, 36.9 us with 19-62 % pooled, 38.9 us all pooled; cfg3
+    // 120.8 / 114.9 / 123.9 us; profiles/r02_walk_pool.txt) -- the late warps are not short of chunks, the SM is short of
+    // issue slots -- so one layer uses static ranges only.  Two-layer stacks are the opposite case (a chunk costs 5-10x more
+    // arithmetic, and 2.5x more when its pillars hold one point each; static ranges left the last warp running at 196 us when
+    // the first was done at 18 us): there every chunk comes from the cursor.
     const uint32_t gw = blockIdx.x * kWarps + warp, n_warps = gridDim.x * kWarps;
     // Bulk phase: the cursor is read one chunk ahead (lane 0 keeps the reply of the atomic issued a chunk earlier) and the
     // next window is fetched during the current chunk, so a warp never waits for either round trip.  Tail phase (the last
@@ -615,14 +614,14 @@ k_pillar_walk(const __grid_constant__ WalkParams p)
     uint32_t ahead = 0;
     bool primed = false;
     auto grab = [&]() {
-        if (!kTwo && p.pool_256 == 0u) return 0x7FFFFFFFu;  // no pool: nothing to wait for
+        if (!kTwo) return 0x7FFFFFFFu;  // one layer: no pool, nothing to wait for
         if (!primed && lane == 0) ahead = atomicAdd(p.chunk_cursor, 1u) + 1u;  // the cursor starts at 0xFFFFFFFF
         const uint32_t i = __shfl_sync(kFull, ahead, 0);
         primed = i < bulk_end;
         if (primed && lane == 0) ahead = atomicAdd(p.chunk_cursor, 1u) + 1u;
         return i;
     };
-    const uint32_t n_static = kTwo ? 0u : n_chunks - static_cast<uint32_t>((static_cast<unsigned long long>(n_chunks) * p.pool_256) >> 8);
+    const uint32_t n_static = kTwo ? 0u : n_chunks;
     uint32_t cur = static_cast<uint32_t>(static_cast<unsigned long long>(n_static) * gw / n_warps);
     const uint32_t c_end = static_cast<uint32_t>(static_cast<unsigned long long>(n_static) * (gw + 1) / n_warps);
     bool pooled = false;
@@ -996,12 +995,6 @@ __global__ void k_fold_pfn(const float *__restrict__ weight, const float *__rest
     folded[12 * 64 + o] = fmaxf(sh, 0.f);
 }
 
-int env_int(const char *name, int dflt)
-{
-    const char *e = getenv(name);
-    return e ? atoi(e) : dflt;
-}
-
 }  // namespace
 
 cudaError_t launch_fold_pfn(const PfnDev &pfn, int c_point, int c_in, float *folded, cudaStream_t st, int f_out)
@@ -1104,46 +1097,20 @@ cudaError_t launch_pillar_features_stream(const FastJob &job, const float *folde
         p.fx_scale[k] = static_cast<float>(std::ldexp(1.0, s));
         p.fx_inv[k] = static_cast<float>(std::ldexp(1.0, -s));
     }
-    // Persistent warps, at most one full wave; each takes 32-position chunks from the grid-wide cursor.
+    // Persistent warps, one per two chunks, at most one full wave of `occ` CTAs per SM (the kernel's minimum-blocks bound).
     const int sms = current_sm_count();
-    static const int occ = [] {
-        const int v = env_int("PILLARS_WALK_OCC", 5);
-        return v < 5 ? 5 : (v > 8 ? 8 : v);
-    }();
-    static const int pool = [] {
-        const int v = env_int("PILLARS_WALK_POOL", 0);
-        return v < 0 ? 0 : (v > 256 ? 256 : v);
-    }();
-    p.pool_256 = job.folded2 ? 256u : static_cast<uint32_t>(pool);
     constexpr int kWarps = 4;
     const int64_t chunks = (job.n + 31) / 32;  // upper bound: listed points <= n
-    int64_t warps = (chunks + 1) / 2;
-    const int64_t wave = static_cast<int64_t>(sms) * occ * kWarps;
-    if (warps > wave) warps = wave;
-    const unsigned grid = static_cast<unsigned>((warps + kWarps - 1) / kWarps);
+    auto grid = [&](int occ) {
+        return dim3(static_cast<unsigned>((tmin<int64_t>((chunks + 1) / 2, static_cast<int64_t>(sms) * occ * kWarps) + kWarps - 1) / kWarps));
+    };
     cudaError_t err;
-    if (job.dynamic) {  // DynamicPillarVFE (one or two layers)
-        const unsigned g2 = static_cast<unsigned>((tmin<int64_t>((chunks + 1) / 2, static_cast<int64_t>(sms) * 3 * kWarps) + kWarps - 1) / kWarps);
-        err = job.folded2 ? launch_pdl(k_pillar_walk<kWarps, 3, true, true>, dim3(g2), dim3(32 * kWarps), 0, st, p)
-                          : launch_pdl(k_pillar_walk<kWarps, 5, false, true>, dim3(static_cast<unsigned>((tmin<int64_t>((chunks + 1) / 2, static_cast<int64_t>(sms) * 5 * kWarps) + kWarps - 1) / kWarps)),
-                                       dim3(32 * kWarps), 0, st, p);
-        if (err != cudaSuccess) return err;
-        note_launch();
-        return cudaGetLastError();
-    }
-    if (job.folded2) {  // two-layer stack: 64 more weight registers per lane
-        err = launch_pdl(k_pillar_walk<kWarps, 3, true>, dim3(static_cast<unsigned>((tmin<int64_t>((chunks + 1) / 2, static_cast<int64_t>(sms) * 3 * kWarps) + kWarps - 1) / kWarps)),
-                         dim3(32 * kWarps), 0, st, p);
-        if (err != cudaSuccess) return err;
-        note_launch();
-        return cudaGetLastError();
-    }
-    switch (occ) {
-    case 8: err = launch_pdl(k_pillar_walk<kWarps, 8>, dim3(grid), dim3(32 * kWarps), 0, st, p); break;
-    case 7: err = launch_pdl(k_pillar_walk<kWarps, 7>, dim3(grid), dim3(32 * kWarps), 0, st, p); break;
-    case 6: err = launch_pdl(k_pillar_walk<kWarps, 6>, dim3(grid), dim3(32 * kWarps), 0, st, p); break;
-    default: err = launch_pdl(k_pillar_walk<kWarps, 5>, dim3(grid), dim3(32 * kWarps), 0, st, p); break;
-    }
+    if (job.dynamic)  // DynamicPillarVFE (one or two layers)
+        err = job.folded2 ? launch_pdl(k_pillar_walk<kWarps, 3, true, true>, grid(3), dim3(32 * kWarps), 0, st, p)
+                          : launch_pdl(k_pillar_walk<kWarps, 5, false, true>, grid(5), dim3(32 * kWarps), 0, st, p);
+    else  // PillarVFE; a two-layer stack has 64 more weight registers per lane: 3 CTAs per SM
+        err = job.folded2 ? launch_pdl(k_pillar_walk<kWarps, 3, true>, grid(3), dim3(32 * kWarps), 0, st, p)
+                          : launch_pdl(k_pillar_walk<kWarps, 5>, grid(5), dim3(32 * kWarps), 0, st, p);
     if (err != cudaSuccess) return err;
     note_launch();
     return cudaGetLastError();

@@ -20,8 +20,6 @@
 // profiles/r01_scatter_variants.md.
 #include <cuda_fp16.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace pillars {
@@ -78,7 +76,7 @@ __global__ void k_rebase_segments(int32_t *__restrict__ coords, int n_seg, int64
 // at a time, the feature rows of its occupied cells with two 16-byte loads per row and composes one float4 per channel.
 // Eight passes of one L2 round trip each per 32 KB keep the SM far above its share of HBM write bandwidth with a handful
 // of resident warps, so the kernel runs at the speed of the write stream.
-template <bool VEC, int CPP, bool PIPE>
+template <bool VEC>
 __global__ void __launch_bounds__(kThreads)
 k_scatter_plain(const float *__restrict__ feats, const int32_t *__restrict__ cell_row, int f, int64_t plane,
                 int tiles_per_plane, float *__restrict__ bev)
@@ -115,8 +113,8 @@ k_scatter_plain(const float *__restrict__ feats, const int32_t *__restrict__ cel
     }
     if (!inb) return;
     if (VEC) {
-        constexpr int kV = CPP / 4;  // 16-byte loads per row and pass
-        float4 cur[4][kV], nxt[4][kV];
+        constexpr int kV = 2;  // 16-byte loads per row and pass of 8 channels
+        float4 cur[4][kV];
         auto fetch = [&](float4 (&dstv)[4][kV], int c0) {
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
@@ -130,8 +128,7 @@ k_scatter_plain(const float *__restrict__ feats, const int32_t *__restrict__ cel
             }
         };
         fetch(cur, 0);
-        for (int c0 = 0; c0 < f; c0 += CPP) {
-            if (PIPE && c0 + CPP < f) fetch(nxt, c0 + CPP);  // next pass in flight while this one is stored
+        for (int c0 = 0; c0 < f; c0 += 8) {
 #pragma unroll
             for (int q = 0; q < kV; ++q) {
                 __stcs(reinterpret_cast<float4 *>(dst + (c0 + 4 * q + 0) * plane), make_float4(cur[0][q].x, cur[1][q].x, cur[2][q].x, cur[3][q].x));
@@ -139,16 +136,7 @@ k_scatter_plain(const float *__restrict__ feats, const int32_t *__restrict__ cel
                 __stcs(reinterpret_cast<float4 *>(dst + (c0 + 4 * q + 2) * plane), make_float4(cur[0][q].z, cur[1][q].z, cur[2][q].z, cur[3][q].z));
                 __stcs(reinterpret_cast<float4 *>(dst + (c0 + 4 * q + 3) * plane), make_float4(cur[0][q].w, cur[1][q].w, cur[2][q].w, cur[3][q].w));
             }
-            if (c0 + CPP < f) {
-                if (PIPE) {
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)
-#pragma unroll
-                        for (int q = 0; q < kV; ++q) cur[k][q] = nxt[k][q];
-                } else {
-                    fetch(cur, c0 + CPP);
-                }
-            }
+            if (c0 + 8 < f) fetch(cur, c0 + 8);
         }
     } else {
         for (int c = 0; c < f; ++c) __stcs(dst + c * plane, r[0] >= 0 ? __ldg(feats + static_cast<int64_t>(r[0]) * f + c) : 0.f);
@@ -169,21 +157,18 @@ __device__ __forceinline__ void stg256(float *p, float a, float b, float c, floa
                  "f"(d), "f"(e), "f"(f), "f"(g), "f"(h)
                  : "memory");
 }
-__device__ __forceinline__ void stg256_cs(float *p, float a, float b, float c, float d, float e, float f, float g, float h)
-{
-    asm volatile("st.global.cs.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d),
-                 "f"(e), "f"(f), "f"(g), "f"(h)
-                 : "memory");
-}
 
-// Work split: a CTA owns blockDim.x * 8 consecutive cells x `chan_per_cta` channels (a multiple of 8).  With 8 channels per
-// CTA the canvas is written as few long sequential streams (measured with profiles/micro/fill_patterns.cu on B200: 64
-// channel-strided streams per thread 164 us for the 1 GiB canvas, 8 channels x 8 KB runs per CTA 149 us, linear fill 146 us);
-// the CTAs of one cell tile then each read one 32-byte sector of every pillar row, so no feature byte is fetched twice.
+// Work split: a CTA owns blockDim.x * 8 consecutive cells x `chan_per_cta` channels (a multiple of 8; every launch uses 8).
+// With 8 channels per CTA the canvas is written as few long sequential streams (measured with
+// profiles/micro/fill_patterns.cu on B200: 64 channel-strided streams per thread 164 us for the 1 GiB canvas, 8 channels x
+// 8 KB runs per CTA 149 us, linear fill 146 us); the CTAs of one cell tile then each read one 32-byte sector of every
+// pillar row, so no feature byte is fetched twice.
 // tile_major != 0: consecutive CTAs are the channel groups of one cell tile (index map and feature rows are shared by CTAs
 // that run together); 0: consecutive CTAs walk the plane for one channel group.
 // occ_next != NULL: the channel group 0 CTAs record each lane's "any cell occupied" test into occ_next.
-template <bool CS, int CPP>
+// chan_per_cta and tile_major stay runtime parameters: with both folded to constants (8, 0) the invalidated cfg2 canvas
+// took 173.1 us against 171.0-171.1 us, in 4 alternated rounds on one B200 at 1000 W (same loads and stores, scheduled
+// differently); cfg4 was unchanged.
 __global__ void __launch_bounds__(kThreads)
 k_scatter_wide(const float *__restrict__ feats, const int32_t *__restrict__ cell_row, int f, int64_t plane,
                int tiles_per_plane, int chan_per_cta, int tile_major, float *__restrict__ bev, uint32_t *__restrict__ occ_next)
@@ -216,20 +201,16 @@ k_scatter_wide(const float *__restrict__ feats, const int32_t *__restrict__ cell
     for (int k = 0; k < 8; ++k) any |= r[k] >= 0;
     const int c_begin = cg * chan_per_cta, c_end = c_begin + chan_per_cta;
     float *dst = bev + (static_cast<int64_t>(b) * f) * plane + cell0;
-    auto store = [&](float *p, float a, float b2, float c, float d, float e, float f2, float g, float h) {
-        if (CS) stg256_cs(p, a, b2, c, d, e, f2, g, h);
-        else stg256(p, a, b2, c, d, e, f2, g, h);
-    };
     const uint32_t now = __ballot_sync(0xffffffffu, any);
     if (occ_next && cg == 0 && (threadIdx.x & 31) == 0 && inb) occ_next[b * occ_words(plane) + (cell0 >> 8)] = now;
     if (!inb) return;
     if (now == 0) {
 #pragma unroll 8
-        for (int c = c_begin; c < c_end; ++c) store(dst + c * plane, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f);
+        for (int c = c_begin; c < c_end; ++c) stg256(dst + c * plane, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f);
         return;
     }
-    constexpr int kV = CPP / 4;  // 16-byte loads per row and pass
-    for (int c0 = c_begin; c0 < c_end; c0 += CPP) {
+    constexpr int kV = 2;  // 16-byte loads per row and pass of 8 channels
+    for (int c0 = c_begin; c0 < c_end; c0 += 8) {
         float4 v[8][kV];
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
@@ -244,10 +225,10 @@ k_scatter_wide(const float *__restrict__ feats, const int32_t *__restrict__ cell
 #pragma unroll
         for (int q = 0; q < kV; ++q) {
             float *d = dst + (c0 + 4 * q) * plane;
-            store(d, v[0][q].x, v[1][q].x, v[2][q].x, v[3][q].x, v[4][q].x, v[5][q].x, v[6][q].x, v[7][q].x);
-            store(d + plane, v[0][q].y, v[1][q].y, v[2][q].y, v[3][q].y, v[4][q].y, v[5][q].y, v[6][q].y, v[7][q].y);
-            store(d + 2 * plane, v[0][q].z, v[1][q].z, v[2][q].z, v[3][q].z, v[4][q].z, v[5][q].z, v[6][q].z, v[7][q].z);
-            store(d + 3 * plane, v[0][q].w, v[1][q].w, v[2][q].w, v[3][q].w, v[4][q].w, v[5][q].w, v[6][q].w, v[7][q].w);
+            stg256(d, v[0][q].x, v[1][q].x, v[2][q].x, v[3][q].x, v[4][q].x, v[5][q].x, v[6][q].x, v[7][q].x);
+            stg256(d + plane, v[0][q].y, v[1][q].y, v[2][q].y, v[3][q].y, v[4][q].y, v[5][q].y, v[6][q].y, v[7][q].y);
+            stg256(d + 2 * plane, v[0][q].z, v[1][q].z, v[2][q].z, v[3][q].z, v[4][q].z, v[5][q].z, v[6][q].z, v[7][q].z);
+            stg256(d + 3 * plane, v[0][q].w, v[1][q].w, v[2][q].w, v[3][q].w, v[4][q].w, v[5][q].w, v[6][q].w, v[7][q].w);
         }
     }
 }
@@ -495,11 +476,8 @@ cudaError_t launch_scatter(const float *feats, const int32_t *cell_row, int nb, 
         constexpr int bs = 128, chan = 8;
         const int tpp = static_cast<int>((plane + bs * 8 - 1) / (bs * 8));
         const unsigned grid = static_cast<unsigned>(nb) * tpp * (f / chan);
-        static const bool cs = getenv("PILLARS_SCATTER_CS") != nullptr;
-        const cudaError_t err = cs ? launch_pdl(k_scatter_wide<true, 8>, dim3(grid), dim3(bs), 0, st, feats, cell_row, f, plane,
-                                                tpp, chan, 0, bev, occ_next)
-                                   : launch_pdl(k_scatter_wide<false, 8>, dim3(grid), dim3(bs), 0, st, feats, cell_row, f,
-                                                plane, tpp, chan, 0, bev, occ_next);
+        const cudaError_t err = launch_pdl(k_scatter_wide, dim3(grid), dim3(bs), 0, st, feats, cell_row, f, plane, tpp, chan,
+                                           0, bev, occ_next);
         if (err != cudaSuccess) return err;
         note_launch();
         return cudaGetLastError();
@@ -512,10 +490,10 @@ cudaError_t launch_scatter(const float *feats, const int32_t *cell_row, int nb, 
     }
     if (vec_ok) {
         const int tpp = static_cast<int>((plane + kThreads * 4 - 1) / (kThreads * 4));
-        k_scatter_plain<true, 8, false><<<static_cast<unsigned>(nb) * tpp, kThreads, 0, st>>>(feats, cell_row, f, plane, tpp, bev);
+        k_scatter_plain<true><<<static_cast<unsigned>(nb) * tpp, kThreads, 0, st>>>(feats, cell_row, f, plane, tpp, bev);
     } else {
         const int tpp = static_cast<int>((plane + kThreads - 1) / kThreads);
-        k_scatter_plain<false, 8, false><<<static_cast<unsigned>(nb) * tpp, kThreads, 0, st>>>(feats, cell_row, f, plane, tpp, bev);
+        k_scatter_plain<false><<<static_cast<unsigned>(nb) * tpp, kThreads, 0, st>>>(feats, cell_row, f, plane, tpp, bev);
     }
     note_launch();
     return cudaGetLastError();

@@ -1,6 +1,5 @@
-import os, sys, numpy as np, torch
+import sys, numpy as np, torch
 sys.path.insert(0, '/root/repo')
-os.environ.setdefault('PILLARS_WALK_EXP','64')
 import lidar_vision_vqa_b200 as L
 from lidar_vision_vqa_b200 import ops, synth
 from oracle import pillar_oracle as po

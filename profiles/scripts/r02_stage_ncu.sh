@@ -1,5 +1,4 @@
 set -x
-for cpw in 1 2 3 4 6; do PILLARS_WALK_CPW=$cpw python profiles/tune_stage.py auto 16; done
 python profiles/tune_stage.py auto 16 > gpurun_out/plain.log 2>&1 && \
 ncu --set full --clock-control none --import-source on -k regex:'k_insert_dense|k_scan_dense|k_place_dense|k_pillar_walk' -s 40 -c 4 -o gpurun_out/r02_group_feat python profiles/tune_stage.py auto 16 > gpurun_out/ncu.log 2>&1
 tail -3 gpurun_out/ncu.log

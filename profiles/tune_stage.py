@@ -1,5 +1,5 @@
-"""Per-stage timing of the fused path for one configuration (env knobs select kernel variants); prints one line.
-Usage: [PILLARS_SCATTER_CELLS=..] python profiles/tune_stage.py [variant] [frames] [--empty] [--memset]"""
+"""Per-stage timing of the fused path for one configuration; prints one line.
+Usage: python profiles/tune_stage.py [variant] [frames] [--empty] [--memset]"""
 import ctypes
 import os
 import sys
@@ -61,6 +61,5 @@ if "--memset" in sys.argv:
         s.record(); bufs.bev.copy_(src); e.record(); torch.cuda.synchronize(); t2.append(s.elapsed_time(e) * 1e3)
     gb = bufs.bev.numel() * 4 / 1e9
     extra = f" | memset {min(t):.1f}us = {gb / min(t) * 1e6:.0f} GB/s | copy {min(t2):.1f}us = {2 * gb / min(t2) * 1e6:.0f} GB/s"
-env = {k: v for k, v in os.environ.items() if k.startswith("PILLARS_")}
 gbs = bufs.bev.numel() * 4 / (med[2] * 1e-6) / 1e9
-print(f"{variant:7s} nb={nb} {env} group={med[0]:.1f}us feat={med[1]:.1f}us scatter={med[2]:.1f}us ({gbs:.0f} GB/s write){extra}", flush=True)
+print(f"{variant:7s} nb={nb} group={med[0]:.1f}us feat={med[1]:.1f}us scatter={med[2]:.1f}us ({gbs:.0f} GB/s write){extra}", flush=True)
