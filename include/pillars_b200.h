@@ -278,7 +278,8 @@ size_t pillars_workspace_cell_row_offset(int64_t n_points, int32_t n_frames, con
  * One layer = Conv2d / ConvTranspose2d (bias=False) + eval-mode BatchNorm2d(eps=1e-3) + ReLU, as ONE implicit-GEMM kernel on
  * the tcgen05 tensor cores (tf32 operands, fp32 accumulation: what nn.Conv2d itself does on this GPU under PyTorch's default
  * cudnn.allow_tf32).  Activations between layers are NHWC fp32.  Supported: c_in a multiple of 32; c_out in {64,128,256};
- * (k, stride, pad) in {(3,1,1), (1,1,0), (3,2,1), (2,2,0)}; up in {2, 4} = ConvTranspose2d(kernel = stride = up), given as k = 1. */
+ * (k, stride, pad) in {(3,1,1), (1,1,0), (3,2,1), (2,2,0)}; up in {2, 4} = ConvTranspose2d(kernel = stride = up), given as k = 1,
+ * with c_out in {64, 128} only.  pillars_conv_weight_bytes returns 0 for every other shape. */
 typedef struct {
     int32_t c_in, c_out;
     int32_t k, stride, pad;

@@ -795,7 +795,8 @@ int pillars_bev_tokens_dense(const float *bev, int32_t n_frames, int32_t h, int3
 static bool conv_ok(const pillars_conv_t *cv)
 {
     if (!cv || cv->c_in < 32 || cv->c_in % 32 != 0 || (cv->c_out != 64 && cv->c_out != 128 && cv->c_out != 256)) return false;
-    if (cv->up == 2 || cv->up == 4) return cv->k == 1 && cv->stride == 1 && cv->pad == 0;
+    // transposed: the two dx phases share one accumulator of 2 * c_out columns, and no kernel is instantiated for 512
+    if (cv->up == 2 || cv->up == 4) return cv->c_out != 256 && cv->k == 1 && cv->stride == 1 && cv->pad == 0;
     if (cv->up != 1) return false;
     return (cv->k == 3 && cv->stride == 1 && cv->pad == 1) || (cv->k == 1 && cv->stride == 1 && cv->pad == 0) ||
            (cv->k == 3 && cv->stride == 2 && cv->pad == 1) || (cv->k == 2 && cv->stride == 2 && cv->pad == 0);

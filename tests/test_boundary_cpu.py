@@ -233,6 +233,26 @@ def test_backbone_has_no_cpu_or_training_path():
         m.eval()({"spatial_features": torch.zeros(1, 64, 32, 32)})
 
 
+def test_conv_weight_bytes_only_for_launchable_transposed_shapes(lib):
+    """A ConvTranspose2d keeps its two dx phases side by side in one accumulator of 2 * c_out columns, and the kernel is
+    instantiated up to 256: c_out = 256 must be refused by the size query, so that `prepare` raises NotImplementedError before
+    it touches a device, instead of the launch failing later."""
+    from lidar_vision_vqa_b200 import _native
+    from lidar_vision_vqa_b200.backbone import _Layer
+
+    def nbytes(c_in, c_out, up):
+        cv = _native.PillarsConv(c_in, c_out, 1, 1, 0, up, 1, 0)
+        return lib.pillars_conv_weight_bytes(ctypes.byref(cv))
+
+    assert nbytes(256, 256, 2) == 0 and nbytes(256, 256, 4) == 0
+    # [up * up phases][c_in / 32 channel blocks][c_out rows of 128 bytes]
+    assert nbytes(256, 128, 2) == 4 * (256 // 32) * 128 * 128
+    assert nbytes(128, 64, 4) == 16 * (128 // 32) * 64 * 128
+    layer = _Layer(torch.nn.ConvTranspose2d(256, 256, 2, stride=2, bias=False), torch.nn.BatchNorm2d(256), True)
+    with pytest.raises(NotImplementedError):
+        layer.prepare(torch.device("cpu"))
+
+
 def test_backbone_output_shape_and_flop_count_match_the_reference_module():
     """`output_shape` against the reference module's actual output, `bench.backbone_flops` against a count over its layers."""
     import importlib.util
