@@ -278,13 +278,15 @@ size_t pillars_workspace_cell_row_offset(int64_t n_points, int32_t n_frames, con
  * One layer = Conv2d / ConvTranspose2d (bias=False) + eval-mode BatchNorm2d(eps=1e-3) + ReLU, as ONE implicit-GEMM kernel on
  * the tcgen05 tensor cores (tf32 operands, fp32 accumulation: what nn.Conv2d itself does on this GPU under PyTorch's default
  * cudnn.allow_tf32).  Activations between layers are NHWC fp32.  Supported: c_in a multiple of 32; c_out in {64,128,256};
- * (k, stride, pad) in {(3,1,1), (1,1,0), (3,2,1), (2,2,0)}; up in {2, 4} = ConvTranspose2d(kernel = stride = up), given as k = 1,
- * with c_out in {64, 128} only.  pillars_conv_weight_bytes returns 0 for every other shape. */
+ * (k, stride, pad) in {(3,1,1), (1,1,0), (3,2,1), (2,2,0), (1,2,0)}; up in {2, 4} = ConvTranspose2d(kernel = stride = up), given
+ * as k = 1, with c_out in {64, 128} only.  pillars_conv_weight_bytes returns 0 for every other shape.  (1,2,0) is the 1x1
+ * stride-2 projection of a ResNet BasicBlock (BaseBEVResBackbone's downsample_layer).  relu = 0 leaves the BatchNorm output as
+ * it is, on every geometry (the projection branch has no ReLU). */
 typedef struct {
     int32_t c_in, c_out;
     int32_t k, stride, pad;
     int32_t up;        /* 1 = convolution; 2 / 4 = transposed convolution with kernel = stride = up (k = 1, stride = 1, pad = 0) */
-    int32_t relu;      /* apply ReLU after the BatchNorm shift */
+    int32_t relu;      /* apply ReLU after the BatchNorm shift (and after the residual, if any); 0 = no ReLU */
     int32_t round_out; /* store tf32-rounded activations (for layers that feed another layer of this kind) */
 } pillars_conv_t;
 
@@ -306,6 +308,16 @@ int pillars_conv_prepare(const pillars_conv_t *cv, const float *weight, const fl
 int pillars_conv_forward(const pillars_conv_t *cv, const void *image, const float *bn_shift, const float *in_nhwc,
                          const float *rows, const int32_t *cell_row, int32_t n_frames, int32_t h_in, int32_t w_in, float *out,
                          int32_t out_c_total, int32_t out_c_off, int32_t out_nchw, uint32_t *error_word, void *stream);
+
+/* pillars_conv_forward with a residual (ResNet BasicBlock: out = relu(bn(conv(x)) + residual), BaseBEVResBackbone):
+ * residual_nhwc is fp32, laid out exactly like out (out[b, oy, ox, out_c_off + n] <- ... + residual_nhwc[b, oy, ox, out_c_off + n],
+ * out_c_total channels per pixel) and 16-byte aligned; it is added after the BatchNorm shift and before the ReLU and the
+ * tf32 rounding.  Only plain convolutions (up == 1) with NHWC output (out_nchw == 0) take one: PILLARS_E_UNSUPPORTED otherwise.
+ * residual_nhwc may not overlap out. */
+int pillars_conv_forward_residual(const pillars_conv_t *cv, const void *image, const float *bn_shift, const float *in_nhwc,
+                                  const float *rows, const int32_t *cell_row, int32_t n_frames, int32_t h_in, int32_t w_in,
+                                  float *out, int32_t out_c_total, int32_t out_c_off, int32_t out_nchw, const float *residual_nhwc,
+                                  uint32_t *error_word, void *stream);
 
 /* Dense canvas [n_frames, c, h, w] -> (rows of its non-zero cells, index map): the input form pillars_conv_forward and the
  * tokeniser gather from.  rows must hold n_frames*h*w*c floats in the worst case; counter is one device uint32 (row count). */

@@ -4,7 +4,7 @@ behind the reference's own module interface.  See DESIGN.md and include/pillars_
 from ._native import NativeLibraryError  # noqa: F401
 from .modules import (MAP_TO_BEV_REGISTRY, VFE_REGISTRY, DynamicPillarVFE, DynamicPillarVFESimple2D,  # noqa: F401
                       PFNLayer, PillarVFE, PillarVFEFromPoints, PointPillarScatter, PointPillarScatter3d, VFETemplate)
-from .backbone import BaseBEVBackbone  # noqa: F401
+from .backbone import BaseBEVBackbone, BaseBEVResBackbone  # noqa: F401
 from .ops import EncodeBuffers, GridSpec, PfnParams, PfnStackParams  # noqa: F401
 
 __version__ = "0.1.0"

@@ -40,6 +40,7 @@ EXPORTED_SYMBOLS = (
     "pillars_conv_weight_bytes",
     "pillars_conv_prepare",
     "pillars_conv_forward",
+    "pillars_conv_forward_residual",
     "pillars_canvas_to_rows",
     "pillars_set_canvas_occupancy",
 )
@@ -169,6 +170,10 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
     lib.pillars_conv_forward.restype = c_int
     lib.pillars_conv_forward.argtypes = [POINTER(PillarsConv), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32,
                                          c_int32, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p]
+    lib.pillars_conv_forward_residual.restype = c_int
+    lib.pillars_conv_forward_residual.argtypes = [POINTER(PillarsConv), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
+                                                  c_int32, c_int32, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p,
+                                                  c_void_p]
     lib.pillars_canvas_to_rows.restype = c_int
     lib.pillars_canvas_to_rows.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]
     lib.pillars_rebase_segments.restype = c_int

@@ -799,7 +799,8 @@ static bool conv_ok(const pillars_conv_t *cv)
     if (cv->up == 2 || cv->up == 4) return cv->c_out != 256 && cv->k == 1 && cv->stride == 1 && cv->pad == 0;
     if (cv->up != 1) return false;
     return (cv->k == 3 && cv->stride == 1 && cv->pad == 1) || (cv->k == 1 && cv->stride == 1 && cv->pad == 0) ||
-           (cv->k == 3 && cv->stride == 2 && cv->pad == 1) || (cv->k == 2 && cv->stride == 2 && cv->pad == 0);
+           (cv->k == 3 && cv->stride == 2 && cv->pad == 1) || (cv->k == 2 && cv->stride == 2 && cv->pad == 0) ||
+           (cv->k == 1 && cv->stride == 2 && cv->pad == 0);
 }
 
 size_t pillars_conv_weight_bytes(const pillars_conv_t *cv)
@@ -821,9 +822,10 @@ int pillars_conv_prepare(const pillars_conv_t *cv, const float *weight, const fl
     return 0;
 }
 
-int pillars_conv_forward(const pillars_conv_t *cv, const void *image, const float *bn_shift, const float *in_nhwc,
-                         const float *rows, const int32_t *cell_row, int32_t n_frames, int32_t h_in, int32_t w_in, float *out,
-                         int32_t out_c_total, int32_t out_c_off, int32_t out_nchw, uint32_t *error_word, void *stream)
+static int conv_forward(const pillars_conv_t *cv, const void *image, const float *bn_shift, const float *in_nhwc,
+                        const float *rows, const int32_t *cell_row, int32_t n_frames, int32_t h_in, int32_t w_in, float *out,
+                        int32_t out_c_total, int32_t out_c_off, int32_t out_nchw, const float *residual_nhwc, uint32_t *error_word,
+                        void *stream)
 {
     if (!conv_ok(cv)) return fail(PILLARS_E_UNSUPPORTED, "convolution shape outside the instantiated set");
     if (!image || !bn_shift || !out) return fail(PILLARS_E_BADARG, "NULL image / shift / out");
@@ -831,8 +833,8 @@ int pillars_conv_forward(const pillars_conv_t *cv, const void *image, const floa
     if (n_frames < 0 || h_in < 1 || w_in < 1) return fail(PILLARS_E_BADARG, "bad image shape");
     if (static_cast<int64_t>(n_frames) * h_in * w_in >= (1ll << 31)) return fail(PILLARS_E_UNSUPPORTED, "more than 2^31 input pixels");
     const auto misaligned = [](const void *q) { return q && reinterpret_cast<uintptr_t>(q) % 16 != 0; };
-    if (misaligned(image) || misaligned(in_nhwc) || misaligned(rows) || misaligned(out))
-        return fail(PILLARS_E_BADARG, "image / activations / rows / out must be 16-byte aligned");
+    if (misaligned(image) || misaligned(in_nhwc) || misaligned(rows) || misaligned(out) || misaligned(residual_nhwc))
+        return fail(PILLARS_E_BADARG, "image / activations / rows / out / residual must be 16-byte aligned");
     if (out_c_off < 0 || out_c_off + cv->c_out > out_c_total || (out_nchw == 0 && (out_c_total % 4 != 0 || out_c_off % 4 != 0)))
         return fail(PILLARS_E_BADARG, "bad output channel window");
     g_launches = 0;
@@ -862,11 +864,32 @@ int pillars_conv_forward(const pillars_conv_t *cv, const void *image, const floa
     j.relu = cv->relu;
     j.round_out = cv->round_out;
     j.error = error_word;
+    j.res = residual_nhwc;
     cudaError_t e = launch_conv_umma(j, static_cast<cudaStream_t>(stream));
     if (e == cudaErrorInvalidValue) return fail(PILLARS_E_UNSUPPORTED, "convolution geometry not instantiated");
     if (e != cudaSuccess) return cuda_fail(e, "conv_forward");
     g_launches_last = g_launches;
     return 0;
+}
+
+int pillars_conv_forward(const pillars_conv_t *cv, const void *image, const float *bn_shift, const float *in_nhwc,
+                         const float *rows, const int32_t *cell_row, int32_t n_frames, int32_t h_in, int32_t w_in, float *out,
+                         int32_t out_c_total, int32_t out_c_off, int32_t out_nchw, uint32_t *error_word, void *stream)
+{
+    return conv_forward(cv, image, bn_shift, in_nhwc, rows, cell_row, n_frames, h_in, w_in, out, out_c_total, out_c_off, out_nchw,
+                        nullptr, error_word, stream);
+}
+
+int pillars_conv_forward_residual(const pillars_conv_t *cv, const void *image, const float *bn_shift, const float *in_nhwc,
+                                  const float *rows, const int32_t *cell_row, int32_t n_frames, int32_t h_in, int32_t w_in,
+                                  float *out, int32_t out_c_total, int32_t out_c_off, int32_t out_nchw, const float *residual_nhwc,
+                                  uint32_t *error_word, void *stream)
+{
+    if (!residual_nhwc) return fail(PILLARS_E_BADARG, "NULL residual");
+    if (cv && (cv->up != 1 || out_nchw != 0))
+        return fail(PILLARS_E_UNSUPPORTED, "a residual is added only by a plain (not transposed) convolution with NHWC output");
+    return conv_forward(cv, image, bn_shift, in_nhwc, rows, cell_row, n_frames, h_in, w_in, out, out_c_total, out_c_off, out_nchw,
+                        residual_nhwc, error_word, stream);
 }
 
 int pillars_canvas_to_rows(const float *bev, int32_t n_frames, int32_t c, int32_t h, int32_t w, int32_t *cell_row, float *rows,

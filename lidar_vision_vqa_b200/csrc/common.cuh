@@ -409,11 +409,12 @@ struct ConvJob {
     const float *shift;        // [c_out]
     float *out;
     int nb, h_in, w_in, c_in, c_out;
-    int k, stride, pad;        // (3,1,1) (3,2,1) (2,2,0) (1,1,0)
+    int k, stride, pad;        // (3,1,1) (3,2,1) (2,2,0) (1,1,0) (1,2,0)
     int up;                    // 1, or 2 = transposed convolution with kernel = stride = 2 (k = 1 per phase)
     int out_c_total, out_c_off, out_nchw;
     int relu, round_out;       // round_out: store tf32-rounded values (the next layer's tensor cores would truncate them)
     uint32_t *error;
+    const float *res;          // NULL, or the residual added before the ReLU: NHWC fp32 laid out like out (out_nchw == 0, up == 1)
 };
 cudaError_t launch_conv_wimg(const float *weight, const float *scale, int c_in, int c_out, int k, int up, float *img, cudaStream_t st);
 cudaError_t launch_conv_umma(const ConvJob &job, cudaStream_t st);

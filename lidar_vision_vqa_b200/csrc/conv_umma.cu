@@ -165,6 +165,9 @@ struct ConvParams {
     int pair;                 // transposed convolution: two dx phases per accumulator (N = 2 * c_out)
     uint32_t *error;          // device word: nonzero when a bounded wait expired
     unsigned long long *timeline;  // measurement hook (pillars_set_debug_times): one CTA's phase stamps, %globaltimer ns
+    // residual kernels (RES): NHWC fp32, laid out exactly like `out` (same pixel pitch, same channel window), added before the
+    // ReLU.  (last, so that the kernels without it keep every parameter offset)
+    const float *res;
 };
 
 __device__ __forceinline__ void tl_stamp(const ConvParams &p, int slot)
@@ -179,7 +182,9 @@ __device__ __forceinline__ void tl_stamp(const ConvParams &p, int slot)
 // Persistent: a CTA walks over tile sets (tile = blockIdx.x, += gridDim.x).  With NB = 2 the accumulator is double buffered in
 // tensor memory, so the epilogue of tile set i (warps 6-9) runs under the MMAs of tile set i + 1, and the loaders (warps 0-3)
 // run ahead into the next tile set's halo as soon as a stage is released -- no prologue or epilogue is exposed after the first.
-template <int N, int T, int SA, int SB, int NB, int MW = 1, int MB = 1>
+// RES: the residual epilogue (ResNet BasicBlock, y = relu(acc + shift + residual)); only the NHWC epilogue of a plain
+// convolution reads it (the host refuses a residual with NCHW output or a transposed convolution).
+template <int N, int T, int SA, int SB, int NB, int MW = 1, int MB = 1, bool RES = false>
 __global__ void __launch_bounds__(kConvThreads, MB) k_conv_umma(const __grid_constant__ ConvParams p)
 {
     extern __shared__ __align__(1024) uint8_t s_raw[];
@@ -469,8 +474,10 @@ __global__ void __launch_bounds__(kConvThreads, MB) k_conv_umma(const __grid_con
 #pragma unroll
                     for (int j = 0; j < 32; ++j) {
                         float x = __uint_as_float(vr[j]) + s_shift[n0 + j];
-                        if (p.relu) x = fmaxf(x, 0.f);
-                        if (p.round_out) x = round_tf32(x);
+                        if (!RES) {  // (with a residual: after the addition, below)
+                            if (p.relu) x = fmaxf(x, 0.f);
+                            if (p.round_out) x = round_tf32(x);
+                        }
                         f[j] = x;
                     }
                     __syncwarp();
@@ -482,23 +489,55 @@ __global__ void __launch_bounds__(kConvThreads, MB) k_conv_umma(const __grid_con
                     const int oyb = y0 + kPatchH * t + 4 * q;
                     float *dst = p.out + (static_cast<size_t>(b) * p.out_h + oyb) * row_stride +
                                  static_cast<size_t>(x0 + pl) * p.out_c_total + p.out_c_off + n0 + ch4;
+                    // residual: the same eight 128-byte pixel lines the stores write, read the same way (eight lanes per
+                    // line), all eight loads in flight together
+                    float4 rv[RES ? 8 : 1];
+                    if (RES) {
+#pragma unroll
+                        for (int i = 0; i < 8; ++i) {
+                            rv[RES ? i : 0] = make_float4(0.f, 0.f, 0.f, 0.f);
+                            if (oyb + (i >> 1) < p.h_out && ((i & 1) ? col_ok1 : col_ok0))
+                                rv[RES ? i : 0] = __ldcs(reinterpret_cast<const float4 *>(
+                                    p.res + (dst - p.out) + (i >> 1) * row_stride + (i & 1) * 4 * p.out_c_total));
+                        }
+                    }
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {  // pixel 4 i + pl of the warp's 32 = patch row 4 q + i / 2, column pl + 4 (i & 1)
                         const int rr = 4 * i + pl;
-                        const float4 val = *reinterpret_cast<const float4 *>(stg + rr * 128 + (((lane & 7) ^ (rr & 7)) << 4));
+                        float4 val = *reinterpret_cast<const float4 *>(stg + rr * 128 + (((lane & 7) ^ (rr & 7)) << 4));
+                        if (RES) {
+                            float *const e = reinterpret_cast<float *>(&val);
+                            const float *const r = reinterpret_cast<const float *>(&rv[RES ? i : 0]);
+#pragma unroll
+                            for (int u = 0; u < 4; ++u) {
+                                float x = e[u] + r[u];
+                                if (p.relu) x = fmaxf(x, 0.f);
+                                if (p.round_out) x = round_tf32(x);
+                                e[u] = x;
+                            }
+                        }
                         if (oyb + (i >> 1) < p.h_out && ((i & 1) ? col_ok1 : col_ok0))
                             *reinterpret_cast<float4 *>(dst + (i >> 1) * row_stride + (i & 1) * 4 * p.out_c_total) = val;
                     }
                 };
-                tmem_ld32_issue(lane_base, va);
+                if (RES) {  // (no next-chunk load in flight: its 32 registers hold the residual lines instead)
 #pragma unroll 1
-                for (int ci = 0; ci < kChunks; ci += 2) {
-                    tmem_ld_wait(va);
-                    tmem_ld32_issue(lane_base + static_cast<uint32_t>((ci + 1) * 32), vb);
-                    chunk(va, ci);
-                    tmem_ld_wait(vb);
-                    if (ci + 2 < kChunks) tmem_ld32_issue(lane_base + static_cast<uint32_t>((ci + 2) * 32), va);
-                    chunk(vb, ci + 1);
+                    for (int ci = 0; ci < kChunks; ++ci) {
+                        tmem_ld32_issue(lane_base + static_cast<uint32_t>(ci * 32), va);
+                        tmem_ld_wait(va);
+                        chunk(va, ci);
+                    }
+                } else {
+                    tmem_ld32_issue(lane_base, va);
+#pragma unroll 1
+                    for (int ci = 0; ci < kChunks; ci += 2) {
+                        tmem_ld_wait(va);
+                        tmem_ld32_issue(lane_base + static_cast<uint32_t>((ci + 1) * 32), vb);
+                        chunk(va, ci);
+                        tmem_ld_wait(vb);
+                        if (ci + 2 < kChunks) tmem_ld32_issue(lane_base + static_cast<uint32_t>((ci + 2) * 32), va);
+                        chunk(vb, ci + 1);
+                    }
                 }
                 tc_fence_before();
                 mbar_arrive(acc_empty + 8u * buf);
@@ -618,7 +657,7 @@ __global__ void k_conv_wimg(const float *__restrict__ weight, const float *__res
     *reinterpret_cast<float4 *>(dst) = make_float4(v[0], v[1], v[2], v[3]);
 }
 
-template <int N, int T, int SA, int SB, int NB, int MW, int MB = 1>
+template <int N, int T, int SA, int SB, int NB, int MW, int MB = 1, bool RES = false>
 cudaError_t launch_one(const ConvParams &p, int phases, cudaStream_t st)
 {
     const size_t a_bytes = (static_cast<size_t>(p.stage_rows) * 128 + 1023) & ~static_cast<size_t>(1023);
@@ -626,12 +665,12 @@ cudaError_t launch_one(const ConvParams &p, int phases, cudaStream_t st)
     const size_t smem = SA * a_bytes + static_cast<size_t>(SB) * N * 128 + 4 * 4096 + 1024 +
                         4 * ((static_cast<size_t>(p.stage_rows) + 15) & ~static_cast<size_t>(15)) + (p.rows ? 16 * occ_cap : 0) + 64;
     if (smem > 225 * 1024) return cudaErrorInvalidValue;
-    cudaError_t e = cudaFuncSetAttribute(k_conv_umma<N, T, SA, SB, NB, MW, MB>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
+    cudaError_t e = cudaFuncSetAttribute(k_conv_umma<N, T, SA, SB, NB, MW, MB, RES>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
     if (e != cudaSuccess) return e;
     const int tiles = p.nb * p.tiles_x * p.tiles_y;
     const int ctas = current_sm_count() * MB;
     const dim3 grid(static_cast<unsigned>(tiles < ctas ? tiles : ctas), 1, static_cast<unsigned>(phases));
-    e = launch_pdl(k_conv_umma<N, T, SA, SB, NB, MW, MB>, grid, dim3(kConvThreads), smem, st, p);
+    e = launch_pdl(k_conv_umma<N, T, SA, SB, NB, MW, MB, RES>, grid, dim3(kConvThreads), smem, st, p);
     note_launch();
     return e != cudaSuccess ? e : cudaGetLastError();
 }
@@ -668,6 +707,7 @@ cudaError_t launch_conv_umma(const ConvJob &j, cudaStream_t st)
     p.round_out = j.round_out;
     p.error = j.error;
     p.timeline = debug_times_ptr();
+    p.res = j.res;
     p.h_out = (j.h_in + 2 * j.pad - j.k) / j.stride + 1;
     p.w_out = (j.w_in + 2 * j.pad - j.k) / j.stride + 1;
     p.out_mul = j.up;
@@ -682,7 +722,9 @@ cudaError_t launch_conv_umma(const ConvJob &j, cudaStream_t st)
     if (j.c_in % 32 != 0 || j.c_in < 32 || (j.stride != 1 && j.stride != 2) || j.k < 1 || j.k > 3 || (j.up != 1 && j.up != 2 && j.up != 4) ||
         (j.up > 1 && (j.k != 1 || j.stride != 1)) || (j.rows && !j.cell_row) || (!j.rows && !j.in) || p.h_out < 1 || p.w_out < 1)
         return cudaErrorInvalidValue;
-    if (j.stride == 2 && !((j.k == 3 && j.pad == 1) || (j.k == 2 && j.pad == 0))) return cudaErrorInvalidValue;
+    if (j.res && (j.up > 1 || j.out_nchw)) return cudaErrorInvalidValue;  // only the plain NHWC epilogue reads a residual
+    // (1x1 stride 2: the one tap of the even/even parity plane; the odd planes are loaded and not read)
+    if (j.stride == 2 && !((j.k == 3 && j.pad == 1) || (j.k == 2 && j.pad == 0) || (j.k == 1 && j.pad == 0))) return cudaErrorInvalidValue;
     if (j.stride == 1 && j.pad != (j.k - 1) / 2) return cudaErrorInvalidValue;
 
     // patches per tile set: two accumulator buffers of T * N columns must fit the 512 columns of tensor memory
@@ -712,7 +754,8 @@ cudaError_t launch_conv_umma(const ConvJob &j, cudaStream_t st)
     p.tiles_x = (p.w_out + kPatchW - 1) / kPatchW;
 
 #define CONV_CASE(n, t, sa, sb, nb, mw) \
-    if (n_eff == n && T == t) return launch_one<n, t, sa, sb, nb, mw>(p, phases, st)
+    if (n_eff == n && T == t)              \
+    return j.res ? launch_one<n, t, sa, sb, nb, mw, 1, true>(p, phases, st) : launch_one<n, t, sa, sb, nb, mw>(p, phases, st)
     if (j.stride == 1) {
         CONV_CASE(64, 4, 2, 4, 2, 2);
         CONV_CASE(64, 2, 2, 4, 2, 2);
