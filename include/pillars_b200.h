@@ -24,6 +24,9 @@
  *   pillars_voxelize                   datasets/processor/data_processor.py:16-61,133-180
  *                                      (VoxelGeneratorWrapper.generate -> spconv point_to_voxel) + the collate of
  *                                      datasets/dataset.py:232-244
+ *   pillars_voxelize_mean              the grouping of pillars_voxelize (any 3-D grid, e.g. VoxelNeXt's 1440 x 1440 x 40,
+ *                                      tools/cfgs/nuscenes_models/cbgs_voxel0075_voxelnext.yaml:69-79) followed by
+ *                                      models/backbones_3d/vfe/mean_vfe.py:14-31 (MeanVFE.forward), no padded voxels
  *   pillars_pfn_dense                  models/backbones_3d/vfe/pillar_vfe.py:94-123 (PillarVFE.forward) with
  *                                      :29-49 (PFNLayer.forward), eval mode
  *   pillars_scatter_bev                models/backbones_2d/map_to_bev/pointpillar_scatter.py:14-37
@@ -110,8 +113,11 @@ const char *pillars_last_error(void);
 /* 0 if device `device` (or the current one when < 0) can run this library (compute capability 10.x). */
 int pillars_device_ok(int device);
 
-/* Scratch bytes needed by pillars_voxelize / pillars_encode_bev for n_points total points in n_frames frames;
- * by pillars_scatter_bev when n_points == 0 (then only the index map counts). */
+/* Scratch bytes needed by pillars_voxelize / pillars_voxelize_mean / pillars_encode_bev / pillars_encode_stack for
+ * n_points total points in n_frames frames; by pillars_scatter_bev when n_points == 0 (then only the index map counts).
+ * It covers the hash table's layout, and the direct-mapped table's too: on a pillar grid (nz == 1) wherever that table
+ * is possible (n_frames * cells < 2^31), whatever the grouping mode; on a voxel grid (nz > 1) only where a call under the
+ * calling thread's grouping mode (pillars_set_grouping) resolves to it. */
 size_t pillars_workspace_bytes(int64_t n_points, int32_t n_frames, const pillars_grid_t *grid);
 
 /* points_b: collated batch_dict['points'] [n, row_stride] with the frame index in column 0, rows sorted by frame.
@@ -126,6 +132,19 @@ int pillars_frame_offsets(const float *points_b, int64_t n, int32_t row_stride, 
 int pillars_voxelize(const float *points, int64_t n, int32_t row_stride, int32_t col0, int32_t c_point,
                      const int32_t *frame_offsets, int32_t n_frames, const pillars_grid_t *grid,
                      const pillars_outputs_t *out, void *workspace, size_t workspace_bytes, void *stream);
+
+/* pillars_voxelize's grouping, then MeanVFE (models/backbones_3d/vfe/mean_vfe.py:14-31) on the voxels it would have
+ * padded:  voxel_mean [capacity, c_point] = voxels.sum(dim=1) / clamp_min(voxel_num_points, 1).
+ * The sum is the sequential fp32 sum over the P padded slots, bit for bit: the kept points' c_point channels (from column
+ * col0) in increasing point index, then +0.0 once when n < P, so a -0.0 sum comes out as +0.0 exactly where the padding
+ * makes it so; then one IEEE division.  No atomics: run to run, the output is bit-identical.
+ * Fills out->{voxel_coords, voxel_num_points, pillar_count} (each optional) as pillars_voxelize does; every other output of
+ * `out` must be NULL (PILLARS_E_UNSUPPORTED).  voxel_mean must not be NULL (PILLARS_E_BADARG); max_points <= 512
+ * (PILLARS_E_UNSUPPORTED).  Workspace: pillars_workspace_bytes(). */
+int pillars_voxelize_mean(const float *points, int64_t n, int32_t row_stride, int32_t col0, int32_t c_point,
+                          const int32_t *frame_offsets, int32_t n_frames, const pillars_grid_t *grid,
+                          const pillars_outputs_t *out, float *voxel_mean, void *workspace, size_t workspace_bytes,
+                          void *stream);
 
 /* Prepares pfn->folded: `folded` (device, PILLARS_FOLDED_FLOATS floats) from pfn->weight/scale/shift.  Fails with
  * PILLARS_E_UNSUPPORTED when the layer is not one the streaming kernel covers (then leave pfn->folded NULL). */
@@ -337,7 +356,7 @@ int pillars_set_stage_events(void *const *events4);
  *      reference's configs), else the open-addressing hash table;
  *   1  always the hash table;   2  the direct-mapped table whenever n_frames * cells < 2^31.
  * Both produce bit-identical outputs (tests run every grouping case through both).  pillars_workspace_bytes() covers
- * either choice. */
+ * either choice on a pillar grid and follows this thread's mode on a voxel grid (query it after setting the mode). */
 int pillars_set_grouping(int mode);
 
 /* Canvas occupancy bitmaps for the next pillars_encode_bev or pillars_encode_stack on this thread, which consumes and

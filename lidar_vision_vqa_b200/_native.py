@@ -17,6 +17,7 @@ EXPORTED_SYMBOLS = (
     "pillars_workspace_bytes",
     "pillars_frame_offsets",
     "pillars_voxelize",
+    "pillars_voxelize_mean",
     "pillars_fold_pfn",
     "pillars_pfn_dense",
     "pillars_scatter_bev",
@@ -123,6 +124,10 @@ def load(build_if_missing: bool = True) -> ctypes.CDLL:
     lib.pillars_voxelize.restype = c_int
     lib.pillars_voxelize.argtypes = [c_void_p, c_int64, c_int32, c_int32, c_int32, c_void_p, c_int32,
                                      POINTER(PillarsGrid), POINTER(PillarsOutputs), c_void_p, c_size_t, c_void_p]
+    lib.pillars_voxelize_mean.restype = c_int
+    lib.pillars_voxelize_mean.argtypes = [c_void_p, c_int64, c_int32, c_int32, c_int32, c_void_p, c_int32,
+                                          POINTER(PillarsGrid), POINTER(PillarsOutputs), c_void_p, c_void_p, c_size_t,
+                                          c_void_p]
     lib.pillars_fold_pfn.restype = c_int
     lib.pillars_fold_pfn.argtypes = [POINTER(PillarsPfn), c_void_p, c_void_p]
     lib.pillars_pfn_dense.restype = c_int

@@ -209,7 +209,13 @@ size_t pillars_workspace_bytes(int64_t n_points, int32_t n_frames, const pillars
 {
     if (!grid || n_points < 0 || n_frames < 0) return 0;
     const int64_t cells_xy = static_cast<int64_t>(grid->grid[0]) * grid->grid[1];
-    return workspace_bytes_any(n_points, n_frames, cells_xy, cells_xy * grid->grid[2]);
+    const int64_t cells = cells_xy * grid->grid[2];
+    // A pillar grid (nz == 1) is charged for the dense layout wherever it is possible, whatever the grouping mode: its
+    // table is at most 8 bytes per BEV cell, and a workspace sized once fits every mode.  A voxel grid is charged only where
+    // a call on this thread resolves to it: 16 x 1440 x 1440 x 40 cells would otherwise cost 10.7 GB that its calls never use.
+    const bool dense = grid->grid[2] == 1 ? dense_possible(n_points, n_frames, cells)
+                                          : resolve_group_mode(true, n_points, n_frames, cells) == kGroupDense;
+    return workspace_bytes_for(n_points, n_frames, cells_xy, cells, dense);
 }
 
 int pillars_frame_offsets(const float *points_b, int64_t n, int32_t row_stride, int32_t n_frames,
@@ -225,7 +231,8 @@ int pillars_frame_offsets(const float *points_b, int64_t n, int32_t row_stride, 
 }
 
 // One call of the fused encoder, as its entry point normalised it.  The features are those of `pfn`
-// (pillars_encode_bev), of `stack` (pillars_encode_stack) or none (pillars_voxelize).
+// (pillars_encode_bev), of `stack` (pillars_encode_stack), the voxel mean (pillars_voxelize_mean) or none
+// (pillars_voxelize).
 struct EncodeCall {
     const float *points;
     int64_t n;
@@ -243,6 +250,7 @@ struct EncodeCall {
     const StackDev *stack;     // checked by check_stack
     bool dynamic;              // PILLARS_MODE_DYNAMIC
     int coords_cols;
+    float *voxel_mean;         // [capacity, c_point] (pillars_voxelize_mean)
 };
 
 // Which kernels compute the per-pillar outputs of a call
@@ -251,6 +259,7 @@ enum FeatureRoute {
     kRoutePfn,     // the general one-layer kernel (pfn.cu)
     kRouteMulti,   // the general stack kernel (pfn_multi.cu)
     kRouteStream,  // the streaming kernel (pfn_stream.cu), on the point records the grouping emits
+    kRouteMean,    // k_voxel_mean (pfn.cu, pillars_voxelize_mean)
 };
 
 // The streaming kernel covers the mainstream configurations; everything else runs a general kernel.  For stacks these are
@@ -259,6 +268,7 @@ enum FeatureRoute {
 // and an empty batch stay on the general kernel.
 static FeatureRoute pick_route(const EncodeCall &c)
 {
+    if (c.voxel_mean) return kRouteMean;
     if (!c.pfn && !c.stack) return kRouteEmit;
     // (the streaming kernel's per-pillar record packs x and y into 16 bits each)
     const bool stream_ok = !g_force_generic && c.grid->grid[0] <= 0xFFFF && c.grid->grid[1] <= 0xFFFF;
@@ -327,6 +337,7 @@ static int encode(const EncodeCall &c)
     PlaceExtras px{};
     px.records = route == kRouteStream;
     px.capacity = out->pillar_capacity;
+    px.skip_index_map = route == kRouteMean;
     if (px.records) {
         for (int i = 0; i < 3; ++i) {
             px.vsz[i] = l0.vsz[i];
@@ -343,8 +354,9 @@ static int encode(const EncodeCall &c)
         return cuda_fail(e, "group_points");
     stage_mark(1, st);
 
-    // membership outputs (pillars_voxelize, pillars_encode_bev) come from k_emit_voxels, whatever computes the features
-    if (route == kRouteEmit || route == kRoutePfn || membership) {
+    // membership outputs (pillars_voxelize, pillars_encode_bev) come from k_emit_voxels, whatever computes the features;
+    // the voxel mean walks the same lists
+    if (route == kRouteEmit || route == kRoutePfn || route == kRouteMean || membership) {
         FeatureJob job{};
         job.points = c.points;
         job.n = c.n;
@@ -361,7 +373,11 @@ static int encode(const EncodeCall &c)
         job.pfn = l0;
         job.out = *out;
         job.write_cell_row = want_map && route != kRouteStream;
-        if ((e = launch_pillar_features(job, gd, ws, st)) != cudaSuccess) return cuda_fail(e, "pillar_features");
+        if (route == kRouteMean) {
+            if ((e = launch_voxel_mean(job, c.voxel_mean, gd, ws, st)) != cudaSuccess) return cuda_fail(e, "voxel_mean");
+        } else if ((e = launch_pillar_features(job, gd, ws, st)) != cudaSuccess) {
+            return cuda_fail(e, "pillar_features");
+        }
     }
     if (route == kRouteStream) {
         // the dynamic variant's pillar entries get their rows (sorted-key order) between the grouping and the feature kernel
@@ -445,6 +461,25 @@ int pillars_voxelize(const float *points, int64_t n, int32_t row_stride, int32_t
 {
     return encode({points, n, row_stride, col0, c_point, frame_offsets, n_frames, grid, out, workspace, workspace_bytes, 0,
                    stream});
+}
+
+int pillars_voxelize_mean(const float *points, int64_t n, int32_t row_stride, int32_t col0, int32_t c_point,
+                          const int32_t *frame_offsets, int32_t n_frames, const pillars_grid_t *grid,
+                          const pillars_outputs_t *out, float *voxel_mean, void *workspace, size_t workspace_bytes,
+                          void *stream)
+{
+    g_launches = 0;
+    if (!voxel_mean) return fail(PILLARS_E_BADARG, "voxel_mean is NULL");
+    if (out && (out->pillar_features || out->voxels || out->point_pillar || out->point_slot || out->bev || out->bev_half ||
+                out->want_index_map))
+        return fail(PILLARS_E_UNSUPPORTED, "pillars_voxelize_mean writes voxel_coords, voxel_num_points and pillar_count "
+                                           "only; the other outputs come from pillars_voxelize");
+    if (grid && grid->max_points > kMeanMaxPoints)
+        return fail(PILLARS_E_UNSUPPORTED, "max_points = %d (the voxel mean is built for up to %d)", grid->max_points,
+                    kMeanMaxPoints);
+    EncodeCall c{points, n, row_stride, col0, c_point, frame_offsets, n_frames, grid, out, workspace, workspace_bytes, 0, stream};
+    c.voxel_mean = voxel_mean;
+    return encode(c);
 }
 
 int pillars_encode_bev(const float *points, int64_t n, int32_t row_stride, int32_t col0, const int32_t *frame_offsets,

@@ -177,11 +177,12 @@ inline Workspace carve_workspace(void *base, int64_t n, int nb, int64_t cells_xy
     return w;
 }
 
-// bytes that fit either layout (what pillars_workspace_bytes reports)
-inline size_t workspace_bytes_any(int64_t n, int nb, int64_t cells_xy, int64_t cells)
+// What pillars_workspace_bytes reports: the hash layout, which every call may use (the dynamic variant and grouping mode 1
+// always do), and the dense layout too when `dense` (see pillars_workspace_bytes for when it is counted).
+inline size_t workspace_bytes_for(int64_t n, int nb, int64_t cells_xy, int64_t cells, bool dense)
 {
     size_t b = carve_workspace(nullptr, n, nb, cells_xy, cells, kGroupHash).total_bytes;
-    if (dense_possible(n, nb, cells)) {
+    if (dense) {
         const size_t d = carve_workspace(nullptr, n, nb, cells_xy, cells, kGroupDense).total_bytes;
         if (d > b) b = d;
     }
@@ -280,6 +281,7 @@ struct PlaceExtras {
     int32_t *voxel_num_points; // [capacity] or NULL
     bool write_cell_row;       // fill ws.cell_row for the BEV scatter
     int64_t capacity;
+    bool skip_index_map;       // hash grouping: nothing reads ws.cell_row, so it is not filled with -1 (B * ny * nx ints)
 };
 cudaError_t launch_group_points(const float *points, int64_t n, int stride, int col0, int c_point,
                                 const int32_t *frame_offsets, int nb, const GridDev &gd, const Workspace &ws,
@@ -307,6 +309,11 @@ struct FeatureJob {
     bool write_cell_row;       // fill ws.cell_row for the BEV scatter
 };
 cudaError_t launch_pillar_features(const FeatureJob &job, const GridDev &gd, const Workspace &ws, cudaStream_t st);
+// MeanVFE on the grouping's lists (pfn.cu): voxel_mean [capacity, c_point] plus job.out's voxel_coords / voxel_num_points.
+// One link of the grouping's PDL chain.  Its shared memory holds kMeanMaxPoints slots per 16-lane group at most.
+constexpr int kMeanMaxPoints = 512;
+cudaError_t launch_voxel_mean(const FeatureJob &job, float *voxel_mean, const GridDev &gd, const Workspace &ws,
+                              cudaStream_t st);
 
 struct FastJob {
     int64_t n;  // upper bound of listed points (the input point count)

@@ -6,6 +6,7 @@
 // fused path walks the pillar's index list straight into the raw point array; padded slots contribute the closed
 // form relu(shift) (pillar_vfe.py:116-118 zeroes them BEFORE the linear, :39-42 lets them take part in the max).
 // The 11 -> 64 contraction stays on the FMA pipes (memory/latency bound, no tensor cores).
+// The same walk over the lists also serves the reference's padded outputs (k_emit_voxels) and MeanVFE (k_voxel_mean).
 #include "common.cuh"
 
 namespace pillars {
@@ -301,6 +302,66 @@ __global__ void __launch_bounds__(kThreads) k_emit_voxels(const FeatParams p)
 }
 
 // ---------------------------------------------------------------------------------------------
+// MeanVFE (models/backbones_3d/vfe/mean_vfe.py:14-31) straight from the lists, without the padded [M,P,C] tensor:
+//   voxel_mean[row][c] = (sequential fp32 sum of the reference's P slots of channel c) / max(n_keep, 1)
+// Slot s holds the kept point of rank s (kept = the n_keep smallest indices of the list, the hard voxeliser's first-P rule),
+// and the padding slots hold +0.0.  So the sum adds the kept points in increasing point index, then one +0.0 when padding
+// follows: that changes nothing but the sign of a -0.0 sum, exactly as the padding does.  A 16-lane group ranks its kept
+// entries (atomic arrival order is no order at all), puts their point indices into shared memory by rank, and lane c then
+// adds channel c slot after slot.  No atomics: the result depends on the points alone.
+// ---------------------------------------------------------------------------------------------
+struct MeanParams {
+    FeatParams f;  // pillar_features, voxels and the membership outputs are not used
+    float *mean;   // [capacity, c_point]
+};
+
+__global__ void __launch_bounds__(kThreads) k_voxel_mean(const __grid_constant__ MeanParams mp)
+{
+    extern __shared__ uint32_t s_slot[];  // [kThreads / kLpp][P]: point index in each kept slot of the group's voxel
+    const FeatParams &p = mp.f;
+    const int lane = threadIdx.x & 31, sub = lane & (kLpp - 1), grp = lane / kLpp;
+    const int warp = threadIdx.x >> 5;
+    constexpr int kGroupsPerWarp = 32 / kLpp;
+    const int P = p.gd.max_points, C = p.c_point;
+    uint32_t *slot = s_slot + (warp * kGroupsPerWarp + grp) * P;
+    pdl_wait();
+    pdl_trigger();
+    const uint32_t total = p.hdr->total_pillars;
+    const uint32_t warp_stride = gridDim.x * (kThreads / 32) * kGroupsPerWarp;
+    for (uint32_t gbase = (blockIdx.x * (kThreads / 32) + warp) * kGroupsPerWarp; gbase < total; gbase += warp_stride) {
+        const uint32_t g = gbase + grp;
+        const PillarInfo pi = resolve_pillar(p, g, total, sub);
+        const uint32_t n_eff = pi.live ? pi.n : 0u;
+        const uint32_t n_keep = min(n_eff, static_cast<uint32_t>(P));
+        for (uint32_t j = sub; j < n_eff; j += kLpp) {
+            const uint32_t idx = p.sorted_idx[pi.list + j];
+            if (idx <= pi.thr) {
+                uint32_t rank = 0;  // kept entries are exactly the n_keep smallest: rank among all == rank among kept
+                for (uint32_t t = 0; t < n_eff; ++t) rank += (p.sorted_idx[pi.list + t] < idx) ? 1u : 0u;
+                slot[rank] = idx;
+            }
+        }
+        __syncwarp();
+        if (pi.live) {
+            // (check_points caps row_stride at 16, so one pass covers every channel; the loop keeps any C correct)
+            for (int c = sub; c < C; c += kLpp) {
+                const float *col = p.points + p.col0 + c;
+                float acc = __ldg(col + static_cast<int64_t>(slot[0]) * p.stride);
+#pragma unroll 4
+                for (uint32_t r = 1; r < n_keep; ++r) acc = __fadd_rn(acc, __ldg(col + static_cast<int64_t>(slot[r]) * p.stride));
+                if (n_keep < static_cast<uint32_t>(P)) acc = __fadd_rn(acc, 0.f);  // the padding slots
+                mp.mean[pi.row * C + c] = __fdiv_rn(acc, static_cast<float>(max(n_keep, 1u)));
+            }
+            if (sub == 0) {
+                if (p.voxel_coords) *reinterpret_cast<int4 *>(p.voxel_coords + pi.row * 4) = make_int4(pi.b, pi.z, pi.y, pi.x);
+                if (p.voxel_num_points) p.voxel_num_points[pi.row] = static_cast<int32_t>(n_keep);
+            }
+        }
+        __syncwarp();  // the slots are rewritten by the next voxel
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // hard variant: the reference's own padded input  voxels [M,P,C], num_points [M], coords [M,4] (b,z,y,x)
 // ---------------------------------------------------------------------------------------------
 struct DenseParams {
@@ -429,9 +490,7 @@ cudaError_t dispatch_dense(const DenseParams &p, bool abs_xyz, bool dist, int gr
     return cudaGetLastError();
 }
 
-}  // namespace
-
-cudaError_t launch_pillar_features(const FeatureJob &job, const GridDev &gd, const Workspace &ws, cudaStream_t st)
+FeatParams make_feat_params(const FeatureJob &job, const GridDev &gd, const Workspace &ws)
 {
     FeatParams p{};
     p.points = job.points;
@@ -456,6 +515,14 @@ cudaError_t launch_pillar_features(const FeatureJob &job, const GridDev &gd, con
     p.point_slot = job.out.point_slot;
     p.voxels = job.out.voxels;
     p.capacity = job.out.pillar_capacity;
+    return p;
+}
+
+}  // namespace
+
+cudaError_t launch_pillar_features(const FeatureJob &job, const GridDev &gd, const Workspace &ws, cudaStream_t st)
+{
+    const FeatParams p = make_feat_params(job, gd, ws);
     if (job.n == 0) return cudaSuccess;
 
     // persistent grids: the pillar count lives on the device, so size for the SM count and stride
@@ -479,6 +546,18 @@ cudaError_t launch_pillar_features(const FeatureJob &job, const GridDev &gd, con
         }
         note_launch();
     }
+    return err;
+}
+
+cudaError_t launch_voxel_mean(const FeatureJob &job, float *voxel_mean, const GridDev &gd, const Workspace &ws,
+                              cudaStream_t st)
+{
+    if (job.n == 0) return cudaSuccess;
+    if (gd.max_points > kMeanMaxPoints) return cudaErrorInvalidValue;
+    const MeanParams mp{make_feat_params(job, gd, ws), voxel_mean};
+    const size_t smem = sizeof(uint32_t) * (kThreads / kLpp) * gd.max_points;
+    const cudaError_t err = launch_pdl(k_voxel_mean, dim3(grid_for(job.n, num_sms() * 8)), dim3(kThreads), smem, st, mp);
+    note_launch();
     return err;
 }
 

@@ -376,15 +376,17 @@ cudaError_t launch_group_points(const float *points, int64_t n, int stride, int 
     cudaError_t err;
     // One memset per call: the hash table must be empty before the first insert.  The rest of the scratch (scan header and
     // tile descriptors: zero; BEV index map: -1) is initialised by the insert kernel itself, unless there is no point at all.
+    // The index map sits at the end of the 0xFF region; a call that reads no map leaves it alone.
     const size_t table_bytes = reinterpret_cast<char *>(ws.cell_row) - ws.ff_begin;
-    const size_t map_bytes = ws.ff_bytes - table_bytes;
+    const size_t map_bytes = extras.skip_index_map ? 0 : ws.ff_bytes - table_bytes;
     const bool in_kernel_init = n > 0 && static_cast<int64_t>(ws.zero_bytes / 16) <= n && ws.zero_bytes % 16 == 0 &&
                                 map_bytes % 16 == 0;
     if (!in_kernel_init) {
         if ((err = cudaMemsetAsync(ws.zero_begin, 0, ws.zero_bytes, st)) != cudaSuccess) return err;
         note_launch();
     }
-    if ((err = cudaMemsetAsync(ws.ff_begin, 0xFF, in_kernel_init ? table_bytes : ws.ff_bytes, st)) != cudaSuccess) return err;
+    if ((err = cudaMemsetAsync(ws.ff_begin, 0xFF, in_kernel_init ? table_bytes : table_bytes + map_bytes, st)) != cudaSuccess)
+        return err;
     note_launch();
     if (n == 0) {
         if (pillar_count) {

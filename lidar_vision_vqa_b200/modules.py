@@ -7,9 +7,12 @@
   models/backbones_3d/vfe/pillar_vfe.py:52-123        PillarVFE              PillarVFE        ('voxels' input)
   models/backbones_3d/vfe/dynamic_pillar_vfe.py:49-142 (point-input contract) PillarVFEFromPoints ('points' input,
                                                                               hard-voxeliser semantics, fused grouping)
+  models/backbones_3d/vfe/mean_vfe.py:6-31            MeanVFE                MeanVFEFromPoints ('points' input, hard
+                                                                              voxeliser + voxel mean, any 3-D grid)
   models/backbones_2d/map_to_bev/pointpillar_scatter.py:5-37  PointPillarScatter  PointPillarScatter
 
-Inference only: BatchNorm is folded from the running statistics, so ``forward`` raises in training mode.
+The PFN modules are inference only: BatchNorm is folded from the running statistics, so ``forward`` raises in training
+mode.  MeanVFEFromPoints has no parameters and runs in either mode.
 The compute is in libpillars_b200.so; a missing library or a non-sm_100 device raises (no eager fallback).
 """
 from __future__ import annotations
@@ -66,6 +69,23 @@ def _points_on_device(points: torch.Tensor) -> torch.Tensor:
             raise NativeLibraryError("the pillar path runs on a B200 only: no CUDA device (no CPU fallback)")
         points = points.cuda(non_blocking=True)
     return points.contiguous()
+
+
+def _point_batch(batch_dict):
+    """``(points on the device, batch size, frame offsets [B+1] int32 on the device, col0)`` of a point-input batch:
+    ``points [N, 1+C]`` with the frame index in column 0, or packed ``[N, C]`` rows with ``points_frame_offsets``."""
+    points = _points_on_device(batch_dict["points"])
+    batch_size = int(batch_dict["batch_size"])
+    packed_offs = batch_dict.get("points_frame_offsets")
+    if packed_offs is None:
+        return points, batch_size, ops.frame_offsets_from_points(points, batch_size), 1
+    # packed [N, C] rows + explicit offsets instead of the frame-index column
+    offs = torch.as_tensor(packed_offs, dtype=torch.int32)
+    if not offs.is_cuda:
+        offs = offs.to(points.device, non_blocking=True)
+    if offs.numel() != batch_size + 1:
+        raise ValueError("points_frame_offsets must have batch_size + 1 entries")
+    return points, batch_size, offs, 0
 
 
 class VFETemplate(nn.Module):
@@ -257,19 +277,7 @@ class PillarVFEFromPoints(_PillarVFEBase):
                                  self.max_voxels)
 
     def forward(self, batch_dict, **kwargs):
-        points = _points_on_device(batch_dict["points"])
-        batch_size = int(batch_dict["batch_size"])
-        packed_offs = batch_dict.get("points_frame_offsets")
-        if packed_offs is not None:  # packed [N, C] rows + explicit offsets instead of the frame-index column
-            offs = torch.as_tensor(packed_offs, dtype=torch.int32)
-            if not offs.is_cuda:
-                offs = offs.to(points.device, non_blocking=True)
-            if offs.numel() != batch_size + 1:
-                raise ValueError("points_frame_offsets must have batch_size + 1 entries")
-            col0 = 0
-        else:
-            offs = ops.frame_offsets_from_points(points, batch_size)
-            col0 = 1
+        points, batch_size, offs, col0 = _point_batch(batch_dict)
         if self._single_layer():
             params, encode = self._params(points.device), ops.encode_bev
         else:
@@ -321,6 +329,51 @@ class PillarVFEFromPoints(_PillarVFEBase):
                                   with_bev=self.fuse_scatter)
             self._ring[i] = b
         return b
+
+
+class MeanVFEFromPoints(VFETemplate):
+    """Point-input MeanVFE (mean_vfe.py:6-31) with the hard voxeliser in front: the equivalent of
+    ``transform_points_to_voxels`` (data_processor.py:133-180) + ``MeanVFE`` on any 3-D grid, e.g. VoxelNeXt's
+    1440 x 1440 x 40 (cbgs_voxel0075_voxelnext.yaml), with no padded ``voxels`` in between.  Reads ``points [N, 1+C]
+    (b,x,y,z,...)``, or packed ``[N, C]`` rows with ``points_frame_offsets`` (as :class:`PillarVFEFromPoints`).  Writes
+    ``voxel_features [M, C]`` (bit-identical to a sequential fp32 sum over the padded slots divided by the capped count),
+    ``voxel_coords [M, 4] int32 (b, z, y, x)`` (what spconv's ``SparseConvTensor`` takes), ``voxel_num_points``,
+    ``pillar_count [B+1]`` (device) and, with synced counts, ``pillars_per_frame`` (host).
+
+    model_cfg keys (all optional): MAX_POINTS_PER_VOXEL (10), MAX_NUMBER_OF_VOXELS (160000; an int or {'train', 'test'},
+    chosen by the module's training flag), SYNC_COUNTS (True; False keeps capacity-sized outputs and the counts on the
+    device, as for :class:`PillarVFEFromPoints`).  The defaults are VoxelNeXt's nuScenes test values.  The module has no
+    parameters, so it runs in training mode too."""
+
+    def __init__(self, model_cfg, num_point_features, voxel_size, point_cloud_range, grid_size, **kwargs):
+        super().__init__(model_cfg=model_cfg)
+        self.num_point_features = int(num_point_features)
+        self.max_points = int(_cfg_get(model_cfg, "MAX_POINTS_PER_VOXEL", 10))
+        self.max_voxels_cfg = _cfg_get(model_cfg, "MAX_NUMBER_OF_VOXELS", 160000)
+        _mode_value(self.max_voxels_cfg, training=False)  # an int or a {train, test} dict, checked here
+        self.sync_counts = bool(_cfg_get(model_cfg, "SYNC_COUNTS", True))
+        self.voxel_size = [float(v) for v in voxel_size]
+        self.point_cloud_range = [float(v) for v in np.asarray(point_cloud_range).tolist()]
+        self.grid_size = [int(v) for v in np.asarray(grid_size).tolist()]
+
+    def get_output_feature_dim(self):
+        return self.num_point_features
+
+    def forward(self, batch_dict, **kwargs):
+        points, batch_size, offs, col0 = _point_batch(batch_dict)
+        grid = ops.GridSpec(self.point_cloud_range, self.voxel_size, self.grid_size, self.max_points,
+                            _mode_value(self.max_voxels_cfg, self.training))
+        res = ops.voxelize_mean(points, offs, grid, col0=col0, c_point=self.num_point_features)
+        batch_dict["pillar_count"] = res["pillar_count"]  # device, [B+1]
+        keys = ("voxel_features", "voxel_coords", "voxel_num_points")
+        if not self.sync_counts:  # capacity-sized outputs, rows beyond the device-side count are padding
+            batch_dict.update({k: res[k] for k in keys})
+            return batch_dict
+        counts = res["pillar_count"].cpu()  # the call's one host synchronisation
+        m = int(counts[-1])
+        batch_dict.update({k: res[k][:m] for k in keys})
+        batch_dict["pillars_per_frame"] = counts[:-1]  # host tensor
+        return batch_dict
 
 
 class DynamicPillarVFE(_PillarVFEBase):
@@ -460,6 +513,7 @@ VFE_REGISTRY = {
     "VFETemplate": VFETemplate,
     "PillarVFE": PillarVFE,
     "PillarVFEFromPoints": PillarVFEFromPoints,
+    "MeanVFEFromPoints": MeanVFEFromPoints,
     "DynPillarVFE": DynamicPillarVFE,
     "DynamicPillarVFESimple2D": DynamicPillarVFESimple2D,
 }

@@ -250,6 +250,37 @@ def voxelize(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, 
     return res
 
 
+def voxelize_mean(points: torch.Tensor, frame_offsets: torch.Tensor, grid: GridSpec, *, col0: int = 0,
+                  c_point: Optional[int] = None, capacity: Optional[int] = None, ws_slot: int = 0) -> Dict[str, torch.Tensor]:
+    """:func:`voxelize`'s grouping followed by MeanVFE (mean_vfe.py:14-31) without the padded voxels:
+    ``voxel_features [capacity, c_point]`` is the mean of each voxel's kept points, bit-identical to a sequential fp32 sum
+    over the reference's padded slots divided by ``max(voxel_num_points, 1)``.  Also returns ``voxel_coords [capacity, 4]``
+    (b, z, y, x), ``voxel_num_points`` and ``pillar_count [B+1]``; rows beyond the count are undefined (``trim`` after a
+    sync).  Nothing synchronises."""
+    _check_points(points, frame_offsets)
+    lib = _native.load()
+    n, stride = points.shape
+    nb = frame_offsets.numel() - 1
+    c_point = stride - col0 if c_point is None else c_point
+    cap = min(n, nb * grid.max_voxels) if capacity is None else capacity
+    cap = max(int(cap), 1)
+    dev = points.device
+    g = grid.native()
+    res = {
+        "voxel_features": torch.empty((cap, c_point), dtype=torch.float32, device=dev),
+        "voxel_coords": torch.empty((cap, 4), dtype=torch.int32, device=dev),
+        "voxel_num_points": torch.empty((cap,), dtype=torch.int32, device=dev),
+        "pillar_count": torch.empty((nb + 1,), dtype=torch.int32, device=dev),
+    }
+    out = _outputs(res, cap)
+    need = lib.pillars_workspace_bytes(n, nb, ctypes.byref(g))
+    ws = workspace(need, dev, ws_slot)
+    check(lib.pillars_voxelize_mean(points.data_ptr(), n, stride, col0, c_point, frame_offsets.data_ptr(), nb,
+                                    ctypes.byref(g), ctypes.byref(out), res["voxel_features"].data_ptr(), ws.data_ptr(),
+                                    ws.numel(), _stream_ptr()), "pillars_voxelize_mean")
+    return res
+
+
 def _padded_inputs(voxels: torch.Tensor, num_points: torch.Tensor, coords: torch.Tensor, c_point: int):
     """Checks the reference's padded input and brings ``num_points`` and ``coords`` to what the library reads, with a
     flag that is 1 for float32: float32 and int32 pass through, other floating types become float32, other integer types

@@ -67,6 +67,12 @@ WORKLOADS = {
     ),
 }
 
+# VoxelNeXt's nuScenes grid (tools/cfgs/nuscenes_models/cbgs_voxel0075_voxelnext.yaml:69-79): 1440 x 1440 x 40 voxels with
+# MAX_POINTS_PER_VOXEL 10 and MAX_NUMBER_OF_VOXELS {train: 120000, test: 160000} (the test value here).  Not a WORKLOAD of
+# bench.py: it feeds MeanVFEFromPoints (tests/test_gpu_voxel_mean.py, profiles/scripts/voxel_mean_times.py).
+VOXELNEXT_NUSCENES = GridConfig(point_cloud_range=(-54.0, -54.0, -5.0, 54.0, 54.0, 3.0), voxel_size=(0.075, 0.075, 0.2),
+                                max_points_per_voxel=10, max_voxels=160000)
+
 
 def _one_revolution(rng: np.random.Generator, m: SweepModel) -> np.ndarray:
     az = (np.arange(m.az_steps, dtype=np.float64) + rng.uniform()) * (2.0 * np.pi / m.az_steps)
